@@ -44,7 +44,7 @@ typedef struct kzb_net_info {
     int32_t policy_len;                       /* product of the policy output's non-batch dims */
     int32_t channels, depth;                  /* tower width / residual blocks                 */
     int32_t max_batch, precision, device;
-    int32_t conv_mode;      /* 0: padded-row 2-D TMA im2col, 1: 8x8-board 4-D TMA box, -1: fp32 path */
+    int32_t conv_mode;      /* 0: row kernels (dense rows), 1: 8x8-board kernels, -1: fp32 */
     double flops_per_position; /* algorithmic FLOPs (no padding/halo), SURVEY.md 8(d)          */
 } kzb_net_info;
 

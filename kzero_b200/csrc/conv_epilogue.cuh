@@ -1,5 +1,5 @@
-// Epilogue shared by the per-layer conv kernels (conv_tc.cu, conv_tch.cu): one epilogue warp drains its 32 TMEM lanes of
-// one 128-row accumulator tile.  tcgen05.ld -> +bias (BN folded on the host) -> relu -> +residual -> bf16 / f32 store.
+// Epilogue of conv_tc.cu: one epilogue warp drains its 32 TMEM lanes of one 128-row accumulator tile.
+// tcgen05.ld -> +bias (BN folded on the host) -> relu -> +residual -> bf16 / f32 store.
 // Order matters: the reference block is x + relu(bn(conv(...))), relu BEFORE the add (python/lib/model/post_act.py:218-228).
 #pragma once
 #include "kernels.cuh"
@@ -15,11 +15,6 @@ __device__ __forceinline__ void conv_epilogue_tile(const ConvTcParams& p, const 
                                                    uint64_t* tmem_full, uint32_t buf_phase, uint64_t* tmem_empty, int ch_base, int n_cols) {
     using namespace tc;
     const int row = tile * 128 + quarter * 32 + lane;
-    bool on_board = true;
-    if (p.mode == 0) {
-        int r = row % p.lay.board_pitch;
-        on_board = (r % p.lay.rank_pitch) < p.lay.W && (r / p.lay.rank_pitch) < p.lay.H;
-    }
     const bool store = row < p.valid_rows;
 
     // residual row (bf16) prefetched into registers BEFORE waiting for the accumulator, so its global
@@ -75,10 +70,6 @@ __device__ __forceinline__ void conv_epilogue_tile(const ConvTcParams& p, const 
                     v[j] += __bfloat162float(h0[j]);
                     v[8 + j] += __bfloat162float(h1[j]);
                 }
-            }
-            if (!on_board) {
-#pragma unroll
-                for (int j = 0; j < 16; j++) v[j] = 0.0f;  // keep the padding rows zero for the next layer
             }
             if (store) {
                 if (p.out_f32) {

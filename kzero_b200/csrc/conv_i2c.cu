@@ -5,7 +5,7 @@
 // channels-last rows [board][y][x][C] with NO padding rows: the TMA engine's im2col mode (cuTensorMapEncodeIm2col, bounding box
 // corners -1 / -1 for a 3x3 filter with zero padding 1) walks 128 consecutive output pixels across ranks and boards, adds the tap
 // offset and zero-fills whatever falls off the board, so every row the tensor core multiplies is a real square (the padded-row
-// kernels conv_tc / conv_tch spend 19 % of their MMAs on zero rows on 9x9, 10 % on 19x19).  Each 128-pixel tile is re-loaded per
+// layout it replaced spent 19 % of the MMAs on zero rows on 9x9, 10 % on 19x19).  Each 128-pixel tile is re-loaded per
 // tap (16 KB, SWIZZLE_128B) next to the half weight tile (cout/2 x 64, 16 KB): exactly the shared-memory traffic of a plain
 // 2-SM GEMM.
 //

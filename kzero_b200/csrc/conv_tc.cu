@@ -1,23 +1,16 @@
-// K1 (generic form): implicit-GEMM conv3x3 / conv1x1 on the 5th-gen tensor cores, one CTA per 128-row tile.  Today it runs the
-// layers conv_i2c.cu / tower8k.cu / heads8.cu do not take: head 1x1 convs with f32 output (scalar conv, policy conv2, attention
-// convs) and, with KZB_NO_I2C=1, 3x3 layers on padded rows (the A/B baseline of conv_i2c.cu).
+// K1 (head form): conv1x1 as a GEMM on the 5th-gen tensor cores, one CTA per 128-row tile.  It runs the head convs with f32
+// output (scalar conv, policy conv2, attention convs), the layers conv_i2c.cu / tower8k.cu / heads8.cu do not take.  Every head conv
+// is 1x1 (net_spec.cpp rejects any other), so a tile needs no tap shifts and no zero padding.
 //
-// Replaces the per-layer `cudnnConvolutionBiasActivationForward` (fp32 NCHW) + separate residual-add
-// and relu autokernels of the reference's CUDA executor (kn-cuda-eval 0.7.3 planner, evidence
-// docs/conv_bn_sm_flow.svg; call site rust/kz-core/src/network/cudnn.rs:73).
+// Replaces the per-layer `cudnnConvolutionBiasActivationForward` (fp32 NCHW) of the reference's CUDA executor (kn-cuda-eval 0.7.3
+// planner, evidence docs/conv_bn_sm_flow.svg; call site rust/kz-core/src/network/cudnn.rs:73).
 //
-// GEMM view (per layer):  D[M=positions, N=cout] = sum_{tap, ci} A_tap[M, ci] * W[N, tap*cin + ci]
-//   * activations are channels-last bf16 rows [position][cin_pad]; one M tile = 128 positions
-//   * A_tap is never materialised: the TMA engine loads the tile *shifted by the tap* and zero-fills
-//     everything that falls off the board:
-//       mode 1 (8x8 boards, dense rows): 4-D tensor map (c, x, y, board), box (64, 8, 8, 2) at (c0, dx, dy, b0)
-//       mode 0 (any board, padded rows): 2-D tensor map (c, row), box (64, 128) at (c0, row0 + dy*rank_pitch + dx);
-//              the padded row layout (kernels.cuh RowLayout) guarantees the shifted row is a zero row
+// GEMM view (per layer):  D[M=positions, N=cout] = sum_ci A[M, ci] * W[N, ci]
+//   * activations are dense channels-last bf16 rows [position][cin_pad], one row per square; one M tile = 128 rows, loaded by a
+//     2-D tensor map (c, row) with box (64, 128) at (c0, tile * 128); rows past the buffer are zero-filled
 //   * both operands land in shared memory in the canonical K-major SWIZZLE_128B layout, tcgen05.mma
 //     (cta_group::1, kind::f16, M=128, N=cout_pad, K=16) accumulates fp32 in TMEM
-//   * epilogue (4 warps): tcgen05.ld -> +bias (BN folded on the host) -> relu -> +residual -> bf16 store.
-//     Order matters: the reference block is x + relu(bn(conv(...))), relu BEFORE the add
-//     (python/lib/model/post_act.py:218-228).
+//   * epilogue (4 warps): tcgen05.ld -> +bias (BN folded on the host) -> relu -> +residual -> bf16 / f32 store (conv_epilogue.cuh)
 //   * persistent CTAs, warp-specialised: warp 0 TMA producer, warp 1 MMA issuer (+TMEM owner),
 //     warps 2..5 epilogue; smem ring of `stages` (A,B) slots; two TMEM accumulators so the epilogue of
 //     tile i overlaps the MMAs of tile i+1.
@@ -66,7 +59,6 @@ __global__ void __launch_bounds__(kThreads, 1)
     const SmemLayout sm = carve(smem, p.n, p.stages);
     const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
     const int stage_bytes = kABytes + p.n * 128;
-    const int iters_per_tile = p.taps * p.kblocks;
     const int my_tiles = (p.num_tiles - int(blockIdx.x) + int(gridDim.x) - 1) / int(gridDim.x);
 
     if (warp == 0 && lane == 0) {
@@ -102,24 +94,16 @@ __global__ void __launch_bounds__(kThreads, 1)
             uint32_t phase = 0;
             for (int ti = 0; ti < my_tiles; ti++) {
                 const int tile = int(blockIdx.x) + ti * int(gridDim.x);
-                for (int tap = 0; tap < p.taps; tap++) {
-                    const int dy = p.taps == 9 ? tap / 3 - 1 : 0;
-                    const int dx = p.taps == 9 ? tap % 3 - 1 : 0;
-                    for (int kb = 0; kb < p.kblocks; kb++) {
-                        mbar_wait(&sm.empty[stage], phase ^ 1);
-                        uint8_t* a_dst = sm.stage_base + size_t(stage) * stage_bytes;
-                        uint8_t* b_dst = a_dst + kABytes;
-                        mbar_expect_tx(&sm.full[stage], uint32_t(stage_bytes));
-                        if (p.mode == 1)
-                            tma_load_4d(&tmap_a, &sm.full[stage], a_dst, kb * kBlockK, dx, dy, tile * p.boards_per_tile);
-                        else
-                            tma_load_2d(&tmap_a, &sm.full[stage], a_dst, kb * kBlockK,
-                                        tile * kTileM + dy * p.lay.rank_pitch + dx);
-                        tma_load_2d(&tmap_b, &sm.full[stage], b_dst, tap * p.cin_pad + kb * kBlockK, 0);
-                        if (++stage == p.stages) {
-                            stage = 0;
-                            phase ^= 1;
-                        }
+                for (int kb = 0; kb < p.kblocks; kb++) {
+                    mbar_wait(&sm.empty[stage], phase ^ 1);
+                    uint8_t* a_dst = sm.stage_base + size_t(stage) * stage_bytes;
+                    uint8_t* b_dst = a_dst + kABytes;
+                    mbar_expect_tx(&sm.full[stage], uint32_t(stage_bytes));
+                    tma_load_2d(&tmap_a, &sm.full[stage], a_dst, kb * kBlockK, tile * kTileM);
+                    tma_load_2d(&tmap_b, &sm.full[stage], b_dst, kb * kBlockK, 0);
+                    if (++stage == p.stages) {
+                        stage = 0;
+                        phase ^= 1;
                     }
                 }
             }
@@ -137,7 +121,7 @@ __global__ void __launch_bounds__(kThreads, 1)
             mbar_wait(&sm.tmem_empty[buf], buf_phase ^ 1);
             tc_fence_after();
             const uint32_t tmem_d = tmem_base + buf * acc_stride;
-            for (int it = 0; it < iters_per_tile; it++) {
+            for (int it = 0; it < p.kblocks; it++) {
                 mbar_wait(&sm.full[stage], phase);
                 tc_fence_after();
                 const uint32_t a_lo = umma_desc_lo(smem_u32(sm.stage_base + size_t(stage) * stage_bytes));

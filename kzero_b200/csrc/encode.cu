@@ -47,29 +47,24 @@ __global__ void __launch_bounds__(kEncodeThreads) encode_nhwc_kernel(EncodeParam
     for (int i = threadIdx.x; i < p.bits_stride; i += kEncodeThreads) s_bits[i] = p.bits[size_t(b) * p.bits_stride + i];
     __syncthreads();
 
-    const int W = p.lay.W, H = p.lay.H, area = W * H;
+    const int area = p.lay.W * p.lay.H;
     const int32_t* sym_row = p.sym ? p.square_src + size_t(p.sym[b]) * area : nullptr;
     const int groups = p.c_pad / 8;
-    const int vecs = p.lay.board_pitch * groups;
-    const size_t vec_base = size_t(b) * p.lay.board_pitch * groups;
+    const int vecs = area * groups;
+    const size_t vec_base = size_t(b) * area * groups;
     for (int v = threadIdx.x; v < vecs; v += kEncodeThreads) {
-        int r = v / groups, g = v % groups;
-        int y = r / p.lay.rank_pitch, x = r % p.lay.rank_pitch;
-        bool on_board = x < W && y < H;
-        int sq = y * W + x;
-        const int src_sq = (sym_row && on_board) ? sym_row[sq] : sq;
+        int sq = v / groups, g = v % groups;
+        const int src_sq = sym_row ? sym_row[sq] : sq;
         Vec8<T> out;
 #pragma unroll
         for (int j = 0; j < 8; j++) {
             int c = g * 8 + j;
             float f = 0.0f;
-            if (on_board) {
-                if (c < p.scalar_count) {
-                    f = s_scalars[c];  // mod.rs:54-56: each scalar broadcast over the plane
-                } else if (c < p.scalar_count + p.bool_channels) {
-                    int i = (c - p.scalar_count) * area + src_sq;  // mod.rs:57-59, bit_buffer.rs:73-75
-                    f = float((s_bits[i >> 3] >> (i & 7)) & 1);
-                }
+            if (c < p.scalar_count) {
+                f = s_scalars[c];  // mod.rs:54-56: each scalar broadcast over the plane
+            } else if (c < p.scalar_count + p.bool_channels) {
+                int i = (c - p.scalar_count) * area + src_sq;  // mod.rs:57-59, bit_buffer.rs:73-75
+                f = float((s_bits[i >> 3] >> (i & 7)) & 1);
             }
             out.set(j, f);
         }
@@ -100,19 +95,17 @@ __global__ void nchw_to_rows_kernel(const float* __restrict__ in, int batch, int
                                     void* out) {
     const int area = lay.W * lay.H;
     const int groups = c_pad / 8;
-    size_t total = size_t(batch) * lay.board_pitch * groups;
+    size_t total = size_t(batch) * area * groups;
     for (size_t v = blockIdx.x * size_t(blockDim.x) + threadIdx.x; v < total; v += size_t(gridDim.x) * blockDim.x) {
         int g = int(v % groups);
         size_t rr = v / groups;
-        int b = int(rr / lay.board_pitch), r = int(rr % lay.board_pitch);
-        int y = r / lay.rank_pitch, x = r % lay.rank_pitch;
-        bool on_board = x < lay.W && y < lay.H;
+        int b = int(rr / area), sq = int(rr % area);
         Vec8<T> o;
 #pragma unroll
         for (int j = 0; j < 8; j++) {
             int c = g * 8 + j;
             float f = 0.0f;
-            if (on_board && c < channels) f = in[(size_t(b) * channels + c) * area + y * lay.W + x];
+            if (c < channels) f = in[(size_t(b) * channels + c) * area + sq];
             o.set(j, f);
         }
         o.store(out, v);
@@ -204,7 +197,7 @@ void launch_encode_nchw_f32(const uint8_t* bits, const float* scalars, int batch
 void launch_nchw_to_rows(const float* in, int batch, int channels, RowLayout lay, int c_pad, void* out, bool out_bf16,
                          cudaStream_t s) {
     if (batch <= 0) return;
-    size_t total = size_t(batch) * lay.board_pitch * (c_pad / 8);
+    size_t total = size_t(batch) * lay.W * lay.H * (c_pad / 8);
     int blocks = int(std::min<size_t>((total + 255) / 256, 148 * 16));
     if (out_bf16)
         nchw_to_rows_kernel<__nv_bfloat16><<<blocks, 256, 0, s>>>(in, batch, channels, lay, c_pad, out);

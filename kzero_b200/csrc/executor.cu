@@ -146,6 +146,8 @@ Net::Net(int device, NetSpec spec, int max_batch, int precision)
     if (spec_.has_extra && spec_.extra_fc.out != 1) throw std::runtime_error("policy head with more than one extra move is not supported");
     if (spec_.channels > 256 || spec_.policy_conv1.cout > 256 || spec_.policy_conv2.cout > 256)
         throw std::runtime_error("more than 256 channels is not supported");
+    if (precision == 1 && (spec_.board_w > 255 || spec_.board_h > 255))
+        throw std::runtime_error("boards wider or taller than 255 squares are not supported in bf16; use precision=fp32");
 
     CK(cudaStreamCreateWithFlags(&stream_, cudaStreamNonBlocking));
     if (const char* bs = std::getenv("KZB_BLOCKING_SYNC")) blocking_sync_ = bs[0] == '1';
@@ -265,37 +267,23 @@ void Net::build_bf16() {
         auto off = [](const char* name) { const char* v = std::getenv(name); return v && v[0] == '1'; };
         const bool small = spec_.board_w <= 8 && spec_.board_h <= 8 && (spec_.board_w < 8 || spec_.board_h < 8);
         const int units = (((max_batch_ + 3) / 4 + 1) & ~1);
-        embed8_ = small && !off("KZB_FORCE_LINEAR") && !off("KZB_NO_CONV8") && !off("KZB_NO_TOWER8") &&
-                  !off("KZB_NO_EMBED8") && round_up(C, 64) <= 128 && (units + num_sms_ - 1) / num_sms_ <= tower8k_max_local_units();
+        embed8_ = small && !off("KZB_FORCE_LINEAR") && !off("KZB_NO_TOWER8") && !off("KZB_NO_EMBED8") && round_up(C, 64) <= 128 &&
+                  (units + num_sms_ - 1) / num_sms_ <= tower8k_max_local_units();
     }
     const int W = embed8_ ? 8 : spec_.board_w, H = embed8_ ? 8 : spec_.board_h;  // the board as the kernels see it
     mode_ = (W == 8 && H == 8 && !(force && force[0] == '1')) ? 1 : 0;
-    // boards the 8x8 kernels do not cover run on DENSE rows: conv_i2c.cu gets a 3x3 layer's zero padding from the TMA engine's
-    // im2col mode (KZB_NO_I2C=1: padded rows and conv_tc.cu, which multiplies the padding rows as well)
-    {
-        const char* no_i2c = std::getenv("KZB_NO_I2C");
-        i2c_ok_ = !(no_i2c && no_i2c[0] == '1') && W <= 255 && H <= 255;
-        dense_i2c_ = mode_ == 0 && i2c_ok_;
-    }
-    if (mode_ == 1 || dense_i2c_)
-        lay_ = RowLayout{W, H, W, W * H};
-    else
-        lay_ = RowLayout{W, H, W + 1, (W + 1) * (H + 1)};
-    const int boards_per_tile = mode_ == 1 ? 128 / (W * H) : 0;
-    // 8x8: whole 4-board units; the cluster-pair tower kernel pads the batch to an even number of units
-    const int boards_alloc = mode_ == 1 ? round_up(max_batch_, 8) : max_batch_;
-    const char* no_tc8 = std::getenv("KZB_NO_CONV8");
-    const bool allow_tc8 = mode_ == 1 && !(no_tc8 && no_tc8[0] == '1');
+    // DENSE rows, one per square: conv_i2c.cu gets a 3x3 layer's zero padding from the TMA engine's im2col mode
+    lay_ = RowLayout{W, H};
     conv_tc_prepare();
-    conv_tc8_prepare();
-    if (i2c_ok_) conv_i2c_prepare();
-    rows_alloc_ = round_up(boards_alloc * lay_.board_pitch, 128);
-    if (dense_i2c_) {  // whole 256-pixel pair tiles, and whole boards under every one of them
+    conv_i2c_prepare();
+    if (mode_ == 1) {
+        // 8x8: whole 4-board units; the cluster-pair tower kernel pads the batch to an even number of units
+        boards_i2c_ = round_up(max_batch_, 8);  // a multiple of 8 boards: whole 256-pixel tiles
+        rows_alloc_ = boards_i2c_ * 64;
+    } else {  // whole 256-pixel pair tiles, and whole boards under every one of them
         const int pixels = round_up(max_batch_ * W * H, 256);
         boards_i2c_ = (pixels + W * H - 1) / (W * H);
         rows_alloc_ = round_up(std::max(pixels, boards_i2c_ * W * H), 128);
-    } else if (mode_ == 1) {
-        boards_i2c_ = rows_alloc_ / 64;  // boards_alloc is a multiple of 8: whole 256-pixel tiles
     }
     cin_pad_ = round_up(spec_.cin, 64);
     c_pad_ = round_up(C, 64);
@@ -338,18 +326,13 @@ void Net::build_bf16() {
                 st->tmap_bh = make_tmap(st->w_bf16.ptr, 2, dims, strides, half);
             }
         }
-        if (mode_ == 1) {
-            uint64_t dims[4] = {uint64_t(in_stride), uint64_t(W), uint64_t(H), uint64_t(rows_alloc_ / (W * H))};
-            uint64_t strides[3] = {uint64_t(in_stride) * 2, uint64_t(in_stride) * 2 * W, uint64_t(in_stride) * 2 * W * H};
-            uint32_t box[4] = {64, uint32_t(W), uint32_t(H), uint32_t(boards_per_tile)};
-            st->tmap_a = make_tmap(in.ptr, 4, dims, strides, box);
-        } else {
+        if (out_f32) {  // the head convs: 1x1 (net_spec.cpp), conv_tc.cu
+            if (st->taps != 1) throw std::logic_error("internal: conv_tc.cu runs 1x1 convs only");
             uint64_t dims[2] = {uint64_t(in_stride), uint64_t(rows_alloc_)};
             uint64_t strides[1] = {uint64_t(in_stride) * 2};
             uint32_t box[2] = {64, 128};
             st->tmap_a = make_tmap(in.ptr, 2, dims, strides, box);
-        }
-        if ((dense_i2c_ || (mode_ == 1 && i2c_ok_)) && cin_pad % 64 == 0 && n % 32 == 0 && n >= 32 && !out_f32 && (relu_n == 0 || relu_n == n) && out_off == 0) {
+        } else {  // conv_i2c.cu: cin_pad and n are multiples of 64, relu_n is 0 or n, out_off is 0
             st->tmap_i2c = make_tmap_im2col(in.ptr, in_stride, W, H, boards_i2c_, 64, 128, st->taps == 9 ? 1 : 0);
             auto rows_map = [&](void* ptr, int stride) {
                 uint64_t dims[2] = {uint64_t(stride), uint64_t(rows_alloc_)};
@@ -369,26 +352,11 @@ void Net::build_bf16() {
             st->use_i2c = true;
             st->i2c_stages = conv_i2c_pick_stages(n);
         }
-        if (allow_tc8 && st->taps == 9 && n <= 128 && !out_f32) {
-            st->use_i2c = false;  // 8x8 boards, narrow layers: the per-layer 8x8 kernel (it only runs when the whole-tower kernel does not)
-            // (c, x, board, y)-ordered view of the same rows, box (64, 8, 4 boards, 10 ranks incl. halo)
-            uint64_t dims[4] = {uint64_t(in_stride), 8, uint64_t(rows_alloc_ / 64), 8};
-            uint64_t strides[3] = {uint64_t(in_stride) * 2, uint64_t(in_stride) * 2 * 64, uint64_t(in_stride) * 2 * 8};
-            uint32_t box[4] = {64, 8, 4, 10};
-            st->tmap_a8 = make_tmap(in.ptr, 4, dims, strides, box);
-            st->use_tc8 = true;
-            st->tc8_b_slots = conv_tc8_pick_b_slots(n);
-            int c8 = 32;
-            while (c8 < 4 * n) c8 *= 2;
-            st->tc8_tmem_cols = c8;
-        }
         ConvTcParams& p = st->tc;
         p.taps = st->taps;
         p.cin_pad = cin_pad;
         p.kblocks = cin_pad / 64;
         p.n = n;
-        p.mode = mode_;
-        p.boards_per_tile = boards_per_tile;
         p.lay = lay_;
         p.bias = st->bias.as<float>();
         p.relu_n = relu_n;
@@ -459,7 +427,7 @@ void Net::build_bf16() {
     // whole-tower persistent kernel: all 2*depth+1 conv3x3 layers in one launch (tower8k.cu)
     const char* no_t8 = std::getenv("KZB_NO_TOWER8");
     const int units_max = ((max_batch_ + 3) / 4 + 1) & ~1;
-    if (allow_tc8 && c_pad_ <= 128 && !(no_t8 && no_t8[0] == '1') &&
+    if (mode_ == 1 && c_pad_ <= 128 && !(no_t8 && no_t8[0] == '1') &&
         (units_max + num_sms_ - 1) / num_sms_ <= tower8k_max_local_units()) {
         tower8k_prepare();
         tower_layers_ = 1 + 2 * spec_.depth;
@@ -567,8 +535,8 @@ void Net::build_f32() {
     act_bf16_ = false;
     const int W = spec_.board_w, H = spec_.board_h, C = spec_.channels;
     mode_ = -1;
-    lay_ = RowLayout{W, H, W, W * H};
-    rows_alloc_ = max_batch_ * lay_.board_pitch;
+    lay_ = RowLayout{W, H};
+    rows_alloc_ = max_batch_ * W * H;
     cin_pad_ = round_up(spec_.cin, 8);
     c_pad_ = round_up(C, 8);
     cp_pad_ = round_up(spec_.policy_conv1.cout, 8);
@@ -749,24 +717,8 @@ void Net::run_network(int batch, const StepHook& hook) {
         auto& st = convs_[si];
         if (precision_ == 1) {
             ConvTcParams p = st->tc;
-            p.timeline = nullptr;
-            if (st->use_tc8) {
-                if (timeline_step_ == st->name) p.timeline = d_timeline_.as<unsigned long long>();
-                p.num_tiles = (batch + 3) / 4;
-                p.valid_rows = batch * 64;
-                p.stages = st->tc8_b_slots;
-                p.tmem_cols = st->tc8_tmem_cols;
-                launch_conv_tc8(st->tmap_a8, st->tmap_b, p, num_sms_, stream_);
-                if (hook) hook(st->name.c_str());
-                continue;
-            }
-            if (mode_ == 1) {
-                p.num_tiles = (batch + p.boards_per_tile - 1) / p.boards_per_tile;
-                p.valid_rows = batch * lay_.board_pitch;
-            } else {
-                p.valid_rows = batch * lay_.board_pitch;
-                p.num_tiles = (p.valid_rows + 127) / 128;
-            }
+            p.valid_rows = batch * lay_.W * lay_.H;
+            p.num_tiles = (p.valid_rows + 127) / 128;
             if (st->use_i2c) {
                 p.stages = st->i2c_stages;
                 // small batches: split the output channels so that twice as many SM pairs share the layer
@@ -1035,7 +987,7 @@ void Net::profile_staged(bool flush, std::vector<std::string>& names, std::vecto
     require_mapper();
     if (staged_batch_ <= 0) throw std::runtime_error("no staged batch: call kzb_stage_packed first");
     CK(cudaSetDevice(device_));
-    const char* tl_env = std::getenv("KZB_TIMELINE");  // development aid: per-CTA clock stamps of one conv step
+    const char* tl_env = std::getenv("KZB_TIMELINE");  // development aid: per-CTA clock stamps of the tower8 or heads8 step
     if (tl_env && tl_env[0]) {
         timeline_step_ = tl_env;
         d_timeline_.alloc(size_t(num_sms_) * 1024 * 8, true);

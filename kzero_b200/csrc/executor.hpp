@@ -47,14 +47,11 @@ struct ConvStep {
     int taps = 9;
     // bf16 tensor-core form
     CUtensorMap tmap_a{}, tmap_b{}, tmap_bh{};
-    bool use_i2c = false;  // conv_i2c.cu (dense rows, TMA im2col, CTA-pair MMA)
+    bool use_i2c = false;  // conv_i2c.cu (TMA im2col, CTA-pair MMA); otherwise conv_tc.cu (1x1, f32 output)
     int i2c_stages = 0;
     CUtensorMap tmap_out{}, tmap_res{};  // conv_i2c: output / residual rows, box (32 channels, 32 rows), SWIZZLE_64B
     CUtensorMap tmap_i2c{}, tmap_bq{};  // im2col map of the input rows; weight box of n / 4 rows (output channels split in two)
     ConvTcParams tc{};
-    bool use_tc8 = false;  // 8x8-board specialisation (conv_tc8.cu)
-    CUtensorMap tmap_a8{};
-    int tc8_b_slots = 0, tc8_tmem_cols = 0;
     DeviceBuffer w_bf16;  // [n][taps*cin_pad]
     // fp32 form
     ConvF32Params f32{};
@@ -110,14 +107,12 @@ private:
 
     int scalar_count_ = -1, bool_channels_ = -1, bits_stride_ = 0;
     RowLayout lay_{};
-    int mode_ = 0;       // bf16 path: 0 padded rows / 2-D TMA, 1 dense 8x8 / 4-D TMA
+    int mode_ = 0;       // bf16 path, dense rows: 0 row kernels (any board), 1 8x8 boards (tower8k / heads8 where they apply)
     int rows_alloc_ = 0; // multiple of 128
     int cin_pad_ = 0, c_pad_ = 0, cp_pad_ = 0, s1_stride_ = 16, pm_stride_ = 0;
     bool act_bf16_ = true;
     bool embed8_ = false;  // a board smaller than 8x8 embedded in the 8x8 grid of the whole-tower kernel
-    bool i2c_ok_ = true;      // conv_i2c.cu may be used (KZB_NO_I2C=1: never)
-    bool dense_i2c_ = false;  // boards the 8x8 kernels do not cover: dense rows, 3x3 layers on conv_i2c.cu
-    int boards_i2c_ = 0;      // boards covered by the im2col tensor maps (>= every 256-pixel tile of a full batch)
+    int boards_i2c_ = 0;   // boards covered by the im2col tensor maps (>= every 256-pixel tile of a full batch)
 
     DeviceBuffer d_bits_, d_scalars_, d_mv_idx_, d_mv_off_, d_nchw_;
     DeviceBuffer act_in_, act_x_, act_t_, act_h1_, act_s1_, act_pm_, act_att_;

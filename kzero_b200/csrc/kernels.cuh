@@ -1,6 +1,6 @@
 // Device-side parameter blocks and host launchers for the hot path's kernels (sm_100a only).
 //   K2  encode      packed bitboards + scalars -> input planes          (encode.cu)      HBM-bound
-//   K1  conv tower  implicit-GEMM conv3x3/1x1 on tcgen05 + TMA + TMEM   (conv_tc.cu)     tensor-bound
+//   K1  conv tower  implicit-GEMM conv3x3/1x1 on tcgen05 + TMA + TMEM   (tower8k.cu, conv_i2c.cu, conv_tc.cu)  tensor-bound
 //       conv fp32   CUDA-core fp32 implicit GEMM, the <=1e-4 parity mode (conv_fp32.cu)
 //   K3  heads tail  scalar-head FCs, policy gather, masked softmax      (heads.cu)       HBM/latency-bound
 #pragma once
@@ -13,16 +13,10 @@
 
 namespace kzb {
 
-// Row index of square (y, x) of board b inside an activation matrix [rows][channels]:
-//   row = b * board_pitch + y * rank_pitch + x
-// dense  layout: rank_pitch = W,   board_pitch = H*W        (no padding rows)
-// padded layout: rank_pitch = W+1, board_pitch = (H+1)*(W+1): one zero column after every rank and one
-//   zero rank after every board, so every 3x3 tap is a pure row shift dy*rank_pitch+dx that lands on a
-//   zero row whenever it leaves the board.
+// Row index of square sq = y * W + x of board b inside an activation matrix [rows][channels]: every row is a real square
 struct RowLayout {
-    int W, H, rank_pitch, board_pitch;
-    __host__ __device__ int row(int b, int sq) const { return b * board_pitch + (sq / W) * rank_pitch + (sq % W); }
-    __host__ __device__ bool padded() const { return rank_pitch != W; }
+    int W, H;
+    __host__ __device__ int row(int b, int sq) const { return b * W * H + sq; }
 };
 
 // ---------------------------------------------------------------------------------------------- K2
@@ -32,7 +26,7 @@ struct EncodeParams {
     int batch, bits_stride, scalar_count, bool_channels;
     RowLayout lay;
     int c_pad;  // channels per row in the output (>= scalar_count + bool_channels, multiple of 8)
-    void* out;  // [batch*board_pitch][c_pad] bf16 or f32
+    void* out;  // [batch*W*H][c_pad] bf16 or f32
     // optional board symmetry (RandomSymmetryNetwork on the GPU, network/symmetry.rs:41-67): plane square sq of board b is
     // read from square square_src[sym[b]*A + sq] of the record; null = identity
     const uint8_t* sym;
@@ -44,7 +38,7 @@ void launch_encode_nhwc(const EncodeParams& p, bool out_bf16, cudaStream_t s);
 // exact twin of InputMapper::encode_input_full (mapping/mod.rs:40-63): out [batch][Cs+Cb][H*W] f32
 void launch_encode_nchw_f32(const uint8_t* bits, const float* scalars, int batch, int bits_stride, int scalar_count,
                             int bool_channels, int area, float* out, cudaStream_t s);
-// f32 NCHW [batch][C][H*W] -> rows [batch*board_pitch][c_pad] (bf16 or f32), zero pad rows / channels
+// f32 NCHW [batch][C][H*W] -> rows [batch*W*H][c_pad] (bf16 or f32), zero pad channels
 void launch_nchw_to_rows(const float* in, int batch, int channels, RowLayout lay, int c_pad, void* out, bool out_bf16,
                          cudaStream_t s);
 
@@ -71,9 +65,7 @@ struct ConvTcParams {
     int taps;       // 1 or 9
     int kblocks;    // cin_pad / 64
     int cin_pad;
-    int n;     // UMMA N = padded cout, multiple of 16, <= 256
-    int mode;  // 0: rows are a padded linear layout, 2-D TMA; 1: dense 8x8 boards, 4-D TMA box (c,x,y,b)
-    int boards_per_tile;
+    int n;  // UMMA N = padded cout, multiple of 16, <= 256
     RowLayout lay;
     int valid_rows;  // rows >= valid_rows are not stored
     const float* bias;  // [n]
@@ -88,9 +80,8 @@ struct ConvTcParams {
     int tmem_cols;
     int n_split;  // conv_i2c: 1, or 2 = a work item is one 256-pixel tile x one half of the output channels
     int pdl;      // conv_i2c: launched with programmatic stream serialization (set-up and the first weight tiles overlap the previous layer's tail)
-    // development aid: when non-null, each CTA writes 16 clock64() stamps (see conv_tc8.cu) -- KZB_TIMELINE=1
-    unsigned long long* timeline;
 };
+// conv_tc.cu: conv1x1 on dense rows (tmap_a: box (64 channels, 128 rows), tmap_b: weight box (64, p.n))
 void launch_conv_tc(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const ConvTcParams& p, int grid, cudaStream_t s);
 // conv_i2c.cu: conv3x3 / conv1x1 (p.taps) on DENSE rows, activation tiles by TMA im2col, CTA-pair MMA (tmap_bh: weight box of p.n / p.n_split / 2 rows)
 void launch_conv_i2c(const CUtensorMap& tmap_a_im2col, const CUtensorMap& tmap_bh, const CUtensorMap& tmap_out, const CUtensorMap& tmap_res,
@@ -101,14 +92,6 @@ void conv_i2c_prepare();
 size_t conv_tc_smem_bytes(int n, int stages);
 int conv_tc_pick_stages(int n);
 void conv_tc_prepare();  // per-device: opt in to 227 KB dynamic shared memory
-
-// 8x8-board specialisation (conv_tc8.cu): p.num_tiles counts 4-board work units, p.stages is the number
-// of weight-ring slots, tmap_a is the (c, x, board, y)-ordered map with box (64, 8, 4, 10).
-void launch_conv_tc8(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const ConvTcParams& p, int grid,
-                     cudaStream_t s);
-size_t conv_tc8_smem_bytes(int n, int b_slots);
-int conv_tc8_pick_b_slots(int n);
-void conv_tc8_prepare();
 
 // whole-tower persistent kernel for 8x8 boards (tower8k.cu)
 struct TowerLayerDev {

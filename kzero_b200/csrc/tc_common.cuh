@@ -104,17 +104,7 @@ __device__ __forceinline__ void cluster_sync_all() {
 //   [0,14) start address >> 4 | [16,30) LBO >> 4 (unused for swizzled K-major) | [32,46) SBO >> 4
 //   [46,48) version = 1 | [49,52) base offset = 0 | [61,64) layout type: 2 = SWIZZLE_128B
 // 8-row groups are 1024 B apart (SBO), rows inside a group 128 B apart.
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= uint64_t((smem_addr >> 4) & 0x3FFF);
-    d |= uint64_t(1) << 16;
-    d |= uint64_t(1024 >> 4) << 32;
-    d |= uint64_t(1) << 46;
-    d |= uint64_t(2) << 61;
-    return d;
-}
-
-// Same descriptor split into its address-independent upper part and the 14-bit start-address field, so the MMA
+// The descriptor is built as its address-independent upper part OR the 14-bit start-address field, so the MMA
 // issue loop only does one integer add per operand (the issue thread is otherwise the bottleneck: measured
 // ~100 cycles per tcgen05.mma when the full descriptor is rebuilt each time vs 64 cycles of tensor work).
 __device__ __forceinline__ uint64_t umma_desc_sw128_hi() {
@@ -179,7 +169,6 @@ __device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, const void*
                  : "memory");
 }
 __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }

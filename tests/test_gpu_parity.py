@@ -126,18 +126,20 @@ def test_fp32_packed_vs_oracle(game, depth, ch, n):
     _check_packed(values, probs, ref_values, ref_probs, mv_off, FP32_TOL, FP32_TOL)
 
 
-@pytest.mark.parametrize("variant", ["default", "no_heads8", "no_tower8", "no_conv8", "linear", "no_embed8", "no_pdl", "no_conv_split", "no_i2c"])
+@pytest.mark.parametrize("variant", ["default", "no_heads8", "no_tower8", "no_conv8", "linear", "no_embed8", "no_pdl", "no_conv_split"])
 @pytest.mark.parametrize("game,depth,ch,n", [("ataxx-7", 8, 64, 256), ("chess", 16, 128, 64), ("go-9", 4, 64, 40),
-                                              ("chess", 2, 32, 7), ("chess", 3, 64, 130), ("chess", 2, 256, 12)])
+                                              ("chess", 2, 32, 7), ("chess", 3, 64, 130), ("chess", 2, 256, 12),
+                                              ("chess", 2, 32, 9600)])
 def test_bf16_packed_vs_oracle(game, depth, ch, n, variant, monkeypatch):
     """The tensor-core path in all its forms: whole-tower persistent kernel + fused heads kernel (tower8k.cu, heads8.cu, default for 8x8
-    boards), the same tower with per-op head convs + tail kernel (KZB_NO_HEADS8=1), the per-layer 8x8 specialisation (conv_tc8.cu,
-    KZB_NO_TOWER8=1), conv_i2c.cu on 8x8 boards (KZB_NO_CONV8=1, and always for layers wider than 128 channels), and the row kernels of
-    every other board (go; KZB_FORCE_LINEAR=1 / KZB_NO_EMBED8=1 push chess / ataxx there): dense rows with TMA im2col loads and the
-    CTA-pair MMA (conv_i2c.cu), without programmatic dependent launch (KZB_PDL=0), without sharing a tile's output channels between
-    two SM pairs at small batches (KZB_CONV_SPLIT=0), and the padded-row kernel it replaced (KZB_NO_I2C=1: conv_tc.cu).  Boards
-    smaller than 8x8 (ataxx 7x7) are embedded in the 8x8 grid and masked after every layer."""
-    row_variants = ("linear", "no_pdl", "no_conv_split", "no_i2c")  # everything off the 8x8 kernels
+    boards), the same tower with per-op head convs + tail kernel (KZB_NO_HEADS8=1), conv_i2c.cu on 8x8 boards with the fused heads kernel
+    (KZB_NO_TOWER8=1; by default for layers wider than 128 channels, and for chess batch 9600, which has more 4-board units per SM than
+    the whole-tower kernel keeps), no 8x8 conv kernel at all (KZB_NO_TOWER8=1 and KZB_NO_HEADS8=1: conv_i2c.cu on 8x8 boards, per-op
+    head convs + tail kernel), and the row kernels of every other board (go; KZB_FORCE_LINEAR=1 / KZB_NO_EMBED8=1 push chess / ataxx
+    there): dense rows with TMA im2col loads and the CTA-pair MMA (conv_i2c.cu), the head 1x1 convs (conv_tc.cu) and the tail kernel,
+    without programmatic dependent launch (KZB_PDL=0), and without sharing a tile's output channels between two SM pairs at small
+    batches (KZB_CONV_SPLIT=0).  Boards smaller than 8x8 (ataxx 7x7) are embedded in the 8x8 grid and masked after every layer."""
+    row_variants = ("linear", "no_pdl", "no_conv_split")  # everything off the 8x8 kernels
     if variant == "no_embed8":
         if game != "ataxx-7":
             pytest.skip("only boards smaller than 8x8 are embedded")
@@ -148,21 +150,21 @@ def test_bf16_packed_vs_oracle(game, depth, ch, n, variant, monkeypatch):
         pytest.skip("the kernel variants are 8x8 specialisations")
     monkeypatch.setenv("KZB_NO_EMBED8", "1" if variant == "no_embed8" else "0")
     force_linear = "1" if variant in row_variants else "0"
-    monkeypatch.setenv("KZB_NO_I2C", "1" if variant == "no_i2c" else "0")
     monkeypatch.setenv("KZB_PDL", "0" if variant == "no_pdl" else "1")
     monkeypatch.setenv("KZB_CONV_SPLIT", "0" if variant == "no_conv_split" else "1")
     monkeypatch.setenv("KZB_FORCE_LINEAR", force_linear)
-    monkeypatch.setenv("KZB_NO_CONV8", "1" if variant == "no_conv8" else "0")
-    monkeypatch.setenv("KZB_NO_TOWER8", "1" if variant == "no_tower8" else "0")
+    monkeypatch.setenv("KZB_NO_TOWER8", "1" if variant in ("no_tower8", "no_conv8") else "0")
     monkeypatch.setenv("KZB_NO_HEADS8", "1" if variant in ("no_heads8", "no_conv8") else "0")
     spec = netgen.game_spec(game)
     onnx_bytes = netgen.build_onnx(spec, depth, ch, seed=9)
     bits, scalars, mv_idx, mv_off = netgen.synthetic_positions(spec, n, seed=10)
     ref_s, ref_p, ref_values, ref_probs = _oracle_packed(spec, onnx_bytes, bits, scalars, mv_idx, mv_off)
     with B200Network(mapper_for(spec), onnx_bytes, n, precision=PRECISION_BF16) as net:
-        # 8x8 boards, and smaller boards embedded in the 8x8 grid (ataxx 7x7), run on the 8x8 kernels; go-9 on padded rows
+        # 8x8 boards, and smaller boards embedded in the 8x8 grid (ataxx 7x7), run on the 8x8 kernels; go-9 on the row kernels
         on_8x8 = (game == "chess" and force_linear == "0") or (game == "ataxx-7" and variant == "default")
         assert net.info().conv_mode == (1 if on_8x8 else 0)
+        if n > 4 * 16 * 148 and variant == "default":  # 148 SMs: conv_i2c.cu runs the tower layer by layer, then heads8
+            assert net.launches_per_eval() == 2 * depth + 3
         values, probs = net.evaluate_packed(bits, scalars, mv_idx, mv_off)
         planes = _oracle_planes(spec, bits, scalars)
         s, p = net.evaluate_planes(planes)
@@ -357,6 +359,17 @@ def test_errors_match_reference_panics():
     wrong = Mapper((spec.bool_channels, 7, 7), spec.scalar_channels, (spec.policy_size + 1,))
     with pytest.raises(KzbError, match="policy shape"):  # common.rs:182
         B200Network(wrong, onnx_bytes, 8)
+
+
+def test_bf16_rejects_boards_wider_than_255_squares():
+    """The bf16 row kernels take boards of up to 255 x 255 squares: a larger board is refused when the network is created, with a
+    message that points to the fp32 path, which does create it."""
+    spec = netgen.game_spec("go-256")
+    onnx_bytes = netgen.build_onnx(spec, 1, 8, seed=18)
+    with pytest.raises(KzbError, match="precision=fp32"):
+        B200Network(mapper_for(spec), onnx_bytes, 1, precision=PRECISION_BF16)
+    with B200Network(mapper_for(spec), onnx_bytes, 1, precision=PRECISION_FP32) as net:
+        assert net.info().conv_mode == -1
 
 
 @pytest.mark.parametrize("game", ["chess", "ataxx-7", "go-9"])
