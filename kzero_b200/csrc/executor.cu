@@ -596,6 +596,23 @@ void Net::build_f32() {
     }
 }
 
+// offsets inside the contiguous input block [mv_off | scalars | bits | mv_idx] -> a single H2D copy per batch
+struct InBlock {
+    size_t off_scalars, off_bits, off_idx;
+};
+static InBlock in_block(int max_batch, int scalar_count, int bits_stride) {
+    InBlock b;
+    b.off_scalars = align16(size_t(max_batch + 1) * 4);
+    b.off_bits = b.off_scalars + align16(size_t(max_batch) * scalar_count * 4);
+    b.off_idx = b.off_bits + align16(size_t(max_batch) * bits_stride);
+    return b;
+}
+// offsets inside the contiguous output block [err word (16 B) | values | probs] -> a single D2H copy per batch
+struct OutBlock {
+    size_t off_values, off_probs;
+};
+static OutBlock out_block(int max_batch) { return {16, 16 + align16(size_t(max_batch) * 5 * 4)}; }
+
 void Net::bind_mapper(int scalar_count, int bool_channels, int h, int w, int policy_len) {
     // twin of check_graph_shapes, rust/kz-core/src/network/common.rs:165-198
     if (scalar_count < 0 || bool_channels < 0) throw std::runtime_error("negative channel count");
@@ -610,13 +627,10 @@ void Net::bind_mapper(int scalar_count, int bool_channels, int h, int w, int pol
     bool_channels_ = bool_channels;
     bits_stride_ = (bool_channels * h * w + 7) / 8;
     mv_cap_ = size_t(max_batch_) * spec_.policy_len;
-    // one contiguous input block [mv_off | scalars | bits | mv_idx] -> a single H2D copy per batch
-    size_t in_bytes = align16(size_t(max_batch_ + 1) * 4) + align16(size_t(max_batch_) * scalar_count_ * 4) +
-                      align16(size_t(max_batch_) * bits_stride_) + mv_cap_ * 4;
+    const size_t in_bytes = in_block(max_batch_, scalar_count_, bits_stride_).off_idx + mv_cap_ * 4;
     d_mv_off_.alloc(in_bytes, true);
     h_in_.alloc(in_bytes);
-    // one contiguous output block [err(16) | values | probs] -> a single D2H copy per batch
-    size_t out_bytes = 16 + align16(size_t(max_batch_) * 5 * 4) + mv_cap_ * 4;
+    const size_t out_bytes = out_block(max_batch_).off_probs + mv_cap_ * 4;
     d_err_.alloc(out_bytes, true);
     h_out_.alloc(out_bytes);
 }
@@ -628,18 +642,6 @@ void Net::check_batch(int batch) const {
 }
 void Net::require_mapper() const {
     if (scalar_count_ < 0) throw std::runtime_error("kzb_net_bind_mapper must be called before packed evaluation");
-}
-
-// offsets inside the contiguous input/output blocks
-struct InBlock {
-    size_t off_scalars, off_bits, off_idx;
-};
-static InBlock in_block(int max_batch, int scalar_count, int bits_stride) {
-    InBlock b;
-    b.off_scalars = align16(size_t(max_batch + 1) * 4);
-    b.off_bits = b.off_scalars + align16(size_t(max_batch) * scalar_count * 4);
-    b.off_idx = b.off_bits + align16(size_t(max_batch) * bits_stride);
-    return b;
 }
 
 void Net::upload_packed(const uint8_t* bits, const float* scalars, int batch, const uint32_t* mv_idx, const uint32_t* mv_off) {
@@ -737,31 +739,41 @@ void Net::run_network(int batch, const StepHook& hook) {
     }
 }
 
+HeadOutputs Net::head_outputs(int batch, bool packed, bool to_host) const {
+    HeadOutputs o{};
+    o.batch = batch;
+    o.policy_len = spec_.policy_len;
+    o.packed = packed ? 1 : 0;
+    o.out_scalars = d_out_scalars_.as<float>();
+    o.out_logits = d_out_logits_.as<float>();
+    if (packed) {
+        const InBlock ib = in_block(max_batch_, scalar_count_, bits_stride_);
+        const OutBlock ob = out_block(max_batch_);
+        o.mv_off = d_mv_off_.as<uint32_t>();
+        o.mv_idx = reinterpret_cast<const uint32_t*>(d_mv_off_.as<uint8_t>() + ib.off_idx);
+        o.sym = cur_sym_;
+        o.policy_map = d_sym_policy_.as<int32_t>();
+        // results either stay in HBM (staged timing) or are written straight into the pinned, device-mapped host block
+        // (kzb_eval_packed: no separate D2H copies, the posted PCIe writes overlap the kernel)
+        uint8_t* out = to_host ? h_out_.as<uint8_t>() : d_err_.as<uint8_t>();
+        o.err_flag = reinterpret_cast<int*>(out);
+        o.out_values = reinterpret_cast<float*>(out + ob.off_values);
+        o.out_probs = reinterpret_cast<float*>(out + ob.off_probs);
+    }
+    return o;
+}
+
 void Net::run_tail(int batch, bool packed, const StepHook& hook, bool to_host) {
+    const HeadOutputs out = head_outputs(batch, packed, to_host);
     if (use_heads8_ && precision_ == 1) {
         Heads8Params p = heads_params_;
+        p.out = out;
         p.num_tiles = (batch + 1) / 2;
-        p.batch = batch;
         p.fc1_t = d_fc1_t_.as<float>();
         p.fc1_b = d_fc1_b_.as<float>();
         p.fc2_w = d_fc2_w_.as<float>();
         p.fc2_b = d_fc2_b_.as<float>();
         p.policy_src = d_policy_src_.as<int32_t>();
-        p.policy_len = spec_.policy_len;
-        p.packed = packed ? 1 : 0;
-        p.out_scalars = d_out_scalars_.as<float>();
-        p.out_logits = d_out_logits_.as<float>();
-        if (packed) {
-            InBlock ib = in_block(max_batch_, scalar_count_, bits_stride_);
-            p.mv_off = d_mv_off_.as<uint32_t>();
-            p.mv_idx = reinterpret_cast<const uint32_t*>(d_mv_off_.as<uint8_t>() + ib.off_idx);
-            p.sym = cur_sym_;
-            p.policy_map = d_sym_policy_.as<int32_t>();
-            uint8_t* out = to_host ? h_out_.as<uint8_t>() : d_err_.as<uint8_t>();
-            p.err_flag = reinterpret_cast<int*>(out);
-            p.out_values = reinterpret_cast<float*>(out + 16);
-            p.out_probs = reinterpret_cast<float*>(out + 16 + align16(size_t(max_batch_) * 5 * 4));
-        }
         p.timeline = timeline_step_ == "heads8" ? d_timeline_.as<unsigned long long>() : nullptr;
         p.pdl = (use_tower8k_ && tower_params_.pdl) ? 1 : 0;  // only behind the tower kernel, which triggers the dependent launch
         launch_heads8(heads_maps_, p, num_sms_, stream_);
@@ -769,7 +781,7 @@ void Net::run_tail(int batch, bool packed, const StepHook& hook, bool to_host) {
         return;
     }
     HeadsTailParams p{};
-    p.batch = batch;
+    p.out = out;
     p.lay = lay_;
     p.s1 = act_s1_.as<float>();
     p.s1_stride = s1_stride_;
@@ -784,28 +796,12 @@ void Net::run_tail(int batch, bool packed, const StepHook& hook, bool to_host) {
     p.extra_w = spec_.has_extra ? d_extra_w_.as<float>() : nullptr;
     p.extra_b = spec_.has_extra ? spec_.extra_fc.b[0] : 0.0f;
     p.policy_src = spec_.has_attention ? nullptr : d_policy_src_.as<int32_t>();
-    p.policy_len = spec_.policy_len;
     p.att = act_att_.as<float>();
     p.att_stride = att_stride_;
     p.att_q = spec_.att_q;
     p.att_div = spec_.att_div;
     p.att_entries = spec_.has_attention ? d_att_entries_.as<AttEntryDev>() : nullptr;
-    p.out_scalars = d_out_scalars_.as<float>();
-    p.out_logits = d_out_logits_.as<float>();
-    if (packed) {
-        InBlock ib = in_block(max_batch_, scalar_count_, bits_stride_);
-        p.mv_off = d_mv_off_.as<uint32_t>();
-        p.mv_idx = reinterpret_cast<const uint32_t*>(d_mv_off_.as<uint8_t>() + ib.off_idx);
-        p.sym = cur_sym_;
-        p.policy_map = d_sym_policy_.as<int32_t>();
-        // results either stay in HBM (staged timing) or are written straight into the pinned, device-mapped host block
-        // (kzb_eval_packed: no separate D2H copies, the posted PCIe writes overlap the kernel)
-        uint8_t* out = to_host ? h_out_.as<uint8_t>() : d_err_.as<uint8_t>();
-        p.err_flag = reinterpret_cast<int*>(out);
-        p.out_values = reinterpret_cast<float*>(out + 16);
-        p.out_probs = reinterpret_cast<float*>(out + 16 + align16(size_t(max_batch_) * 5 * 4));
-    }
-    launch_heads_tail(p, packed, stream_);
+    launch_heads_tail(p, stream_);
     if (hook) hook("heads_tail");
 }
 
@@ -907,7 +903,6 @@ void Net::eval_packed(const uint8_t* bits, const float* scalars, int batch, cons
         run_network(batch, nullptr);
         run_tail(batch, true, nullptr, /*to_host=*/true);
     }
-    const size_t probs_off = 16 + align16(size_t(max_batch_) * 5 * 4);
     if (trace) t2 = clk::now();
     if (blocking_sync_) {  // the calling thread sleeps while the GPU works (self-play: executor threads share cores with generators)
         if (!done_event_) CK(cudaEventCreateWithFlags(&done_event_, cudaEventBlockingSync | cudaEventDisableTiming));
@@ -922,8 +917,9 @@ void Net::eval_packed(const uint8_t* bits, const float* scalars, int batch, cons
     if (err != 0)
         throw std::runtime_error("Softmax input sum must be strictly positive (board " + std::to_string(err - 1) +
                                  "): the network produced NaN/inf logits");
-    std::memcpy(out_values, h_out_.as<uint8_t>() + 16, size_t(batch) * 5 * 4);
-    if (staged_moves_) std::memcpy(out_policy, h_out_.as<uint8_t>() + probs_off, staged_moves_ * 4);
+    const OutBlock ob = out_block(max_batch_);
+    std::memcpy(out_values, h_out_.as<uint8_t>() + ob.off_values, size_t(batch) * 5 * 4);
+    if (staged_moves_) std::memcpy(out_policy, h_out_.as<uint8_t>() + ob.off_probs, staged_moves_ * 4);
     if (trace) {
         t4 = clk::now();
         auto us = [](clk::time_point a, clk::time_point b) { return std::chrono::duration<double, std::micro>(b - a).count(); };

@@ -97,6 +97,7 @@ private:
     void upload_packed(const uint8_t* bits, const float* scalars, int batch, const uint32_t* mv_idx, const uint32_t* mv_off);
     void run_encode(int batch, const StepHook& hook);
     void run_network(int batch, const StepHook& hook);
+    HeadOutputs head_outputs(int batch, bool packed, bool to_host) const;
     void run_tail(int batch, bool packed, const StepHook& hook, bool to_host = false);
     void flush_l2();
 
@@ -118,7 +119,7 @@ private:
     DeviceBuffer act_in_, act_x_, act_t_, act_h1_, act_s1_, act_pm_, act_att_;
     int att_stride_ = 0;
     DeviceBuffer d_fc1_t_, d_fc1_b_, d_fc2_w_, d_fc2_b_, d_extra_w_, d_policy_src_, d_att_entries_;
-    DeviceBuffer d_out_scalars_, d_out_logits_, d_out_values_, d_out_probs_, d_err_;
+    DeviceBuffer d_out_scalars_, d_out_logits_, d_err_;
     DeviceBuffer d_flush_, d_timeline_;
     std::string timeline_step_;
     PinnedBuffer h_in_, h_out_;

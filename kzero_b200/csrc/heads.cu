@@ -8,9 +8,9 @@
 //   - and, in packed mode, the CPU-side decode_output (rust/kz-core/src/network/common.rs:16-100):
 //     value = tanh(s0), wdl = softmax(s1..3), moves_left = s4, policy = softmax over the LEGAL moves only
 //     (gathered by the host-supplied move_to_index list), so only n_legal probabilities per position cross
-//     PCIe instead of the full [B, P] logit matrix.
+//     PCIe instead of the full [B, P] logit matrix.  The decode itself is shared with heads8.cu (head_decode.cuh).
 // HBM/latency-bound: algorithmic bytes per position = hc*A*4 + (n_legal or P)*4 read, (5 + n_legal or P)*4 written.
-#include "kernels.cuh"
+#include "head_decode.cuh"
 
 namespace kzb {
 namespace {
@@ -18,23 +18,12 @@ namespace {
 constexpr int kWarpsPerBlock = 4;
 constexpr int kMaxHiddenPerLane = 4;  // hs <= 128
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-
 template <bool PACKED, int HPL>  // HPL = hidden units per lane = ceil(hs / 32)
 __global__ void __launch_bounds__(kWarpsPerBlock * 32) heads_tail_kernel(HeadsTailParams p) {
     extern __shared__ float smem[];
     const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
     const int b = blockIdx.x * kWarpsPerBlock + warp;
-    if (b >= p.batch) return;  // whole warp exits together, no block-level sync below
+    if (b >= p.out.batch) return;  // whole warp exits together, no block-level sync below
 
     const int area = p.lay.W * p.lay.H;
     const int n_in = p.hc * area;
@@ -109,96 +98,23 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) heads_tail_kernel(HeadsTa
     };
 
     if (!PACKED) {
-        if (lane < 5) p.out_scalars[size_t(b) * 5 + lane] = sc[lane];
-        for (int i = lane; i < p.policy_len; i += 32) p.out_logits[size_t(b) * p.policy_len + i] = logit(i);
+        if (lane < 5) p.out.out_scalars[size_t(b) * 5 + lane] = sc[lane];
+        for (int i = lane; i < p.out.policy_len; i += 32) p.out.out_logits[size_t(b) * p.out.policy_len + i] = logit(i);
         return;
     }
-
-    // decode_output, common.rs:59-74
-    if (lane == 0) {
-        float* ov = p.out_values + size_t(b) * 5;
-        ov[0] = tanhf(sc[0]);
-        float mx = fmaxf(sc[1], fmaxf(sc[2], sc[3]));
-        float e0 = expf(sc[1] - mx), e1 = expf(sc[2] - mx), e2 = expf(sc[3] - mx);
-        float sum = (e0 + e1) + e2;
-        if (!(sum > 0.0f)) *reinterpret_cast<volatile int*>(p.err_flag) = 1 + b;
-        ov[1] = e0 / sum;
-        ov[2] = e1 / sum;
-        ov[3] = e2 / sum;
-        ov[4] = sc[4];
-    }
-    // masked softmax over the legal moves only, common.rs:76-86 + softmax_in_place :102-114
-    const uint32_t o0 = p.mv_off[b], o1 = p.mv_off[b + 1];
-    const int n = int(o1 - o0);
-    if (n <= 0) return;  // terminal board: empty policy (common.rs:77)
-    const int32_t* pmap = p.sym ? p.policy_map + size_t(p.sym[b]) * p.policy_len : nullptr;
-    constexpr int kRegMoves = 12;  // up to 384 legal moves stay in registers (chess <= 218, go-19 <= 362)
-    if (n <= 32 * kRegMoves) {
-        float l[kRegMoves];
-        float mx = -INFINITY;
-#pragma unroll
-        for (int k = 0; k < kRegMoves; k++) {
-            const int j = lane + 32 * k;
-            l[k] = -INFINITY;
-            if (j < n) {
-                uint32_t idx = p.mv_idx[o0 + j];
-                if (pmap && idx < uint32_t(p.policy_len)) idx = uint32_t(pmap[idx]);
-                l[k] = idx < uint32_t(p.policy_len) ? logit(int(idx)) : NAN;
-                mx = fmaxf(mx, l[k]);
-            }
-        }
-        mx = warp_max(mx);
-        float sum = 0.0f;
-#pragma unroll
-        for (int k = 0; k < kRegMoves; k++) {
-            const int j = lane + 32 * k;
-            if (j < n) {
-                l[k] = expf(l[k] - mx);
-                sum += l[k];
-            }
-        }
-        sum = warp_sum(sum);
-        if (!(sum > 0.0f)) {  // NaN logits: the reference panics here (common.rs:110)
-            if (lane == 0) *reinterpret_cast<volatile int*>(p.err_flag) = 1 + b;
-        }
-#pragma unroll
-        for (int k = 0; k < kRegMoves; k++) {
-            const int j = lane + 32 * k;
-            if (j < n) p.out_probs[o0 + j] = l[k] / sum;
-        }
-        return;
-    }
-    float mx = -INFINITY;
-    for (int j = lane; j < n; j += 32) {
-        uint32_t idx = p.mv_idx[o0 + j];
-        if (pmap && idx < uint32_t(p.policy_len)) idx = uint32_t(pmap[idx]);
-        float l = idx < uint32_t(p.policy_len) ? logit(int(idx)) : NAN;
-        p.out_probs[o0 + j] = l;  // stage the gathered logit; each lane re-reads only its own entries
-        mx = fmaxf(mx, l);
-    }
-    mx = warp_max(mx);
-    float sum = 0.0f;
-    for (int j = lane; j < n; j += 32) {
-        float e = expf(p.out_probs[o0 + j] - mx);
-        p.out_probs[o0 + j] = e;
-        sum += e;
-    }
-    sum = warp_sum(sum);
-    if (!(sum > 0.0f)) {
-        if (lane == 0) *reinterpret_cast<volatile int*>(p.err_flag) = 1 + b;
-    }
-    for (int j = lane; j < n; j += 32) p.out_probs[o0 + j] /= sum;
+    if (lane == 0) decode_values(sc, b, p.out);
+    legal_softmax<12>(p.out, b, lane, logit);  // up to 384 legal moves stay in registers (chess <= 218, go-19 <= 362)
 }
 
 }  // namespace
 
-void launch_heads_tail(const HeadsTailParams& p, bool packed, cudaStream_t s) {
-    if (p.batch <= 0) return;
-    int blocks = (p.batch + kWarpsPerBlock - 1) / kWarpsPerBlock;
+void launch_heads_tail(const HeadsTailParams& p, cudaStream_t s) {
+    if (p.out.batch <= 0) return;
+    int blocks = (p.out.batch + kWarpsPerBlock - 1) / kWarpsPerBlock;
     size_t smem = size_t(kWarpsPerBlock) * p.hc * p.lay.W * p.lay.H * sizeof(float);
     const int hpl = (p.hs + 31) / 32;
 #define KZB_TAIL(PACKED, HPL) heads_tail_kernel<PACKED, HPL><<<blocks, kWarpsPerBlock * 32, smem, s>>>(p)
-    if (packed) {
+    if (p.out.packed) {
         if (hpl <= 1) KZB_TAIL(true, 1);
         else if (hpl == 2) KZB_TAIL(true, 2);
         else KZB_TAIL(true, 4);

@@ -15,11 +15,11 @@
 //   epi2  D2 + b2 -> fp32 logits L[board][pc*64 + sq] in shared memory (aliases H)
 //   tail  per board: fc1 + relu + fc2 (post_act.py:17-19); then either
 //           packed: value = tanh, wdl = softmax, legal-move gather through policy_src + softmax over the legal moves
-//                   only (rust/kz-core/src/network/common.rs:59-86,102-114), or
+//                   only (rust/kz-core/src/network/common.rs:59-86,102-114; shared with heads.cu in head_decode.cuh), or
 //           planes: raw scalars + all P logits (twin of CudaExecutor::evaluate, network/cudnn.rs:73)
 // MMA1/MMA3 of tile t+1 overlap epi2 + tail of tile t (D1/Ds are free once epi1 has drained them).
 // Warp roles: warp 0 TMA producer, warp 1 MMA issuer (+TMEM owner), warps 2..5 epilogue/tail (thread = tile row).
-#include "kernels.cuh"
+#include "head_decode.cuh"
 #include "tc_common.cuh"
 
 namespace kzb {
@@ -79,16 +79,6 @@ __device__ __forceinline__ SmemH carve_h(uint8_t* base, const Heads8Params& p) {
     return s;
 }
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
 
 __global__ void __launch_bounds__(kThreads, 1)
@@ -298,7 +288,7 @@ __global__ void __launch_bounds__(kThreads, 1)
 
             // ---- tail: two warps per board; the even one runs the scalar head, both split the policy work
             const int b = tile * 2 + (quarter >> 1);
-            if (b >= p.batch) continue;  // whole warps skip together; epi_bar at the loop top keeps the count (all 4 warps loop)
+            if (b >= p.out.batch) continue;  // whole warps skip together; epi_bar at the loop top keeps the count (all 4 warps loop)
             const int wb = quarter >> 1, sub = quarter & 1;
             const float* S = sm.s + wb * n_in;
             const float* Lb = L + size_t(wb) * p.pc * 64;
@@ -325,89 +315,21 @@ __global__ void __launch_bounds__(kThreads, 1)
                     float part = lane < p.hs ? p.fc2_w[k * p.hs + lane] * h : 0.0f;
                     sc[k] = warp_sum(part) + p.fc2_b[k];
                 }
-                if (!p.packed) {
-                    if (lane < 5) p.out_scalars[size_t(b) * 5 + lane] = sc[lane];
-                } else if (lane == 0) {  // decode_output, common.rs:59-74
-                    float* ov = p.out_values + size_t(b) * 5;
-                    ov[0] = tanhf(sc[0]);
-                    float mx = fmaxf(sc[1], fmaxf(sc[2], sc[3]));
-                    float e0 = expf(sc[1] - mx), e1 = expf(sc[2] - mx), e2 = expf(sc[3] - mx);
-                    float sum = (e0 + e1) + e2;
-                    if (!(sum > 0.0f)) *reinterpret_cast<volatile int*>(p.err_flag) = 1 + b;
-                    ov[1] = e0 / sum;
-                    ov[2] = e1 / sum;
-                    ov[3] = e2 / sum;
-                    ov[4] = sc[4];
+                if (!p.out.packed) {
+                    if (lane < 5) p.out.out_scalars[size_t(b) * 5 + lane] = sc[lane];
+                } else if (lane == 0) {
+                    decode_values(sc, b, p.out);
                 }
             }
             auto logit = [&](int i) -> float {
                 const int src = p.policy_src[i];
                 return src >= 0 ? Lb[src] : 0.0f;  // -1: constant zero column
             };
-            if (!p.packed) {
-                for (int i = sub * 32 + lane; i < p.policy_len; i += 64) p.out_logits[size_t(b) * p.policy_len + i] = logit(i);
+            if (!p.out.packed) {
+                for (int i = sub * 32 + lane; i < p.out.policy_len; i += 64) p.out.out_logits[size_t(b) * p.out.policy_len + i] = logit(i);
                 continue;
             }
-            if (sub != 1) continue;
-            // masked softmax over the legal moves only, common.rs:76-86 + softmax_in_place :102-114
-            const uint32_t o0 = p.mv_off[b], o1 = p.mv_off[b + 1];
-            const int n = int(o1 - o0);
-            if (n <= 0) continue;  // terminal board: empty policy (common.rs:77)
-            const int32_t* pmap = p.sym ? p.policy_map + size_t(p.sym[b]) * p.policy_len : nullptr;
-            constexpr int kRegMoves = 8;  // up to 256 legal moves in registers (chess <= 218)
-            if (n <= 32 * kRegMoves) {
-                float l[kRegMoves];
-                float mx = -INFINITY;
-#pragma unroll
-                for (int k = 0; k < kRegMoves; k++) {
-                    const int j = lane + 32 * k;
-                    l[k] = -INFINITY;
-                    if (j < n) {
-                        uint32_t idx = p.mv_idx[o0 + j];
-                        if (pmap && idx < uint32_t(p.policy_len)) idx = uint32_t(pmap[idx]);
-                        l[k] = idx < uint32_t(p.policy_len) ? logit(int(idx)) : NAN;
-                        mx = fmaxf(mx, l[k]);
-                    }
-                }
-                mx = warp_max(mx);
-                float sum = 0.0f;
-#pragma unroll
-                for (int k = 0; k < kRegMoves; k++) {
-                    const int j = lane + 32 * k;
-                    if (j < n) {
-                        l[k] = expf(l[k] - mx);
-                        sum += l[k];
-                    }
-                }
-                sum = warp_sum(sum);
-                if (!(sum > 0.0f) && lane == 0) *reinterpret_cast<volatile int*>(p.err_flag) = 1 + b;  // common.rs:110
-#pragma unroll
-                for (int k = 0; k < kRegMoves; k++) {
-                    const int j = lane + 32 * k;
-                    if (j < n) p.out_probs[o0 + j] = l[k] / sum;
-                }
-            } else {
-                float mx = -INFINITY;
-                for (int j = lane; j < n; j += 32) {
-                    uint32_t idx = p.mv_idx[o0 + j];
-                        if (pmap && idx < uint32_t(p.policy_len)) idx = uint32_t(pmap[idx]);
-                    mx = fmaxf(mx, idx < uint32_t(p.policy_len) ? logit(int(idx)) : NAN);
-                }
-                mx = warp_max(mx);
-                float sum = 0.0f;
-                for (int j = lane; j < n; j += 32) {
-                    uint32_t idx = p.mv_idx[o0 + j];
-                        if (pmap && idx < uint32_t(p.policy_len)) idx = uint32_t(pmap[idx]);
-                    sum += expf((idx < uint32_t(p.policy_len) ? logit(int(idx)) : NAN) - mx);
-                }
-                sum = warp_sum(sum);
-                if (!(sum > 0.0f) && lane == 0) *reinterpret_cast<volatile int*>(p.err_flag) = 1 + b;
-                for (int j = lane; j < n; j += 32) {
-                    uint32_t idx = p.mv_idx[o0 + j];
-                        if (pmap && idx < uint32_t(p.policy_len)) idx = uint32_t(pmap[idx]);
-                    p.out_probs[o0 + j] = expf((idx < uint32_t(p.policy_len) ? logit(int(idx)) : NAN) - mx) / sum;
-                }
-            }
+            if (sub == 1) legal_softmax<8>(p.out, b, lane, logit);  // up to 256 legal moves in registers (chess <= 218)
         }
     }
 

@@ -2,7 +2,7 @@
 //   K2  encode      packed bitboards + scalars -> input planes          (encode.cu)      HBM-bound
 //   K1  conv tower  implicit-GEMM conv3x3/1x1 on tcgen05 + TMA + TMEM   (tower8k.cu, conv_i2c.cu, conv_tc.cu)  tensor-bound
 //       conv fp32   CUDA-core fp32 implicit GEMM, the <=1e-4 parity mode (conv_fp32.cu)
-//   K3  heads tail  scalar-head FCs, policy gather, masked softmax      (heads.cu)       HBM/latency-bound
+//   K3  heads tail  scalar-head FCs, policy gather, masked softmax      (heads.cu, decode: head_decode.cuh)  HBM/latency-bound
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -151,8 +151,26 @@ void launch_nchw_to_kc(const float* in, int batch, int channels, int rec_w, int 
 struct AttEntryDev {  // same layout as NetSpec::AttEntry
     int32_t a_chan, a_stride, a_sq, b_chan, b_stride, b_sq;
 };
+// What a head kernel writes for one batch: the raw scalars and logits (planes mode), or their decode (packed mode, head_decode.cuh)
+struct HeadOutputs {
+    int batch, policy_len;
+    int packed;
+    // planes mode (twin of CudaExecutor::evaluate, network/cudnn.rs:73)
+    float* out_scalars;  // [batch][5] raw
+    float* out_logits;   // [batch][P]
+    // packed mode (fused decode_output, network/common.rs:16-114)
+    const uint32_t* mv_idx;  // legal moves' policy indices, CSR
+    const uint32_t* mv_off;  // [batch+1]
+    // optional symmetry: legal index i of board b is looked up at policy_map[sym[b]*P + i] (unmap_eval, symmetry.rs:126-148)
+    const uint8_t* sym;
+    const int32_t* policy_map;
+    float* out_values;  // [batch][5]: tanh(v), softmax(wdl), moves_left
+    float* out_probs;   // CSR-aligned with mv_idx
+    int* err_flag;      // set to 1+board (any failing board) when a softmax sum is not > 0 (common.rs:110); may be host memory
+};
+
 struct HeadsTailParams {
-    int batch;
+    HeadOutputs out;
     RowLayout lay;
     const float* s1;  // [rows][s1_stride]: ch 0..hc-1 relu(scalar conv), ch hc = extra policy conv (no relu)
     int s1_stride, hc;
@@ -166,26 +184,13 @@ struct HeadsTailParams {
     const float* extra_w;  // [A] or null
     float extra_b;
     const int32_t* policy_src;  // [P]; null for the attention head
-    int policy_len;
     // attention policy head (post_act.py:115-141): logit[i] = dot_q(E[a.sq][a.chan + q*a.stride], E[b.sq][b.chan + q*b.stride]) / att_div
     const float* att;  // [rows][att_stride]: concatenated outputs of the head's 1x1 convs
     int att_stride, att_q;
     float att_div;
     const AttEntryDev* att_entries;  // [P] or null
-    // planes mode (twin of CudaExecutor::evaluate, network/cudnn.rs:73)
-    float* out_scalars;  // [batch][5] raw
-    float* out_logits;   // [batch][P]
-    // packed mode (fused decode_output, network/common.rs:16-100)
-    const uint32_t* mv_idx;
-    const uint32_t* mv_off;  // [batch+1]
-    // optional symmetry: legal index i of board b is looked up at policy_map[sym[b]*P + i] (unmap_eval, symmetry.rs:126-148)
-    const uint8_t* sym;
-    const int32_t* policy_map;
-    float* out_values;       // [batch][5]: tanh(v), softmax(wdl), moves_left
-    float* out_probs;        // CSR-aligned with mv_idx
-    int* err_flag;           // set to 1+board (any failing board) when a softmax sum is not > 0 (common.rs:110); may be host memory
 };
-void launch_heads_tail(const HeadsTailParams& p, bool packed, cudaStream_t s);
+void launch_heads_tail(const HeadsTailParams& p, cudaStream_t s);
 
 // ---------------------------------------------------------------------------------------------- K1' + K3 fused (heads8.cu)
 struct Heads8Maps {
@@ -195,8 +200,8 @@ struct Heads8Maps {
     CUtensorMap ws;  // scalar conv  [16][c_pad], box (64, 16)
 };
 struct Heads8Params {
+    HeadOutputs out;
     int num_tiles;  // 128-row tiles = pairs of 8x8 boards
-    int batch;
     int kblocks;    // c_pad / 64
     int n1, n2;     // padded output channels of policy conv1 (multiple of 64) / conv2 (multiple of 16)
     int pc;         // real output channels of policy conv2
@@ -207,17 +212,6 @@ struct Heads8Params {
     const float* fc2_w;         // [5][hs]
     const float* fc2_b;         // [5]
     const int32_t* policy_src;  // [P]: pc*64 + sq, or -1 for a constant-zero logit
-    int policy_len;
-    int packed;
-    const uint32_t* mv_idx;
-    const uint32_t* mv_off;
-    const uint8_t* sym;         // optional symmetry, as in HeadsTailParams
-    const int32_t* policy_map;
-    float* out_values;
-    float* out_probs;
-    int* err_flag;
-    float* out_scalars;
-    float* out_logits;
     int pdl;  // launched with programmatic stream serialization: set-up and the resident weights' loads overlap the tower's tail
     unsigned long long* timeline;  // development aid (KZB_TIMELINE=heads8): per-CTA clock64() stamps
 };

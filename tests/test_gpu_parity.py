@@ -194,6 +194,27 @@ def test_attention_head_vs_oracle(depth, ch, q, n, precision, tol_logit, tol_v, 
     _check_packed(values, probs, ref_values, ref_probs, mv_off, tol_v, tol_p)
 
 
+@pytest.mark.parametrize("path", ["heads8", "tail", "fp32", "attention"])
+def test_long_legal_move_lists_vs_oracle(path, monkeypatch):
+    """Legal-move lists longer than real positions have, so that every form of the masked softmax (head_decode.cuh) runs: up to
+    256 moves (registers in both kernels), 257..384 (registers in the tail kernel, the long-list form in heads8) and more than 384
+    (the long-list form in both).  On heads8 (bf16 default), the tail kernel (bf16 with KZB_NO_HEADS8=1, and fp32) and the tail
+    kernel's attention logits (chess-att)."""
+    monkeypatch.setenv("KZB_NO_HEADS8", "1" if path == "tail" else "0")
+    spec = netgen.game_spec("chess-att" if path == "attention" else "chess")
+    precision = PRECISION_FP32 if path == "fp32" else PRECISION_BF16
+    onnx_bytes = netgen.build_onnx(spec, 2, 32, seed=23)
+    bits, scalars, mv_idx, mv_off = netgen.synthetic_positions(spec, 24, seed=42, min_moves=200, max_moves=600)
+    n_moves = np.diff(mv_off)
+    assert (n_moves <= 256).any() and ((n_moves > 256) & (n_moves <= 384)).any() and (n_moves > 384).any()
+    _, _, ref_values, ref_probs = _oracle_packed(spec, onnx_bytes, bits, scalars, mv_idx, mv_off)
+    with B200Network(mapper_for(spec), onnx_bytes, 24, precision=precision) as net:
+        assert (net.launches_per_eval() == 3) == (path == "heads8")  # encode, tower8k, heads8
+        values, probs = net.evaluate_packed(bits, scalars, mv_idx, mv_off)
+    tol_v, tol_p = (FP32_TOL, FP32_TOL) if precision == PRECISION_FP32 else (5e-2, 1e-2)
+    _check_packed(values, probs, ref_values, ref_probs, mv_off, tol_v, tol_p)
+
+
 @pytest.mark.parametrize("n", [887, 888, 1024, 1036, 1184, 1185])
 def test_bf16_balanced_units_match_uniform_units(n, monkeypatch):
     """tower8k's balanced board assignment (every SM owns 6..8 boards as two units of 4 / 3 boards, batches 888..1184)
