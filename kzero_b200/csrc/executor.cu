@@ -154,6 +154,7 @@ Net::Net(int device, NetSpec spec, int max_batch, int precision)
     if (const char* ng = std::getenv("KZB_NO_GRAPH")) use_graph_ = ng[0] != '1';
     if (const char* tr = std::getenv("KZB_TRACE"))
         if (tr[0] == '1') trace_ = new double[5]();
+    heads_tail_prepare();
     if (precision_ == 1)
         build_bf16();
     else

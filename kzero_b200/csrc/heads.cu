@@ -17,8 +17,12 @@ namespace {
 
 constexpr int kWarpsPerBlock = 4;
 constexpr int kMaxHiddenPerLane = 4;  // hs <= 128
+constexpr size_t kMaxSmem = 227 * 1024;
 
-template <bool PACKED, int HPL>  // HPL = hidden units per lane = ceil(hs / 32)
+// STAGED: the warp copies its board's fc1 inputs to shared memory first (kWarpsPerBlock * hc * area floats a block).  Boards too
+// large for that (above about 60 x 60 squares at hc = 4, go-256 at any hc) read them from global memory instead, in the same order,
+// so both forms give the same bits.
+template <bool PACKED, int HPL, bool STAGED>  // HPL = hidden units per lane = ceil(hs / 32)
 __global__ void __launch_bounds__(kWarpsPerBlock * 32) heads_tail_kernel(HeadsTailParams p) {
     extern __shared__ float smem[];
     const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
@@ -28,11 +32,15 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) heads_tail_kernel(HeadsTa
     const int area = p.lay.W * p.lay.H;
     const int n_in = p.hc * area;
     float* s_in = smem + size_t(warp) * n_in;  // flatten order (channel, y, x), post_act.py:16
+    auto fc1_in = [&](int i) -> float {
+        return STAGED ? s_in[i] : p.s1[size_t(p.lay.row(b, i % area)) * p.s1_stride + i / area];
+    };
 
-    for (int i = lane; i < n_in; i += 32) {
-        int c = i / area, sq = i % area;
-        s_in[i] = p.s1[size_t(p.lay.row(b, sq)) * p.s1_stride + c];
-    }
+    if (STAGED)
+        for (int i = lane; i < n_in; i += 32) {
+            int c = i / area, sq = i % area;
+            s_in[i] = p.s1[size_t(p.lay.row(b, sq)) * p.s1_stride + c];
+        }
     float extra = 0.0f;
     if (p.extra_w) {
         float e = 0.0f;
@@ -52,7 +60,7 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) heads_tail_kernel(HeadsTa
         for (int k = 0; k < 8; k++) {
             const int i = i0 + k;
             const bool ok = i < n_in;
-            v[k] = ok ? s_in[i] : 0.0f;
+            v[k] = ok ? fc1_in(i) : 0.0f;
 #pragma unroll
             for (int u = 0; u < HPL; u++) {
                 const int j = lane + 32 * u;
@@ -108,12 +116,28 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) heads_tail_kernel(HeadsTa
 
 }  // namespace
 
+void heads_tail_prepare() {
+#define KZB_OPT_IN(PACKED, HPL) \
+    cudaFuncSetAttribute(heads_tail_kernel<PACKED, HPL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kMaxSmem))
+    KZB_OPT_IN(true, 1);
+    KZB_OPT_IN(true, 2);
+    KZB_OPT_IN(true, 4);
+    KZB_OPT_IN(false, 1);
+    KZB_OPT_IN(false, 2);
+    KZB_OPT_IN(false, 4);
+#undef KZB_OPT_IN
+}
+
 void launch_heads_tail(const HeadsTailParams& p, cudaStream_t s) {
     if (p.out.batch <= 0) return;
     int blocks = (p.out.batch + kWarpsPerBlock - 1) / kWarpsPerBlock;
-    size_t smem = size_t(kWarpsPerBlock) * p.hc * p.lay.W * p.lay.H * sizeof(float);
+    const size_t stage = size_t(kWarpsPerBlock) * p.hc * p.lay.W * p.lay.H * sizeof(float);
+    const bool staged = stage <= kMaxSmem;
+    const size_t smem = staged ? stage : 0;
     const int hpl = (p.hs + 31) / 32;
-#define KZB_TAIL(PACKED, HPL) heads_tail_kernel<PACKED, HPL><<<blocks, kWarpsPerBlock * 32, smem, s>>>(p)
+#define KZB_TAIL(PACKED, HPL)                                                                       \
+    (staged ? heads_tail_kernel<PACKED, HPL, true><<<blocks, kWarpsPerBlock * 32, smem, s>>>(p) \
+            : heads_tail_kernel<PACKED, HPL, false><<<blocks, kWarpsPerBlock * 32, smem, s>>>(p))
     if (p.out.packed) {
         if (hpl <= 1) KZB_TAIL(true, 1);
         else if (hpl == 2) KZB_TAIL(true, 2);

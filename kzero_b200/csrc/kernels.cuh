@@ -190,6 +190,7 @@ struct HeadsTailParams {
     float att_div;
     const AttEntryDev* att_entries;  // [P] or null
 };
+void heads_tail_prepare();  // per-device: opt in to 227 KB dynamic shared memory for the staged fc1 inputs
 void launch_heads_tail(const HeadsTailParams& p, cudaStream_t s);
 
 // ---------------------------------------------------------------------------------------------- K1' + K3 fused (heads8.cu)

@@ -87,7 +87,8 @@ def _value_info(name: str, shape: Sequence) -> bytes:
 
 
 class _GraphBuilder:
-    def __init__(self):
+    def __init__(self, replace: Optional[dict] = None):
+        self.replace = replace or {}
         self.nodes: List[bytes] = []
         self.inits: List[bytes] = []
         self.ops: List[str] = []
@@ -95,6 +96,11 @@ class _GraphBuilder:
         self._n = 0
 
     def init(self, name: str, arr: np.ndarray) -> str:
+        if name in self.replace:
+            new = np.asarray(self.replace[name], dtype=arr.dtype)
+            if new.shape != arr.shape:
+                raise ValueError(f"weights_in[{name!r}] has shape {new.shape}, the graph needs {arr.shape}")
+            arr = new
         self.inits.append(_tensor(name, arr))
         self.arrays[name] = arr
         return name
@@ -187,7 +193,8 @@ _BN = dict(epsilon=float(np.float32(1e-5)), momentum=float(np.float32(0.9)))
 
 def build_onnx(game: GameSpec, depth: int, channels: int, seed: int = 0, scalar_hidden_channels: int = 4,
                scalar_hidden_size: int = 32, query_channels: int = 32, fold_bn: bool = True,
-               weights_out: Optional[dict] = None, legacy_three_outputs: bool = False) -> bytes:
+               weights_out: Optional[dict] = None, legacy_three_outputs: bool = False,
+               weights_in: Optional[dict] = None) -> bytes:
     """ONNX bytes for PredictionHeads(ResTower(depth, C_in, channels), ScalarHead, <policy head>).
 
     fold_bn=False keeps Conv -> BatchNormalization -> Relu un-folded inside blocks (what older torch
@@ -197,9 +204,12 @@ def build_onnx(game: GameSpec, depth: int, channels: int, seed: int = 0, scalar_
     and this library rejects at load time (only used to test that rejection).
 
     weights_out: optional dict that receives every initializer (name -> array; tower convs are w1/b1 = input conv,
-    w2.. = block convs in order) -- what bench.py's library comparator builds the same tower from."""
+    w2.. = block convs in order) -- what bench.py's library comparator builds the same tower from.
+
+    weights_in: optional dict (same names as weights_out) whose arrays replace those initializers; the random draws are made
+    all the same, so the initializers it does not name keep their values.  Without it the bytes are unchanged."""
     rng = np.random.default_rng(seed)
-    g = _GraphBuilder()
+    g = _GraphBuilder(weights_in)
     c, a, s = channels, game.area, game.board_size
     eps = np.float32(1e-5)
     k = 0
