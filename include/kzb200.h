@@ -31,6 +31,10 @@ typedef struct kzb_net kzb_net;
 
 #define KZB_PRECISION_FP32 0 /* CUDA-core fp32, <= 1e-4 max-abs vs the CPU executor            */
 #define KZB_PRECISION_BF16 1 /* tcgen05 tensor cores: bf16 operands, fp32 accumulate (the fast path) */
+/* tcgen05 kind::tf32 on the row kernels for every board: f32 activations rounded to TF32 (round to nearest, ties away), fp32
+ * accumulate.  Logits and raw scalars within 4e-3 * max(1, max |logit|) of the f32 CPU executor, probabilities within 1e-3
+ * (tests/test_tf32.py); about 7x closer than bf16 on deep towers. */
+#define KZB_PRECISION_TF32 2
 
 /* Replaces CudaDevice::all() (rust/kz-selfplay/src/server/server.rs:49-51). */
 int kzb_device_count(void);
@@ -44,7 +48,7 @@ typedef struct kzb_net_info {
     int32_t policy_len;                       /* product of the policy output's non-batch dims */
     int32_t channels, depth;                  /* tower width / residual blocks                 */
     int32_t max_batch, precision, device;
-    int32_t conv_mode;      /* 0: row kernels (dense rows), 1: 8x8-board kernels, -1: fp32 */
+    int32_t conv_mode;      /* 0: row kernels (dense rows; always in tf32), 1: 8x8-board kernels, -1: fp32 */
     double flops_per_position; /* algorithmic FLOPs (no padding/halo), SURVEY.md 8(d)          */
 } kzb_net_info;
 

@@ -23,7 +23,7 @@ __device__ __forceinline__ void conv_epilogue_tile(const ConvTcParams& p, const 
     uint4 resq[kResPrefetch];
     const bool has_res = p.res != nullptr && store;
     if (has_res) {
-        const uint4* rp = reinterpret_cast<const uint4*>(p.res + size_t(row) * p.res_stride + ch_base);
+        const uint4* rp = reinterpret_cast<const uint4*>(static_cast<const __nv_bfloat16*>(p.res) + size_t(row) * p.res_stride + ch_base);
 #pragma unroll
         for (int j = 0; j < kResPrefetch; j++)
             if (j * 8 < n_cols) resq[j] = rp[j];
@@ -59,7 +59,7 @@ __device__ __forceinline__ void conv_epilogue_tile(const ConvTcParams& p, const 
                     q0 = resq[cc * 4 + h * 2];
                     q1 = resq[cc * 4 + h * 2 + 1];
                 } else {
-                    const uint4* rp = reinterpret_cast<const uint4*>(p.res + size_t(row) * p.res_stride + ch);
+                    const uint4* rp = reinterpret_cast<const uint4*>(static_cast<const __nv_bfloat16*>(p.res) + size_t(row) * p.res_stride + ch);
                     q0 = rp[0];
                     q1 = rp[1];
                 }

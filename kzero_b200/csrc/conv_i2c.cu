@@ -24,6 +24,13 @@
 // of a tile's MMA time: profiles/r02_go_kernels.md).
 // p.n_split = 2 (small batches): a work item is one 256-pixel tile x one half of the output channels (M256 N128 MMAs).
 // p.pdl: launched with programmatic stream serialization -- set-up and the first weight tiles overlap the previous layer's tail.
+//
+// Two instances, one per operand type T; a k-block is one 128-byte row in either:
+//   bf16  (p.tf32 = 0): 64 channels per k-block, kind::f16 MMAs of K = 16, bf16 rows, 2 KB SWIZZLE_64B staging boxes
+//   float (p.tf32 = 1): 32 channels per k-block, kind::tf32 MMAs of K = 8 on f32 values that are TF32-exact; f32 rows, 4 KB
+//                       SWIZZLE_128B staging boxes, and every stored value rounded to TF32 (tf32_round), since it is the next
+//                       layer's MMA operand.  Twice the k-blocks of bf16 for the same channels, so twice the stages per layer.
+// Stages, the pair logic, PDL, n_split and the barrier protocol are the same in both.
 #include "kernels.cuh"
 #include "tc_common.cuh"
 
@@ -31,13 +38,16 @@ namespace kzb {
 namespace {
 
 constexpr int kTileM = 128;
-constexpr int kBlockK = 64;
 constexpr int kThreads = 192;
-constexpr uint32_t kABytes = kTileM * kBlockK * 2;  // one im2col tile
-constexpr uint32_t kStageBytes = 2 * kABytes;       // + a half weight tile of up to 128 rows
-constexpr int kChunk = 32;                          // output channels per epilogue step
-constexpr uint32_t kStgBytes = 32 * kChunk * 2;     // one staging box: 32 rows x 32 channels bf16
-constexpr int kStgBufs = 4;                         // per epilogue warp
+constexpr uint32_t kABytes = kTileM * 128;    // one im2col tile: 128 pixels x one 128-byte k-block
+constexpr uint32_t kStageBytes = 2 * kABytes;  // + a half weight tile of up to 128 rows
+constexpr int kMmasPerStage = 4;               // 32 bytes of K each: K = 16 bf16 or K = 8 TF32
+constexpr int kChunk = 32;                     // output channels per epilogue step
+constexpr int kStgBufs = 4;                    // per epilogue warp
+template <typename T>
+constexpr int kBlockKOf = 128 / int(sizeof(T));  // channels per k-block
+template <typename T>
+constexpr uint32_t kStgBytesOf = 32 * kChunk * sizeof(T);  // one staging box: 32 rows x 32 channels
 constexpr uint16_t kPairMask = 3;
 constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;
 
@@ -45,17 +55,18 @@ using namespace tc;
 
 struct SmemLayout {
     uint8_t* stages;   // [stage][A 16 KB | B 16 KB], 1024-byte aligned
-    uint8_t* staging;  // [epilogue warp][kStgBufs][2 KB]
+    uint8_t* staging;  // [epilogue warp][kStgBufs][kStgBytes]
     uint64_t *full, *empty, *tmem_full, *tmem_empty, *res_full;
     uint32_t* tmem_ptr;
     float* bias;
 };
 
+template <typename T>
 __device__ __forceinline__ SmemLayout carve(uint8_t* base, int stages) {
     SmemLayout s;
     s.stages = base;
     s.staging = base + size_t(stages) * kStageBytes;
-    s.full = reinterpret_cast<uint64_t*>(s.staging + 4 * kStgBufs * kStgBytes);
+    s.full = reinterpret_cast<uint64_t*>(s.staging + 4 * kStgBufs * kStgBytesOf<T>);
     s.empty = s.full + stages;
     s.tmem_full = s.empty + stages;
     s.tmem_empty = s.tmem_full + 2;
@@ -65,7 +76,7 @@ __device__ __forceinline__ SmemLayout carve(uint8_t* base, int stages) {
     return s;
 }
 
-// im2col load of kTileM pixels x 64 channels starting at base pixel (w, h, n) (bounding-box coordinates: output pixel - 1),
+// im2col load of kTileM pixels x one k-block of channels starting at base pixel (w, h, n) (bounding-box coordinates: output pixel - 1),
 // tap offset (off_w, off_h) in 0..2; issued by either CTA of the pair, bytes completed on the LEADER's barrier
 __device__ __forceinline__ void tma2_load_im2col(const CUtensorMap* map, uint64_t* bar, void* dst, int c, int w, int h, int n, uint16_t off_w,
                                                  uint16_t off_h) {
@@ -92,15 +103,26 @@ __device__ __forceinline__ void tma_store_wait_read() {  // at most kPending of 
     asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(kPending) : "memory");
 }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void umma2_bf16(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d),
-        "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
+template <typename T>
+__device__ __forceinline__ void umma2(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+    if constexpr (sizeof(T) == 4)
+        asm volatile(
+            "{\n\t"
+            ".reg .pred p;\n\t"
+            "setp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t"
+            "}" ::"r"(tmem_d),
+            "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+            : "memory");
+    else
+        asm volatile(
+            "{\n\t"
+            ".reg .pred p;\n\t"
+            "setp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
+            "}" ::"r"(tmem_d),
+            "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+            : "memory");
 }
 __device__ __forceinline__ void umma2_commit(uint64_t* bar) {  // arrives on `bar` in both CTAs of the pair
     asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
@@ -108,12 +130,15 @@ __device__ __forceinline__ void umma2_commit(uint64_t* bar) {  // arrives on `ba
                  : "memory");
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kThreads, 1)
     conv_i2c_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_bh, const __grid_constant__ CUtensorMap tmap_out,
                     const __grid_constant__ CUtensorMap tmap_res, const ConvTcParams p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    const SmemLayout sm = carve(smem, p.stages);
+    const SmemLayout sm = carve<T>(smem, p.stages);
+    constexpr int kBlockK = kBlockKOf<T>;
+    constexpr uint32_t kStgBytes = kStgBytesOf<T>;
     const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
     const uint32_t rank = cluster_ctarank();
     const bool leader = rank == 0;
@@ -201,7 +226,7 @@ __global__ void __launch_bounds__(kThreads, 1)
     } else if (warp == 1) {
         // ------------------------------------------------------------------ MMA warp: only the leader's issues
         if (leader) {
-            const uint32_t idesc = umma_idesc_bf16(2 * kTileM, n_eff);
+            const uint32_t idesc = umma_idesc<T>(2 * kTileM, n_eff);
             const uint64_t hi = umma_desc_sw128_hi();
             int stage = 0;
             uint32_t phase = 0;
@@ -220,8 +245,8 @@ __global__ void __launch_bounds__(kThreads, 1)
                     const uint32_t b_lo = a_lo + (kABytes >> 4);
                     if (lane == 0) {
 #pragma unroll
-                        for (int k = 0; k < kBlockK / 16; k++)
-                            umma2_bf16(tmem_d, hi | uint64_t(a_lo + 2 * k), hi | uint64_t(b_lo + 2 * k), idesc, (it != 0 || k != 0) ? 1u : 0u);
+                        for (int k = 0; k < kMmasPerStage; k++)
+                            umma2<T>(tmem_d, hi | uint64_t(a_lo + 2 * k), hi | uint64_t(b_lo + 2 * k), idesc, (it != 0 || k != 0) ? 1u : 0u);
                         umma2_commit(&sm.empty[stage]);
                     }
                     __syncwarp();
@@ -262,7 +287,10 @@ __global__ void __launch_bounds__(kThreads, 1)
             if (total > 0) load_res(0);
             if (total > 1) load_res(1);
         }
-        const int sw = (lane >> 1) & 3;  // SWIZZLE_64B: 16-byte chunk index ^ bits 7..8 of the address
+        // 16-byte chunk index ^ the address bits above the row: SWIZZLE_64B (64-byte bf16 rows) bits 7..8, SWIZZLE_128B (128-byte f32
+        // rows) bits 7..9
+        const int sw = sizeof(T) == 4 ? (lane & 7) : ((lane >> 1) & 3);
+        constexpr int kVec = 16 / int(sizeof(T));  // channels per 16-byte unit
 #pragma unroll 1
         for (uint32_t f = 0; f < total; f++) {
             const uint32_t li = f / cpi, c = f - li * cpi, buf = li & 1, sb = f % kStgBufs;
@@ -286,28 +314,40 @@ __global__ void __launch_bounds__(kThreads, 1)
                 if (lane == 0) tma_store_wait_read<kStgBufs - 1>();  // the store that last read this buffer (chunk f - 4) is done with it
                 __syncwarp();
             }
-            uint8_t* row_ptr = stg + sb * kStgBytes + lane * (kChunk * 2);
+            uint8_t* row_ptr = stg + sb * kStgBytes + lane * (kChunk * int(sizeof(T)));
             const float* bias = sm.bias + col0;
 #pragma unroll
-            for (int j = 0; j < 4; j++) {  // 8 channels = one 16-byte unit of the row
-                float v[8];
+            for (int j = 0; j < kChunk / kVec; j++) {  // kVec channels = one 16-byte unit of the row
+                float v[kVec];
 #pragma unroll
-                for (int k = 0; k < 8; k++) {
-                    float x = __uint_as_float(r[j * 8 + k]) + bias[j * 8 + k];
+                for (int k = 0; k < kVec; k++) {
+                    float x = __uint_as_float(r[j * kVec + k]) + bias[j * kVec + k];
                     v[k] = relu ? (x < 0.0f ? 0.0f : x) : x;  // NaN stays NaN, like torch / ONNX Relu
                 }
                 uint4* cell = reinterpret_cast<uint4*>(row_ptr + ((j ^ sw) << 4));
-                if (has_res) {  // the reference block is x + relu(bn(conv(...))): relu BEFORE the add (post_act.py:218-228)
-                    const uint4 q = *cell;
-                    const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&q);
-#pragma unroll
-                    for (int k = 0; k < 4; k++) {
-                        const float2 t = __bfloat1622float2(h[k]);
-                        v[2 * k] += t.x;
-                        v[2 * k + 1] += t.y;
+                if constexpr (sizeof(T) == 4) {
+                    if (has_res) {  // the reference block is x + relu(bn(conv(...))): relu BEFORE the add (post_act.py:218-228)
+                        const uint4 q = *cell;
+                        v[0] += __uint_as_float(q.x);
+                        v[1] += __uint_as_float(q.y);
+                        v[2] += __uint_as_float(q.z);
+                        v[3] += __uint_as_float(q.w);
                     }
+                    *cell = make_uint4(__float_as_uint(tf32_round(v[0])), __float_as_uint(tf32_round(v[1])), __float_as_uint(tf32_round(v[2])),
+                                       __float_as_uint(tf32_round(v[3])));
+                } else {
+                    if (has_res) {  // the reference block is x + relu(bn(conv(...))): relu BEFORE the add (post_act.py:218-228)
+                        const uint4 q = *cell;
+                        const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&q);
+#pragma unroll
+                        for (int k = 0; k < 4; k++) {
+                            const float2 t = __bfloat1622float2(h[k]);
+                            v[2 * k] += t.x;
+                            v[2 * k + 1] += t.y;
+                        }
+                    }
+                    *cell = make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
                 }
-                *cell = make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
             }
             fence_proxy_async_smem();  // generic-proxy writes -> visible to the TMA store
             __syncwarp();
@@ -335,22 +375,27 @@ __global__ void __launch_bounds__(kThreads, 1)
 
 }  // namespace
 
-size_t conv_i2c_smem_bytes(int n, int stages) {
-    return 1024 /*alignment slack*/ + size_t(stages) * kStageBytes + 4 * kStgBufs * kStgBytes + (2 * stages + 4 + 4 * kStgBufs) * 8 + 16 + size_t(n) * 4;
+size_t conv_i2c_smem_bytes(int n, int stages, bool tf32) {
+    const size_t stg = tf32 ? kStgBytesOf<float> : kStgBytesOf<__nv_bfloat16>;
+    return 1024 /*alignment slack*/ + size_t(stages) * kStageBytes + 4 * kStgBufs * stg + (2 * stages + 4 + 4 * kStgBufs) * 8 + 16 + size_t(n) * 4;
 }
 
-int conv_i2c_pick_stages(int n) {
+// bf16: 6 stages; TF32: 5 (its staging boxes take 32 KB more)
+int conv_i2c_pick_stages(int n, bool tf32) {
     const size_t budget = 227 * 1024;
     int stages = 6;
-    while (stages > 2 && conv_i2c_smem_bytes(n, stages) > budget) stages--;
+    while (stages > 2 && conv_i2c_smem_bytes(n, stages, tf32) > budget) stages--;
     return stages;
 }
 
-void conv_i2c_prepare() { cudaFuncSetAttribute(conv_i2c_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024); }
+void conv_i2c_prepare() {
+    cudaFuncSetAttribute(conv_i2c_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaFuncSetAttribute(conv_i2c_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+}
 
-// tmap_a: im2col map over the dense channels-last activations (C, W, H, boards), 64 channels x 128 pixels per load, SWIZZLE_128B;
+// tmap_a: im2col map over the dense channels-last activations (C, W, H, boards), one k-block x 128 pixels per load, SWIZZLE_128B;
 // tmap_bh: weight map whose box holds p.n / p.n_split / 2 rows; tmap_out / tmap_res: output / residual rows, box (32 channels, 32 rows),
-// SWIZZLE_64B (tmap_res is only read when p.res is set)
+// SWIZZLE_64B for bf16, SWIZZLE_128B for TF32 (tmap_res is only read when p.res is set)
 void launch_conv_i2c(const CUtensorMap& tmap_a, const CUtensorMap& tmap_bh, const CUtensorMap& tmap_out, const CUtensorMap& tmap_res,
                      const ConvTcParams& p, int grid, cudaStream_t s) {
     if (p.num_tiles <= 0) return;
@@ -358,7 +403,7 @@ void launch_conv_i2c(const CUtensorMap& tmap_a, const CUtensorMap& tmap_bh, cons
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(unsigned(2 * std::min(grid / 2, items)));
     cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = conv_i2c_smem_bytes(p.n, p.stages);
+    cfg.dynamicSmemBytes = conv_i2c_smem_bytes(p.n, p.stages, p.tf32 != 0);
     cfg.stream = s;
     cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -369,7 +414,10 @@ void launch_conv_i2c(const CUtensorMap& tmap_a, const CUtensorMap& tmap_bh, cons
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = p.pdl ? 2 : 1;
-    cudaLaunchKernelEx(&cfg, conv_i2c_kernel, tmap_a, tmap_bh, tmap_out, tmap_res, p);
+    if (p.tf32)
+        cudaLaunchKernelEx(&cfg, conv_i2c_kernel<float>, tmap_a, tmap_bh, tmap_out, tmap_res, p);
+    else
+        cudaLaunchKernelEx(&cfg, conv_i2c_kernel<__nv_bfloat16>, tmap_a, tmap_bh, tmap_out, tmap_res, p);
 }
 
 }  // namespace kzb

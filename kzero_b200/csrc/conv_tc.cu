@@ -14,6 +14,9 @@
 //   * persistent CTAs, warp-specialised: warp 0 TMA producer, warp 1 MMA issuer (+TMEM owner),
 //     warps 2..5 epilogue; smem ring of `stages` (A,B) slots; two TMEM accumulators so the epilogue of
 //     tile i overlaps the MMAs of tile i+1.
+//   * two instances: bf16 rows (kind::f16, K = 16, 64 channels per k-block) and, for the TF32 precision, f32 rows holding TF32-exact
+//     values (kind::tf32, K = 8, 32 channels per k-block); a k-block is one 128-byte row in both, so the stage layout is the same.
+//     The output is f32 and is not rounded: the tail kernel's CUDA-core FCs read it.
 #include "conv_epilogue.cuh"
 #include "kernels.cuh"
 #include "tc_common.cuh"
@@ -22,8 +25,8 @@ namespace kzb {
 namespace {
 
 constexpr int kTileM = 128;
-constexpr int kBlockK = 64;                       // bf16 elements per smem row = 128 bytes = one swizzle span
-constexpr int kABytes = kTileM * kBlockK * 2;     // 16 KiB
+constexpr int kABytes = kTileM * 128;            // 16 KiB: one 128-byte smem row (= one swizzle span) per tile row
+constexpr int kMmasPerKBlock = 4;                 // 32 bytes of K each: K = 16 bf16 or K = 8 TF32
 constexpr int kThreads = 192;
 
 using namespace tc;
@@ -51,12 +54,14 @@ __device__ __forceinline__ SmemLayout carve(uint8_t* base, int n, int stages) {
     return s;
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kThreads, 1)
     conv_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, const ConvTcParams p) {
     extern __shared__ uint8_t smem_raw[];
     // SWIZZLE_128B atoms need 1024-byte alignment
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const SmemLayout sm = carve(smem, p.n, p.stages);
+    constexpr int kBlockK = 128 / int(sizeof(T));  // channels per k-block
     const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
     const int stage_bytes = kABytes + p.n * 128;
     const int my_tiles = (p.num_tiles - int(blockIdx.x) + int(gridDim.x) - 1) / int(gridDim.x);
@@ -111,7 +116,7 @@ __global__ void __launch_bounds__(kThreads, 1)
     } else if (warp == 1) {
         // ------------------------------------------------------------------ MMA issuer
         // whole warp walks the loops (uniform datapath for the address arithmetic); lane 0 issues MMAs + commits
-        const uint32_t idesc = umma_idesc_bf16(kTileM, p.n);
+        const uint32_t idesc = umma_idesc<T>(kTileM, p.n);
         const uint64_t desc_hi = umma_desc_sw128_hi();
         int stage = 0;
         uint32_t phase = 0;
@@ -128,10 +133,13 @@ __global__ void __launch_bounds__(kThreads, 1)
                 const uint32_t b_lo = a_lo + (kABytes >> 4);
                 if (lane == 0) {
 #pragma unroll
-                    for (int k = 0; k < kBlockK / 16; k++) {
-                        // advancing 16 bf16 = 32 bytes along K stays inside the 128-byte swizzle span
-                        umma_bf16(tmem_d, desc_hi | uint64_t(a_lo + 2 * k), desc_hi | uint64_t(b_lo + 2 * k), idesc,
-                                  (it | k) != 0);
+                    for (int k = 0; k < kMmasPerKBlock; k++) {
+                        // advancing 32 bytes along K stays inside the 128-byte swizzle span
+                        if constexpr (sizeof(T) == 4)
+                            umma_tf32(tmem_d, desc_hi | uint64_t(a_lo + 2 * k), desc_hi | uint64_t(b_lo + 2 * k), idesc, (it | k) != 0);
+                        else
+                            umma_bf16(tmem_d, desc_hi | uint64_t(a_lo + 2 * k), desc_hi | uint64_t(b_lo + 2 * k), idesc,
+                                      (it | k) != 0);
                     }
                     // frees the smem slot once these MMAs have read it
                     umma_commit(&sm.empty[stage]);
@@ -179,11 +187,17 @@ int conv_tc_pick_stages(int n) {
     return stages;
 }
 
-void conv_tc_prepare() { cudaFuncSetAttribute(conv_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024); }
+void conv_tc_prepare() {
+    cudaFuncSetAttribute(conv_tc_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaFuncSetAttribute(conv_tc_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+}
 
 void launch_conv_tc(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const ConvTcParams& p, int grid, cudaStream_t s) {
     if (p.num_tiles <= 0) return;
-    conv_tc_kernel<<<std::min(grid, p.num_tiles), kThreads, conv_tc_smem_bytes(p.n, p.stages), s>>>(tmap_a, tmap_b, p);
+    if (p.tf32)
+        conv_tc_kernel<float><<<std::min(grid, p.num_tiles), kThreads, conv_tc_smem_bytes(p.n, p.stages), s>>>(tmap_a, tmap_b, p);
+    else
+        conv_tc_kernel<__nv_bfloat16><<<std::min(grid, p.num_tiles), kThreads, conv_tc_smem_bytes(p.n, p.stages), s>>>(tmap_a, tmap_b, p);
 }
 
 }  // namespace kzb

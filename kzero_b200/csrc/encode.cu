@@ -35,6 +35,11 @@ struct Vec8<float> {
         reinterpret_cast<float4*>(base)[vec_index * 2 + 1] = b;
     }
 };
+struct Tf32;  // f32 rows whose values are rounded to TF32: what the TF32 precision's first conv reads (scalar planes need not be exact)
+template <>
+struct Vec8<Tf32> : Vec8<float> {
+    __device__ void set(int i, float f) { Vec8<float>::set(i, tf32_round(f)); }
+};
 
 template <typename T>
 __global__ void __launch_bounds__(kEncodeThreads) encode_nhwc_kernel(EncodeParams p) {
@@ -177,11 +182,13 @@ void launch_nchw_to_kc(const float* in, int batch, int channels, int rec_w, int 
     encode_kc_kernel<false><<<batch, std::min(kc_total * 64, 512), 0, s>>>(p, in, channels, kc_total, boards_total);
 }
 
-void launch_encode_nhwc(const EncodeParams& p, bool out_bf16, cudaStream_t s) {
+void launch_encode_nhwc(const EncodeParams& p, Act out, cudaStream_t s) {
     if (p.batch <= 0) return;
     size_t smem = ((p.scalar_count * 4 + 15) / 16) * 16 + p.bits_stride;
-    if (out_bf16)
+    if (out == Act::kBf16)
         encode_nhwc_kernel<__nv_bfloat16><<<p.batch, kEncodeThreads, smem, s>>>(p);
+    else if (out == Act::kTf32)
+        encode_nhwc_kernel<Tf32><<<p.batch, kEncodeThreads, smem, s>>>(p);
     else
         encode_nhwc_kernel<float><<<p.batch, kEncodeThreads, smem, s>>>(p);
 }
@@ -194,13 +201,15 @@ void launch_encode_nchw_f32(const uint8_t* bits, const float* scalars, int batch
     encode_nchw_f32_kernel<<<blocks, 256, 0, s>>>(bits, scalars, batch, bits_stride, scalar_count, bool_channels, area, out);
 }
 
-void launch_nchw_to_rows(const float* in, int batch, int channels, RowLayout lay, int c_pad, void* out, bool out_bf16,
+void launch_nchw_to_rows(const float* in, int batch, int channels, RowLayout lay, int c_pad, void* out, Act out_type,
                          cudaStream_t s) {
     if (batch <= 0) return;
     size_t total = size_t(batch) * lay.W * lay.H * (c_pad / 8);
     int blocks = int(std::min<size_t>((total + 255) / 256, 148 * 16));
-    if (out_bf16)
+    if (out_type == Act::kBf16)
         nchw_to_rows_kernel<__nv_bfloat16><<<blocks, 256, 0, s>>>(in, batch, channels, lay, c_pad, out);
+    else if (out_type == Act::kTf32)
+        nchw_to_rows_kernel<Tf32><<<blocks, 256, 0, s>>>(in, batch, channels, lay, c_pad, out);
     else
         nchw_to_rows_kernel<float><<<blocks, 256, 0, s>>>(in, batch, channels, lay, c_pad, out);
 }

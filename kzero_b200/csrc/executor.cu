@@ -36,9 +36,10 @@ EncodeTiledFn encode_tiled_fn() {
     return fn;
 }
 
-// bf16 tensor map, SWIZZLE_128B, zero OOB fill.  dims/box innermost first; strides in bytes for dims 1..rank-1.
+// tensor map (bf16 unless `dtype` says otherwise), SWIZZLE_128B, zero OOB fill.  dims/box innermost first; strides in bytes for
+// dims 1..rank-1.
 CUtensorMap make_tmap(void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box,
-                      bool swizzle128 = true, bool swizzle64 = false) {
+                      bool swizzle128 = true, bool swizzle64 = false, CUtensorMapDataType dtype = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16) {
     CUtensorMap m;
     cuuint64_t gdim[5], gstr[4];
     cuuint32_t bdim[5], estr[5];
@@ -48,7 +49,7 @@ CUtensorMap make_tmap(void* base, int rank, const uint64_t* dims, const uint64_t
         estr[i] = 1;
         if (i > 0) gstr[i - 1] = strides_bytes[i - 1];
     }
-    CUresult r = encode_tiled_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, cuuint32_t(rank), base, gdim, gstr, bdim, estr,
+    CUresult r = encode_tiled_fn()(&m, dtype, cuuint32_t(rank), base, gdim, gstr, bdim, estr,
                                    CU_TENSOR_MAP_INTERLEAVE_NONE,
                                    swizzle64 ? CU_TENSOR_MAP_SWIZZLE_64B : swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
                                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -61,9 +62,10 @@ typedef CUresult (*EncodeIm2colFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t
                                    const int*, cuuint32_t, cuuint32_t, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-// bf16 im2col map over channels-last activations [boards][H][W][C] for a (2 * pad + 1)^2 filter with zero padding `pad`: a load
-// brings `pixels` consecutive output pixels x `channels` channels, shifted by the instruction's tap offset, zero-filled off the board
-CUtensorMap make_tmap_im2col(void* base, int C, int W, int H, int boards, int channels, int pixels, int pad) {
+// im2col map over channels-last activations [boards][H][W][C] of `dtype` (bf16 or f32) for a (2 * pad + 1)^2 filter with zero
+// padding `pad`: a load brings `pixels` consecutive output pixels x `channels` channels, shifted by the instruction's tap offset,
+// zero-filled off the board
+CUtensorMap make_tmap_im2col(void* base, int C, int W, int H, int boards, int channels, int pixels, int pad, CUtensorMapDataType dtype) {
     static EncodeIm2colFn fn = [] {
         void* p = nullptr;
         cudaDriverEntryPointQueryResult q;
@@ -72,17 +74,18 @@ CUtensorMap make_tmap_im2col(void* base, int C, int W, int H, int boards, int ch
         return reinterpret_cast<EncodeIm2colFn>(p);
     }();
     CUtensorMap m;
+    const size_t esz = dtype == CU_TENSOR_MAP_DATA_TYPE_FLOAT32 ? 4 : 2;
     cuuint64_t gdim[4] = {cuuint64_t(C), cuuint64_t(W), cuuint64_t(H), cuuint64_t(boards)};
-    cuuint64_t gstr[3] = {cuuint64_t(C) * 2, cuuint64_t(C) * 2 * W, cuuint64_t(C) * 2 * W * H};
+    cuuint64_t gstr[3] = {cuuint64_t(C) * esz, cuuint64_t(C) * esz * W, cuuint64_t(C) * esz * W * H};
     int lower[2] = {-pad, -pad}, upper[2] = {-pad, -pad};  // -padding, padding - (filter - 1)
     cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = fn(&m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, gdim, gstr, lower, upper, cuuint32_t(channels), cuuint32_t(pixels), estr,
+    CUresult r = fn(&m, dtype, 4, base, gdim, gstr, lower, upper, cuuint32_t(channels), cuuint32_t(pixels), estr,
                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) throw std::runtime_error("cuTensorMapEncodeIm2col failed with CUresult " + std::to_string(int(r)));
     // drivers up to CUDA 13.1 mis-encode im2col maps of tensors smaller than 128 KiB (bit 21 of the second descriptor word must be
     // clear); the same correction CUTLASS applies in make_im2col_tma_copy_desc
     int driver = 0;
-    if (cudaDriverGetVersion(&driver) == cudaSuccess && driver <= 13010 && size_t(C) * 2 * W * H * boards < 131072)
+    if (cudaDriverGetVersion(&driver) == cudaSuccess && driver <= 13010 && size_t(C) * esz * W * H * boards < 131072)
         reinterpret_cast<uint64_t*>(&m)[1] &= ~(1ull << 21);
     return m;
 }
@@ -128,7 +131,7 @@ Net::Net(int device, const void* onnx, size_t len, int max_batch, int precision)
 Net::Net(int device, NetSpec spec, int max_batch, int precision)
     : device_(device), max_batch_(max_batch), precision_(precision) {
     if (max_batch < 1) throw std::runtime_error("max_batch must be >= 1");
-    if (precision != 0 && precision != 1) throw std::runtime_error("precision must be 0 (fp32) or 1 (bf16)");
+    if (precision < 0 || precision > 2) throw std::runtime_error("precision must be 0 (fp32), 1 (bf16) or 2 (tf32)");
     int count = 0;
     cudaError_t e = cudaGetDeviceCount(&count);
     if (e != cudaSuccess || count == 0)
@@ -146,8 +149,9 @@ Net::Net(int device, NetSpec spec, int max_batch, int precision)
     if (spec_.has_extra && spec_.extra_fc.out != 1) throw std::runtime_error("policy head with more than one extra move is not supported");
     if (spec_.channels > 256 || spec_.policy_conv1.cout > 256 || spec_.policy_conv2.cout > 256)
         throw std::runtime_error("more than 256 channels is not supported");
-    if (precision == 1 && (spec_.board_w > 255 || spec_.board_h > 255))
-        throw std::runtime_error("boards wider or taller than 255 squares are not supported in bf16; use precision=fp32");
+    if (precision != 0 && (spec_.board_w > 255 || spec_.board_h > 255))  // im2col coordinates
+        throw std::runtime_error(std::string("boards wider or taller than 255 squares are not supported in ") + (precision == 1 ? "bf16" : "tf32") +
+                                 "; use precision=fp32");
 
     CK(cudaStreamCreateWithFlags(&stream_, cudaStreamNonBlocking));
     if (const char* bs = std::getenv("KZB_BLOCKING_SYNC")) blocking_sync_ = bs[0] == '1';
@@ -155,8 +159,8 @@ Net::Net(int device, NetSpec spec, int max_batch, int precision)
     if (const char* tr = std::getenv("KZB_TRACE"))
         if (tr[0] == '1') trace_ = new double[5]();
     heads_tail_prepare();
-    if (precision_ == 1)
-        build_bf16();
+    if (precision_ != 0)
+        build_tc();
     else
         build_f32();
 
@@ -257,8 +261,14 @@ static std::vector<AttChunk> att_chunks(const NetSpec& s) {
     return out;
 }
 
-void Net::build_bf16() {
-    act_bf16_ = true;
+// bf16 and TF32.  TF32 runs the row kernels on every board (no tower8k / heads8, no 8x8 embedding); its activations are f32 rows
+// holding TF32-exact values, its weights f32 rounded to TF32 on the host, and a k-block is 32 channels instead of 64.
+void Net::build_tc() {
+    const bool tf32 = precision_ == 2;
+    act_ = tf32 ? Act::kTf32 : Act::kBf16;
+    const int esz = tf32 ? 4 : 2;   // bytes per activation / weight element
+    const int kb = 128 / esz;       // channels per k-block (one 128-byte row of a SWIZZLE_128B tile)
+    const CUtensorMapDataType dtype = tf32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
     const int C = spec_.channels;
     const char* force = std::getenv("KZB_FORCE_LINEAR");
     // Boards smaller than 8x8 (ataxx 2..7, ttt) are embedded top-left in an 8x8 grid and run on the 8x8 whole-tower kernel:
@@ -268,11 +278,11 @@ void Net::build_bf16() {
         auto off = [](const char* name) { const char* v = std::getenv(name); return v && v[0] == '1'; };
         const bool small = spec_.board_w <= 8 && spec_.board_h <= 8 && (spec_.board_w < 8 || spec_.board_h < 8);
         const int units = (((max_batch_ + 3) / 4 + 1) & ~1);
-        embed8_ = small && !off("KZB_FORCE_LINEAR") && !off("KZB_NO_TOWER8") && !off("KZB_NO_EMBED8") && round_up(C, 64) <= 128 &&
+        embed8_ = !tf32 && small && !off("KZB_FORCE_LINEAR") && !off("KZB_NO_TOWER8") && !off("KZB_NO_EMBED8") && round_up(C, 64) <= 128 &&
                   (units + num_sms_ - 1) / num_sms_ <= tower8k_max_local_units();
     }
     const int W = embed8_ ? 8 : spec_.board_w, H = embed8_ ? 8 : spec_.board_h;  // the board as the kernels see it
-    mode_ = (W == 8 && H == 8 && !(force && force[0] == '1')) ? 1 : 0;
+    mode_ = (!tf32 && W == 8 && H == 8 && !(force && force[0] == '1')) ? 1 : 0;
     // DENSE rows, one per square: conv_i2c.cu gets a 3x3 layer's zero padding from the TMA engine's im2col mode
     lay_ = RowLayout{W, H};
     conv_tc_prepare();
@@ -286,16 +296,16 @@ void Net::build_bf16() {
         boards_i2c_ = (pixels + W * H - 1) / (W * H);
         rows_alloc_ = round_up(std::max(pixels, boards_i2c_ * W * H), 128);
     }
-    cin_pad_ = round_up(spec_.cin, 64);
-    c_pad_ = round_up(C, 64);
-    cp_pad_ = round_up(spec_.policy_conv1.cout, 64);
+    cin_pad_ = round_up(spec_.cin, kb);
+    c_pad_ = round_up(C, kb);
+    cp_pad_ = round_up(spec_.policy_conv1.cout, kb);
     pm_stride_ = round_up(spec_.policy_conv2.cout, 16);
     s1_stride_ = 16;
 
-    act_in_.alloc(size_t(rows_alloc_) * cin_pad_ * 2);
-    act_x_.alloc(size_t(rows_alloc_) * c_pad_ * 2);
-    act_t_.alloc(size_t(rows_alloc_) * c_pad_ * 2);
-    act_h1_.alloc(size_t(rows_alloc_) * cp_pad_ * 2);
+    act_in_.alloc(size_t(rows_alloc_) * cin_pad_ * esz);
+    act_x_.alloc(size_t(rows_alloc_) * c_pad_ * esz);
+    act_t_.alloc(size_t(rows_alloc_) * c_pad_ * esz);
+    act_h1_.alloc(size_t(rows_alloc_) * cp_pad_ * esz);
     act_s1_.alloc(size_t(rows_alloc_) * s1_stride_ * 4);
     act_pm_.alloc(size_t(rows_alloc_) * pm_stride_ * 4);
     att_stride_ = spec_.has_attention ? spec_.att_chan_base.back() : 0;
@@ -308,62 +318,70 @@ void Net::build_bf16() {
         st->taps = c.ksize * c.ksize;
         const int cin_pad = in_stride;
         const int ktot = st->taps * cin_pad;
-        std::vector<__nv_bfloat16> w(size_t(n) * ktot, __float2bfloat16_rn(0.0f));
+        std::vector<float> wf(size_t(n) * ktot, 0.0f);
         for (int co = 0; co < c.cout; co++)
             for (int ci = 0; ci < c.cin; ci++)
                 for (int t = 0; t < st->taps; t++)
-                    w[size_t(co) * ktot + size_t(t) * cin_pad + ci] = __float2bfloat16_rn(c.w[(size_t(co) * c.cin + ci) * st->taps + t]);
-        upload(st->w_bf16, w);
+                    wf[size_t(co) * ktot + size_t(t) * cin_pad + ci] = c.w[(size_t(co) * c.cin + ci) * st->taps + t];
+        if (tf32) {
+            for (float& v : wf) v = tf32_round(v);
+            upload(st->w_tc, wf);
+        } else {
+            std::vector<__nv_bfloat16> w(wf.size());
+            for (size_t i = 0; i < wf.size(); i++) w[i] = __float2bfloat16_rn(wf[i]);
+            upload(st->w_tc, w);
+        }
         upload(st->bias, padded_bias(c.b, n));
 
         {
             uint64_t dims[2] = {uint64_t(ktot), uint64_t(n)};
-            uint64_t strides[1] = {uint64_t(ktot) * 2};
-            uint32_t box[2] = {64, uint32_t(n)};
-            st->tmap_b = make_tmap(st->w_bf16.ptr, 2, dims, strides, box);
+            uint64_t strides[1] = {uint64_t(ktot) * esz};
+            uint32_t box[2] = {uint32_t(kb), uint32_t(n)};
+            st->tmap_b = make_tmap(st->w_tc.ptr, 2, dims, strides, box, true, false, dtype);
             st->tmap_bh = st->tmap_b;
             if (n % 32 == 0) {  // half-height box: each CTA of a pair stages half of every weight tile (conv_i2c.cu)
-                uint32_t half[2] = {64, uint32_t(n / 2)};
-                st->tmap_bh = make_tmap(st->w_bf16.ptr, 2, dims, strides, half);
+                uint32_t half[2] = {uint32_t(kb), uint32_t(n / 2)};
+                st->tmap_bh = make_tmap(st->w_tc.ptr, 2, dims, strides, half, true, false, dtype);
             }
         }
         if (out_f32) {  // the head convs: 1x1 (net_spec.cpp), conv_tc.cu
             if (st->taps != 1) throw std::logic_error("internal: conv_tc.cu runs 1x1 convs only");
             uint64_t dims[2] = {uint64_t(in_stride), uint64_t(rows_alloc_)};
-            uint64_t strides[1] = {uint64_t(in_stride) * 2};
-            uint32_t box[2] = {64, 128};
-            st->tmap_a = make_tmap(in.ptr, 2, dims, strides, box);
-        } else {  // conv_i2c.cu: cin_pad and n are multiples of 64, relu_n is 0 or n, out_off is 0
-            st->tmap_i2c = make_tmap_im2col(in.ptr, in_stride, W, H, boards_i2c_, 64, 128, st->taps == 9 ? 1 : 0);
-            auto rows_map = [&](void* ptr, int stride) {
+            uint64_t strides[1] = {uint64_t(in_stride) * esz};
+            uint32_t box[2] = {uint32_t(kb), 128};
+            st->tmap_a = make_tmap(in.ptr, 2, dims, strides, box, true, false, dtype);
+        } else {  // conv_i2c.cu: cin_pad and n are multiples of kb, relu_n is 0 or n, out_off is 0
+            st->tmap_i2c = make_tmap_im2col(in.ptr, in_stride, W, H, boards_i2c_, kb, 128, st->taps == 9 ? 1 : 0, dtype);
+            auto rows_map = [&](void* ptr, int stride) {  // staging boxes of 32 rows x 32 channels: 64-byte (bf16) or 128-byte (f32) rows
                 uint64_t dims[2] = {uint64_t(stride), uint64_t(rows_alloc_)};
-                uint64_t strides[1] = {uint64_t(stride) * 2};
+                uint64_t strides[1] = {uint64_t(stride) * esz};
                 uint32_t box[2] = {32, 32};
-                return make_tmap(ptr, 2, dims, strides, box, false, true);
+                return make_tmap(ptr, 2, dims, strides, box, tf32, !tf32, dtype);
             };
             st->tmap_out = rows_map(out.ptr, out_stride);
             st->tmap_res = res ? rows_map(res->ptr, c_pad_) : st->tmap_out;
             st->tmap_bq = st->tmap_bh;
             if (n % 64 == 0) {
                 uint64_t dims[2] = {uint64_t(ktot), uint64_t(n)};
-                uint64_t strides[1] = {uint64_t(ktot) * 2};
-                uint32_t quarter[2] = {64, uint32_t(n / 4)};
-                st->tmap_bq = make_tmap(st->w_bf16.ptr, 2, dims, strides, quarter);
+                uint64_t strides[1] = {uint64_t(ktot) * esz};
+                uint32_t quarter[2] = {uint32_t(kb), uint32_t(n / 4)};
+                st->tmap_bq = make_tmap(st->w_tc.ptr, 2, dims, strides, quarter, true, false, dtype);
             }
             st->use_i2c = true;
-            st->i2c_stages = conv_i2c_pick_stages(n);
+            st->i2c_stages = conv_i2c_pick_stages(n, tf32);
         }
         ConvTcParams& p = st->tc;
         p.taps = st->taps;
         p.cin_pad = cin_pad;
-        p.kblocks = cin_pad / 64;
+        p.kblocks = cin_pad / kb;
+        p.tf32 = tf32 ? 1 : 0;
         p.n = n;
         p.lay = lay_;
         p.bias = st->bias.as<float>();
         p.relu_n = relu_n;
-        p.res = res ? res->as<__nv_bfloat16>() : nullptr;
+        p.res = res ? res->ptr : nullptr;
         p.res_stride = c_pad_;
-        p.out = static_cast<uint8_t*>(out.ptr) + size_t(out_off) * (out_f32 ? 4 : 2);
+        p.out = static_cast<uint8_t*>(out.ptr) + size_t(out_off) * (out_f32 ? 4 : esz);
         p.out_stride = out_stride;
         p.out_f32 = out_f32 ? 1 : 0;
         p.n_store = n;
@@ -440,12 +458,12 @@ void Net::build_bf16() {
             uint64_t dims[2] = {uint64_t(9 * cin_pad_), uint64_t(n)};
             uint64_t strides[1] = {uint64_t(9 * cin_pad_) * 2};
             uint32_t box[2] = {64, uint32_t(n / cluster)};
-            tower_kmaps_.w[0] = make_tmap(f.w_bf16.ptr, 2, dims, strides, box);
+            tower_kmaps_.w[0] = make_tmap(f.w_tc.ptr, 2, dims, strides, box);
         }
         const size_t layer_w_bytes = size_t(n) * 9 * c_pad_ * 2;
         w_tower_.alloc(std::max<size_t>(layer_w_bytes * 2 * spec_.depth, 256), true);
         for (int i = 0; i < 2 * spec_.depth; i++)
-            CK(cudaMemcpy(w_tower_.as<uint8_t>() + layer_w_bytes * i, convs_[1 + i]->w_bf16.ptr, layer_w_bytes, cudaMemcpyDeviceToDevice));
+            CK(cudaMemcpy(w_tower_.as<uint8_t>() + layer_w_bytes * i, convs_[1 + i]->w_tc.ptr, layer_w_bytes, cudaMemcpyDeviceToDevice));
         {
             uint64_t dims[2] = {uint64_t(9 * c_pad_), uint64_t(std::max(1, 2 * spec_.depth) * n)};
             uint64_t strides[1] = {uint64_t(9 * c_pad_) * 2};
@@ -533,7 +551,7 @@ void Net::build_bf16() {
 }
 
 void Net::build_f32() {
-    act_bf16_ = false;
+    act_ = Act::kF32;
     const int W = spec_.board_w, H = spec_.board_h, C = spec_.channels;
     mode_ = -1;
     lay_ = RowLayout{W, H};
@@ -689,7 +707,7 @@ void Net::run_encode(int batch, const StepHook& hook) {
         p.out = act_ink_.ptr;
         launch_encode_kc(p, cin_pad_ / 8, rows_alloc_ / 64, stream_);
     } else {
-        launch_encode_nhwc(p, act_bf16_, stream_);
+        launch_encode_nhwc(p, act_, stream_);
     }
     if (hook) hook("encode");
 }
@@ -718,7 +736,7 @@ void Net::run_network(int batch, const StepHook& hook) {
     const size_t last_step = (use_heads8_ && precision_ == 1) ? head_first_ : convs_.size();
     for (size_t si = first_step; si < last_step; si++) {
         auto& st = convs_[si];
-        if (precision_ == 1) {
+        if (precision_ != 0) {
             ConvTcParams p = st->tc;
             p.valid_rows = batch * lay_.W * lay_.H;
             p.num_tiles = (p.valid_rows + 127) / 128;
@@ -816,7 +834,7 @@ void Net::eval_planes(const float* nchw, int batch, float* out_scalars, float* o
         launch_nchw_to_kc(d_nchw_.as<float>(), batch, spec_.cin, spec_.board_w, spec_.board_h, cin_pad_ / 8, rows_alloc_ / 64, act_ink_.ptr,
                           stream_);
     else
-        launch_nchw_to_rows(d_nchw_.as<float>(), batch, spec_.cin, lay_, cin_pad_, act_in_.ptr, act_bf16_, stream_);
+        launch_nchw_to_rows(d_nchw_.as<float>(), batch, spec_.cin, lay_, cin_pad_, act_in_.ptr, act_, stream_);
     run_network(batch, nullptr);
     run_tail(batch, false, nullptr);
     CK(cudaMemcpyAsync(out_scalars, d_out_scalars_.ptr, size_t(batch) * 5 * 4, cudaMemcpyDeviceToHost, stream_));

@@ -45,14 +45,14 @@ struct PinnedBuffer {
 struct ConvStep {
     std::string name;
     int taps = 9;
-    // bf16 tensor-core form
+    // tensor-core form (bf16, or f32 rounded to TF32)
     CUtensorMap tmap_a{}, tmap_b{}, tmap_bh{};
     bool use_i2c = false;  // conv_i2c.cu (TMA im2col, CTA-pair MMA); otherwise conv_tc.cu (1x1, f32 output)
     int i2c_stages = 0;
     CUtensorMap tmap_out{}, tmap_res{};  // conv_i2c: output / residual rows, box (32 channels, 32 rows), SWIZZLE_64B
     CUtensorMap tmap_i2c{}, tmap_bq{};  // im2col map of the input rows; weight box of n / 4 rows (output channels split in two)
     ConvTcParams tc{};
-    DeviceBuffer w_bf16;  // [n][taps*cin_pad]
+    DeviceBuffer w_tc;  // [n][taps*cin_pad] bf16, or f32 rounded to TF32
     // fp32 form
     ConvF32Params f32{};
     DeviceBuffer w_f32;  // [taps][cin][cout]
@@ -86,11 +86,11 @@ public:
     int device() const { return device_; }
     int max_batch() const { return max_batch_; }
     int precision() const { return precision_; }
-    int conv_mode() const { return precision_ == 1 ? mode_ : -1; }
+    int conv_mode() const { return precision_ != 0 ? mode_ : -1; }
 
 private:
     using StepHook = std::function<void(const char*)>;
-    void build_bf16();
+    void build_tc();  // bf16 and TF32: the tcgen05 kernels
     void build_f32();
     void check_batch(int batch) const;
     void require_mapper() const;
@@ -108,10 +108,10 @@ private:
 
     int scalar_count_ = -1, bool_channels_ = -1, bits_stride_ = 0;
     RowLayout lay_{};
-    int mode_ = 0;       // bf16 path, dense rows: 0 row kernels (any board), 1 8x8 boards (tower8k / heads8 where they apply)
+    int mode_ = 0;       // tensor-core paths, dense rows: 0 row kernels (any board; always in TF32), 1 8x8 boards (tower8k / heads8 where they apply)
     int rows_alloc_ = 0; // multiple of 128
     int cin_pad_ = 0, c_pad_ = 0, cp_pad_ = 0, s1_stride_ = 16, pm_stride_ = 0;
-    bool act_bf16_ = true;
+    Act act_ = Act::kBf16;
     bool embed8_ = false;  // a board smaller than 8x8 embedded in the 8x8 grid of the whole-tower kernel
     int boards_i2c_ = 0;   // boards covered by the im2col tensor maps (>= every 256-pixel tile of a full batch)
 

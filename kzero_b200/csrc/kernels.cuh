@@ -10,8 +10,37 @@
 #include <stdint.h>
 
 #include <algorithm>
+#include <cstring>
 
 namespace kzb {
+
+// Element type of the activation rows: bf16 (tensor-core path), f32 (CUDA-core fp32 path), or f32 rounded to TF32 (tensor-core
+// TF32 path: every value a kind::tf32 MMA reads is stored TF32-exact, see tf32_round)
+enum class Act { kBf16, kF32, kTf32 };
+
+// f32 -> the nearest TF32 value (round to nearest, ties away from zero, the low 13 mantissa bits cleared), as a float.  The rule of
+// cvt.rna.tf32.f32; a value at or above the midpoint between the largest TF32 value and 2^128 becomes Inf.  Inf stays Inf, NaN stays
+// NaN (a plain add-and-mask would turn a NaN whose payload sits in the low 13 bits into Inf).  Host (weights) and device (epilogues,
+// encode) use this one definition.
+__host__ __device__ __forceinline__ float tf32_round(float x) {
+#ifdef __CUDA_ARCH__
+    uint32_t u = __float_as_uint(x);
+#else
+    uint32_t u;
+    std::memcpy(&u, &x, 4);
+#endif
+    if ((u & 0x7F800000u) != 0x7F800000u)
+        u += 0x1000u;  // finite: half an ulp of TF32 on the magnitude, carries into the exponent
+    else if (u & 0x007FFFFFu)
+        u |= 0x00400000u;  // NaN: quiet bit set, so the payload survives the mask
+    u &= 0xFFFFE000u;
+#ifdef __CUDA_ARCH__
+    return __uint_as_float(u);
+#else
+    std::memcpy(&x, &u, 4);
+    return x;
+#endif
+}
 
 // Row index of square sq = y * W + x of board b inside an activation matrix [rows][channels]: every row is a real square
 struct RowLayout {
@@ -26,7 +55,7 @@ struct EncodeParams {
     int batch, bits_stride, scalar_count, bool_channels;
     RowLayout lay;
     int c_pad;  // channels per row in the output (>= scalar_count + bool_channels, multiple of 8)
-    void* out;  // [batch*W*H][c_pad] bf16 or f32
+    void* out;  // [batch*W*H][c_pad] bf16 or f32 (f32 rounded to TF32 for Act::kTf32)
     // optional board symmetry (RandomSymmetryNetwork on the GPU, network/symmetry.rs:41-67): plane square sq of board b is
     // read from square square_src[sym[b]*A + sq] of the record; null = identity
     const uint8_t* sym;
@@ -34,12 +63,12 @@ struct EncodeParams {
     // k-chunk-major output only: the record's own board (<= 8x8), embedded top-left in the 8x8 grid the tower works on
     int rec_w, rec_h;
 };
-void launch_encode_nhwc(const EncodeParams& p, bool out_bf16, cudaStream_t s);
+void launch_encode_nhwc(const EncodeParams& p, Act out, cudaStream_t s);
 // exact twin of InputMapper::encode_input_full (mapping/mod.rs:40-63): out [batch][Cs+Cb][H*W] f32
 void launch_encode_nchw_f32(const uint8_t* bits, const float* scalars, int batch, int bits_stride, int scalar_count,
                             int bool_channels, int area, float* out, cudaStream_t s);
-// f32 NCHW [batch][C][H*W] -> rows [batch*W*H][c_pad] (bf16 or f32), zero pad channels
-void launch_nchw_to_rows(const float* in, int batch, int channels, RowLayout lay, int c_pad, void* out, bool out_bf16,
+// f32 NCHW [batch][C][H*W] -> rows [batch*W*H][c_pad] of element type `out_type`, zero pad channels
+void launch_nchw_to_rows(const float* in, int batch, int channels, RowLayout lay, int c_pad, void* out, Act out_type,
                          cudaStream_t s);
 
 // ---------------------------------------------------------------------------------------------- conv fp32
@@ -63,16 +92,16 @@ void launch_conv_fp32(const ConvF32Params& p, cudaStream_t s);
 struct ConvTcParams {
     int num_tiles;  // 128-row M tiles
     int taps;       // 1 or 9
-    int kblocks;    // cin_pad / 64
+    int kblocks;    // cin_pad / (channels per 128-byte k-block: 64 bf16 or 32 TF32)
     int cin_pad;
     int n;  // UMMA N = padded cout, multiple of 16, <= 256
     RowLayout lay;
     int valid_rows;  // rows >= valid_rows are not stored
     const float* bias;  // [n]
     int relu_n;
-    const __nv_bfloat16* res;  // optional [rows][res_stride]
+    const void* res;  // optional [rows][res_stride], the activation type
     int res_stride;
-    void* out;  // [rows][out_stride] bf16 or f32
+    void* out;  // [rows][out_stride] bf16 or f32 (conv_i2c TF32: f32 rounded to TF32)
     int out_stride;
     int out_f32;
     int n_store;  // channels written per row (multiple of 16, <= n)
@@ -80,18 +109,19 @@ struct ConvTcParams {
     int tmem_cols;
     int n_split;  // conv_i2c: 1, or 2 = a work item is one 256-pixel tile x one half of the output channels
     int pdl;      // conv_i2c: launched with programmatic stream serialization (set-up and the first weight tiles overlap the previous layer's tail)
+    int tf32;     // operands and activations are f32 rounded to TF32 (tcgen05 kind::tf32, 32 channels per k-block); 0: bf16
 };
-// conv_tc.cu: conv1x1 on dense rows (tmap_a: box (64 channels, 128 rows), tmap_b: weight box (64, p.n))
+// conv_tc.cu: conv1x1 on dense rows (tmap_a: box (one 128-byte k-block of channels, 128 rows), tmap_b: weight box (k-block, p.n))
 void launch_conv_tc(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const ConvTcParams& p, int grid, cudaStream_t s);
 // conv_i2c.cu: conv3x3 / conv1x1 (p.taps) on DENSE rows, activation tiles by TMA im2col, CTA-pair MMA (tmap_bh: weight box of p.n / p.n_split / 2 rows)
 void launch_conv_i2c(const CUtensorMap& tmap_a_im2col, const CUtensorMap& tmap_bh, const CUtensorMap& tmap_out, const CUtensorMap& tmap_res,
                      const ConvTcParams& p, int grid, cudaStream_t s);
-size_t conv_i2c_smem_bytes(int n, int stages);
-int conv_i2c_pick_stages(int n);
+size_t conv_i2c_smem_bytes(int n, int stages, bool tf32);
+int conv_i2c_pick_stages(int n, bool tf32);
 void conv_i2c_prepare();
 size_t conv_tc_smem_bytes(int n, int stages);
 int conv_tc_pick_stages(int n);
-void conv_tc_prepare();  // per-device: opt in to 227 KB dynamic shared memory
+void conv_tc_prepare();  // per-device (both operand types): opt in to 227 KB dynamic shared memory
 
 // whole-tower persistent kernel for 8x8 boards (tower8k.cu)
 struct TowerLayerDev {

@@ -117,6 +117,18 @@ __device__ __forceinline__ uint32_t umma_desc_lo(uint32_t smem_addr) { return (s
 __device__ __forceinline__ uint32_t umma_idesc_bf16(int m, int n) {
     return (1u << 4) | (1u << 7) | (1u << 10) | (uint32_t(n >> 3) << 17) | (uint32_t(m >> 4) << 24);
 }
+// Instruction descriptor, kind::tf32: c=f32 [4,6)=1, a=tf32 [7,10)=2, b=tf32 [10,13)=2, both K-major; N, M as above.
+__device__ __forceinline__ uint32_t umma_idesc_tf32(int m, int n) {
+    return (1u << 4) | (2u << 7) | (2u << 10) | (uint32_t(n >> 3) << 17) | (uint32_t(m >> 4) << 24);
+}
+// the instruction descriptor of one 128-byte-per-row operand type: bf16 (kind::f16) or f32 rounded to TF32 (kind::tf32)
+template <typename T>
+__device__ __forceinline__ uint32_t umma_idesc(int m, int n) {
+    if constexpr (sizeof(T) == 4)
+        return umma_idesc_tf32(m, n);
+    else
+        return umma_idesc_bf16(m, n);
+}
 
 __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
                                           uint32_t accumulate) {
@@ -125,6 +137,17 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t a_desc, uint
         ".reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
+        "}" ::"r"(tmem_d),
+        "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
+                                          uint32_t accumulate) {
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t"
         "}" ::"r"(tmem_d),
         "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
         : "memory");

@@ -26,6 +26,7 @@ from ._abi import KzbError, NetInfo  # noqa: F401
 
 PRECISION_FP32 = 0
 PRECISION_BF16 = 1
+PRECISION_TF32 = 2  # tcgen05 kind::tf32 on the row kernels, f32 activations rounded to TF32 (include/kzb200.h)
 
 
 @dataclass(frozen=True)
