@@ -56,7 +56,10 @@ typedef struct kzb_net_info {
  * with `load_graph_from_onnx_path` + `optimize_graph` (rust/kz-selfplay/src/server/server_alphazero.rs:126-128):
  * parses the ONNX bytes, recognises the ResNet tower + heads, folds every BatchNorm, packs weights,
  * allocates device buffers for `max_batch` positions.  Fails with a message for graphs that are not the
- * reference architecture (python/lib/model/post_act.py). */
+ * reference architecture (python/lib/model/post_act.py).  Widths, in every precision: tower and policy conv1 up to 1024
+ * channels, policy conv2 up to 256 output channels; a wider net fails with a message naming the layer and the limit.  Tensor-core
+ * layers wider than 256 channels run in slices of at most 256 output channels, padded to a multiple of 64 (704 -> 768, 832 -> 896,
+ * so that every slice keeps at least 128 channels). */
 int kzb_net_create_from_onnx(int device, const void* onnx_bytes, size_t onnx_len, int max_batch, int precision,
                              kzb_net** out);
 
@@ -77,6 +80,7 @@ typedef struct kzb_fc_weights {
     const float* w; /* [out][in] (Gemm with transB = 1) */
     const float* b; /* [out] */
 } kzb_fc_weights;
+/* channels and policy_conv1.cout: 1..1024; policy_conv2.cout: at most 256 (see kzb_net_create_from_onnx) */
 typedef struct kzb_net_spec {
     int32_t input_channels, board_h, board_w, channels, depth;
     kzb_conv_weights first;         /* conv3x3 input_channels -> channels, bias, no ReLU (post_act.py:203)             */

@@ -6,11 +6,11 @@
 // corners -1 / -1 for a 3x3 filter with zero padding 1) walks 128 consecutive output pixels across ranks and boards, adds the tap
 // offset and zero-fills whatever falls off the board, so every row the tensor core multiplies is a real square (the padded-row
 // layout it replaced spent 19 % of the MMAs on zero rows on 9x9, 10 % on 19x19).  Each 128-pixel tile is re-loaded per
-// tap (16 KB, SWIZZLE_128B) next to the half weight tile (cout/2 x 64, 16 KB): exactly the shared-memory traffic of a plain
+// tap (16 KB, SWIZZLE_128B) next to the half weight tile (slice/2 x 64, up to 16 KB): exactly the shared-memory traffic of a plain
 // 2-SM GEMM.
 //
 // Two CTAs of a cluster own 256 consecutive pixels (128 each); each stages its own pixels and HALF of every weight tile; the
-// leader issues tcgen05.mma.cta_group::2 with M = 256 and both CTAs' TMEM receive their own 128 rows x n columns.
+// leader issues tcgen05.mma.cta_group::2 with M = 256 and both CTAs' TMEM receive their own 128 rows x (n / n_split) columns.
 // Synchronisation (L = leader = cluster rank 0, P = peer); only L's MMA thread issues, one barrier wait per stage:
 //   full[s] (L's copy)     armed by L's producer with the bytes of BOTH CTAs; P's TMA loads complete their bytes on L's barrier
 //                          (cp.async.bulk.tensor .cta_group::2, peer bit of the barrier address cleared)
@@ -22,7 +22,11 @@
 // arrives by TMA two chunks ahead, is updated IN PLACE and leaves by TMA store -- no per-thread global loads / stores, and a code
 // body of a few hundred instructions (the shared conv_epilogue_tile unrolls to 90 KB of code and kept the epilogue warps busy 80-90 %
 // of a tile's MMA time: profiles/r02_go_kernels.md).
-// p.n_split = 2 (small batches): a work item is one 256-pixel tile x one half of the output channels (M256 N128 MMAs).
+// Output channels in slices (p.n_split): a work item is one 256-pixel tile x one slice of n / n_split output channels, so every MMA
+// has N = n / n_split <= 256 (the cta_group::2 limit; also the largest TMA box and half of a CTA's 512 TMEM columns, since an
+// accumulator pair takes 2 N columns).  Layers wider than 256 always run in slices; small batches split further to fill the SMs
+// (executor.cu).  The bias of a chunk is read from global memory (one 128-byte line, the same for every lane) rather than staged:
+// shared memory and the stage count do not depend on the width.
 // p.pdl: launched with programmatic stream serialization -- set-up and the first weight tiles overlap the previous layer's tail.
 //
 // Two instances, one per operand type T; a k-block is one 128-byte row in either:
@@ -58,7 +62,6 @@ struct SmemLayout {
     uint8_t* staging;  // [epilogue warp][kStgBufs][kStgBytes]
     uint64_t *full, *empty, *tmem_full, *tmem_empty, *res_full;
     uint32_t* tmem_ptr;
-    float* bias;
 };
 
 template <typename T>
@@ -72,7 +75,6 @@ __device__ __forceinline__ SmemLayout carve(uint8_t* base, int stages) {
     s.tmem_empty = s.tmem_full + 2;
     s.res_full = s.tmem_empty + 2;
     s.tmem_ptr = reinterpret_cast<uint32_t*>(s.res_full + 4 * kStgBufs);
-    s.bias = reinterpret_cast<float*>(s.tmem_ptr + 4);
     return s;
 }
 
@@ -172,7 +174,6 @@ __global__ void __launch_bounds__(kThreads, 1)
                      : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
     }
-    for (int i = threadIdx.x; i < p.n; i += kThreads) sm.bias[i] = p.bias[i];
     tc_fence_before();
     __syncthreads();
     cluster_sync_all();  // the peer's barriers exist before anything is committed to / completes on them
@@ -294,6 +295,17 @@ __global__ void __launch_bounds__(kThreads, 1)
 #pragma unroll 1
         for (uint32_t f = 0; f < total; f++) {
             const uint32_t li = f / cpi, c = f - li * cpi, buf = li & 1, sb = f % kStgBufs;
+            int row0, col0;
+            coords(f, row0, col0);
+            float bias[kChunk];  // one 128-byte line, the same address in every lane (a broadcast); issued before the waits below
+#pragma unroll
+            for (int j = 0; j < kChunk / 4; j++) {
+                const float4 b = __ldg(reinterpret_cast<const float4*>(p.bias + col0) + j);
+                bias[4 * j] = b.x;
+                bias[4 * j + 1] = b.y;
+                bias[4 * j + 2] = b.z;
+                bias[4 * j + 3] = b.w;
+            }
             if (c == 0) {
                 mbar_wait(&sm.tmem_full[buf], (li >> 1) & 1);
                 tc_fence_after();
@@ -306,8 +318,6 @@ __global__ void __launch_bounds__(kThreads, 1)
                 __syncwarp();
                 if (lane == 0) mbar_arrive_remote(&sm.tmem_empty[buf], 0);  // the leader's barrier, from either CTA
             }
-            int row0, col0;
-            coords(f, row0, col0);
             if (has_res) {
                 mbar_wait(&res_bar[sb], (f / kStgBufs) & 1);
             } else {
@@ -315,7 +325,6 @@ __global__ void __launch_bounds__(kThreads, 1)
                 __syncwarp();
             }
             uint8_t* row_ptr = stg + sb * kStgBytes + lane * (kChunk * int(sizeof(T)));
-            const float* bias = sm.bias + col0;
 #pragma unroll
             for (int j = 0; j < kChunk / kVec; j++) {  // kVec channels = one 16-byte unit of the row
                 float v[kVec];
@@ -375,16 +384,17 @@ __global__ void __launch_bounds__(kThreads, 1)
 
 }  // namespace
 
-size_t conv_i2c_smem_bytes(int n, int stages, bool tf32) {
+// the same for every layer width: the ring holds up to 128 weight rows per CTA (a slice of <= 256 channels), biases are not staged
+size_t conv_i2c_smem_bytes(int stages, bool tf32) {
     const size_t stg = tf32 ? kStgBytesOf<float> : kStgBytesOf<__nv_bfloat16>;
-    return 1024 /*alignment slack*/ + size_t(stages) * kStageBytes + 4 * kStgBufs * stg + (2 * stages + 4 + 4 * kStgBufs) * 8 + 16 + size_t(n) * 4;
+    return 1024 /*alignment slack*/ + size_t(stages) * kStageBytes + 4 * kStgBufs * stg + (2 * stages + 4 + 4 * kStgBufs) * 8 + 16;
 }
 
 // bf16: 6 stages; TF32: 5 (its staging boxes take 32 KB more)
-int conv_i2c_pick_stages(int n, bool tf32) {
+int conv_i2c_pick_stages(bool tf32) {
     const size_t budget = 227 * 1024;
     int stages = 6;
-    while (stages > 2 && conv_i2c_smem_bytes(n, stages, tf32) > budget) stages--;
+    while (stages > 2 && conv_i2c_smem_bytes(stages, tf32) > budget) stages--;
     return stages;
 }
 
@@ -394,7 +404,7 @@ void conv_i2c_prepare() {
 }
 
 // tmap_a: im2col map over the dense channels-last activations (C, W, H, boards), one k-block x 128 pixels per load, SWIZZLE_128B;
-// tmap_bh: weight map whose box holds p.n / p.n_split / 2 rows; tmap_out / tmap_res: output / residual rows, box (32 channels, 32 rows),
+// tmap_bh: weight map whose box holds p.n / p.n_split / 2 rows (this CTA's half of a slice); tmap_out / tmap_res: output / residual rows, box (32 channels, 32 rows),
 // SWIZZLE_64B for bf16, SWIZZLE_128B for TF32 (tmap_res is only read when p.res is set)
 void launch_conv_i2c(const CUtensorMap& tmap_a, const CUtensorMap& tmap_bh, const CUtensorMap& tmap_out, const CUtensorMap& tmap_res,
                      const ConvTcParams& p, int grid, cudaStream_t s) {
@@ -403,7 +413,7 @@ void launch_conv_i2c(const CUtensorMap& tmap_a, const CUtensorMap& tmap_bh, cons
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(unsigned(2 * std::min(grid / 2, items)));
     cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = conv_i2c_smem_bytes(p.n, p.stages, p.tf32 != 0);
+    cfg.dynamicSmemBytes = conv_i2c_smem_bytes(p.stages, p.tf32 != 0);
     cfg.stream = s;
     cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeClusterDimension;

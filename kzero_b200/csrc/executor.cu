@@ -21,6 +21,27 @@ void cuda_check(cudaError_t e, const char* what) {
 int round_up(int v, int m) { return (v + m - 1) / m * m; }
 size_t align16(size_t v) { return (v + 15) / 16 * 16; }
 
+// Widest tower / policy conv1 the tensor-core and fp32 paths take
+constexpr int kMaxChannels = 1024;
+
+// conv_i2c.cu: the fewest slices an n-channel layer runs in -- each at most 256 output channels (one cta_group::2 MMA, one TMA box,
+// two accumulators in 512 TMEM columns) and a whole number of 32-channel epilogue chunks; 0 if there is no such split
+int base_split(int n) {
+    for (int s = 1; s <= n / 32; s++)
+        if (n % s == 0 && n / s <= 256 && (n / s) % 32 == 0) return s;
+    return 0;
+}
+
+// output width of a conv_i2c layer with c channels: a whole k-block up to 256 channels; above that a multiple of 64 (whole 32-channel
+// chunks in both precisions after the small-batch halving) whose base slices hold at least 128 channels.  Most widths only round
+// up to 64 (288 -> 320); 704 and 832, whose 64-multiples split only into 64-channel slices, become 768 (3 x 256) and 896 (4 x 224).
+int i2c_width(int c, int kb) {
+    if (c <= 256) return round_up(c, kb);
+    int n = round_up(c, 64);
+    while (n / base_split(n) < 128) n += 64;
+    return n;
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -147,8 +168,15 @@ Net::Net(int device, NetSpec spec, int max_batch, int precision)
     if (spec_.scalar_conv.cout + (spec_.has_extra ? 1 : 0) > 16) throw std::runtime_error("scalar head with more than 15 hidden channels is not supported");
     if (spec_.fc1.out > 128) throw std::runtime_error("scalar head hidden size > 128 is not supported");
     if (spec_.has_extra && spec_.extra_fc.out != 1) throw std::runtime_error("policy head with more than one extra move is not supported");
-    if (spec_.channels > 256 || spec_.policy_conv1.cout > 256 || spec_.policy_conv2.cout > 256)
-        throw std::runtime_error("more than 256 channels is not supported");
+    if (spec_.channels > kMaxChannels)
+        throw std::runtime_error("a tower of " + std::to_string(spec_.channels) + " channels is not supported (at most " +
+                                 std::to_string(kMaxChannels) + ")");
+    if (spec_.policy_conv1.cout > kMaxChannels)
+        throw std::runtime_error("policy conv1 with " + std::to_string(spec_.policy_conv1.cout) + " output channels is not supported (at most " +
+                                 std::to_string(kMaxChannels) + ")");
+    if (spec_.policy_conv2.cout > 256)
+        throw std::runtime_error("policy conv2 with " + std::to_string(spec_.policy_conv2.cout) +
+                                 " output channels is not supported (at most 256)");
     if (precision != 0 && (spec_.board_w > 255 || spec_.board_h > 255))  // im2col coordinates
         throw std::runtime_error(std::string("boards wider or taller than 255 squares are not supported in ") + (precision == 1 ? "bf16" : "tf32") +
                                  "; use precision=fp32");
@@ -297,8 +325,8 @@ void Net::build_tc() {
         rows_alloc_ = round_up(std::max(pixels, boards_i2c_ * W * H), 128);
     }
     cin_pad_ = round_up(spec_.cin, kb);
-    c_pad_ = round_up(C, kb);
-    cp_pad_ = round_up(spec_.policy_conv1.cout, kb);
+    c_pad_ = i2c_width(C, kb);
+    cp_pad_ = i2c_width(spec_.policy_conv1.cout, kb);
     pm_stride_ = round_up(spec_.policy_conv2.cout, 16);
     s1_stride_ = 16;
 
@@ -333,17 +361,15 @@ void Net::build_tc() {
         }
         upload(st->bias, padded_bias(c.b, n));
 
-        {
+        // weight map with a box of `rows` output channels x one k-block
+        auto wmap = [&](int rows) {
             uint64_t dims[2] = {uint64_t(ktot), uint64_t(n)};
             uint64_t strides[1] = {uint64_t(ktot) * esz};
-            uint32_t box[2] = {uint32_t(kb), uint32_t(n)};
-            st->tmap_b = make_tmap(st->w_tc.ptr, 2, dims, strides, box, true, false, dtype);
-            st->tmap_bh = st->tmap_b;
-            if (n % 32 == 0) {  // half-height box: each CTA of a pair stages half of every weight tile (conv_i2c.cu)
-                uint32_t half[2] = {uint32_t(kb), uint32_t(n / 2)};
-                st->tmap_bh = make_tmap(st->w_tc.ptr, 2, dims, strides, half, true, false, dtype);
-            }
-        }
+            uint32_t box[2] = {uint32_t(kb), uint32_t(rows)};
+            return make_tmap(st->w_tc.ptr, 2, dims, strides, box, true, false, dtype);
+        };
+        if (n <= 256) st->tmap_b = wmap(n);  // conv_tc.cu and heads8.cu: every output channel in one box
+        int slice = n;                       // output channels per MMA
         if (out_f32) {  // the head convs: 1x1 (net_spec.cpp), conv_tc.cu
             if (st->taps != 1) throw std::logic_error("internal: conv_tc.cu runs 1x1 convs only");
             uint64_t dims[2] = {uint64_t(in_stride), uint64_t(rows_alloc_)};
@@ -360,15 +386,16 @@ void Net::build_tc() {
             };
             st->tmap_out = rows_map(out.ptr, out_stride);
             st->tmap_res = res ? rows_map(res->ptr, c_pad_) : st->tmap_out;
-            st->tmap_bq = st->tmap_bh;
-            if (n % 64 == 0) {
-                uint64_t dims[2] = {uint64_t(ktot), uint64_t(n)};
-                uint64_t strides[1] = {uint64_t(ktot) * esz};
-                uint32_t quarter[2] = {uint32_t(kb), uint32_t(n / 4)};
-                st->tmap_bq = make_tmap(st->w_tc.ptr, 2, dims, strides, quarter, true, false, dtype);
-            }
+            // output channels in split0 slices (twice as many for small batches, run_network); each CTA of a pair stages half of
+            // every weight tile of its slice
+            st->split0 = base_split(n);
+            if (st->split0 == 0) throw std::logic_error("internal: conv_i2c layer of " + std::to_string(n) + " channels has no slicing");
+            slice = n / st->split0;
+            st->split_double = slice % 64 == 0;  // the halved slice is still whole 32-channel chunks
+            st->tmap_w[0] = wmap(slice / 2);
+            st->tmap_w[1] = st->split_double ? wmap(slice / 4) : st->tmap_w[0];
             st->use_i2c = true;
-            st->i2c_stages = conv_i2c_pick_stages(n, tf32);
+            st->i2c_stages = conv_i2c_pick_stages(tf32);
         }
         ConvTcParams& p = st->tc;
         p.taps = st->taps;
@@ -386,8 +413,8 @@ void Net::build_tc() {
         p.out_f32 = out_f32 ? 1 : 0;
         p.n_store = n;
         p.stages = conv_tc_pick_stages(n);
-        int cols = 32;
-        while (cols < 2 * n) cols *= 2;
+        int cols = 32;  // two accumulators of the widest slice
+        while (cols < 2 * slice) cols *= 2;
         p.tmem_cols = cols;
         p.n_split = 1;
         const char* pdl_env = std::getenv("KZB_PDL");  // programmatic dependent launch of consecutive conv_i2c layers (KZB_PDL=0: off)
@@ -742,10 +769,13 @@ void Net::run_network(int batch, const StepHook& hook) {
             p.num_tiles = (p.valid_rows + 127) / 128;
             if (st->use_i2c) {
                 p.stages = st->i2c_stages;
-                // small batches: split the output channels so that twice as many SM pairs share the layer
+                // the output channels in split0 slices of <= 256; small batches: twice the slices, so that twice as many SM pairs
+                // share the layer, when the work items fill at most half of them (KZB_CONV_SPLIT=0: never)
                 const char* split = std::getenv("KZB_CONV_SPLIT");
-                p.n_split = (!(split && split[0] == '0') && p.n % 64 == 0 && p.n_store == p.n && 2 * ((p.num_tiles + 1) / 2) <= num_sms_ / 2) ? 2 : 1;
-                launch_conv_i2c(st->tmap_i2c, p.n_split == 2 ? st->tmap_bq : st->tmap_bh, st->tmap_out, st->tmap_res, p, num_sms_, stream_);
+                const bool dbl = !(split && split[0] == '0') && st->split_double && p.n_store == p.n &&
+                                 2 * ((p.num_tiles + 1) / 2) * st->split0 <= num_sms_ / 2;
+                p.n_split = st->split0 * (dbl ? 2 : 1);
+                launch_conv_i2c(st->tmap_i2c, st->tmap_w[dbl ? 1 : 0], st->tmap_out, st->tmap_res, p, num_sms_, stream_);
             } else {
                 launch_conv_tc(st->tmap_a, st->tmap_b, p, num_sms_, stream_);
             }

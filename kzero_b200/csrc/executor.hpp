@@ -46,11 +46,16 @@ struct ConvStep {
     std::string name;
     int taps = 9;
     // tensor-core form (bf16, or f32 rounded to TF32)
-    CUtensorMap tmap_a{}, tmap_b{}, tmap_bh{};
+    CUtensorMap tmap_a{}, tmap_b{};  // tmap_b: weight box of all n rows (n <= 256 only)
     bool use_i2c = false;  // conv_i2c.cu (TMA im2col, CTA-pair MMA); otherwise conv_tc.cu (1x1, f32 output)
     int i2c_stages = 0;
     CUtensorMap tmap_out{}, tmap_res{};  // conv_i2c: output / residual rows, box (32 channels, 32 rows), SWIZZLE_64B
-    CUtensorMap tmap_i2c{}, tmap_bq{};  // im2col map of the input rows; weight box of n / 4 rows (output channels split in two)
+    CUtensorMap tmap_i2c{};  // im2col map of the input rows
+    // conv_i2c output channel slices: split0 slices of n / split0 <= 256 channels, or (split_double, small batches) 2 * split0;
+    // tmap_w[i]: weight box of half a slice (n / split0 / 2, n / split0 / 4 rows)
+    int split0 = 1;
+    bool split_double = false;
+    CUtensorMap tmap_w[2]{};
     ConvTcParams tc{};
     DeviceBuffer w_tc;  // [n][taps*cin_pad] bf16, or f32 rounded to TF32
     // fp32 form

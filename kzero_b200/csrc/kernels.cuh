@@ -94,7 +94,7 @@ struct ConvTcParams {
     int taps;       // 1 or 9
     int kblocks;    // cin_pad / (channels per 128-byte k-block: 64 bf16 or 32 TF32)
     int cin_pad;
-    int n;  // UMMA N = padded cout, multiple of 16, <= 256
+    int n;  // padded cout: conv_tc UMMA N, multiple of 16, <= 256; conv_i2c multiple of 32, <= 1024 (UMMA N = n / n_split <= 256)
     RowLayout lay;
     int valid_rows;  // rows >= valid_rows are not stored
     const float* bias;  // [n]
@@ -107,7 +107,7 @@ struct ConvTcParams {
     int n_store;  // channels written per row (multiple of 16, <= n)
     int stages;
     int tmem_cols;
-    int n_split;  // conv_i2c: 1, or 2 = a work item is one 256-pixel tile x one half of the output channels
+    int n_split;  // conv_i2c: slices of the output channels; a work item is one 256-pixel tile x n / n_split channels (n / n_split <= 256, multiple of 32)
     int pdl;      // conv_i2c: launched with programmatic stream serialization (set-up and the first weight tiles overlap the previous layer's tail)
     int tf32;     // operands and activations are f32 rounded to TF32 (tcgen05 kind::tf32, 32 channels per k-block); 0: bf16
 };
@@ -116,8 +116,8 @@ void launch_conv_tc(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const 
 // conv_i2c.cu: conv3x3 / conv1x1 (p.taps) on DENSE rows, activation tiles by TMA im2col, CTA-pair MMA (tmap_bh: weight box of p.n / p.n_split / 2 rows)
 void launch_conv_i2c(const CUtensorMap& tmap_a_im2col, const CUtensorMap& tmap_bh, const CUtensorMap& tmap_out, const CUtensorMap& tmap_res,
                      const ConvTcParams& p, int grid, cudaStream_t s);
-size_t conv_i2c_smem_bytes(int n, int stages, bool tf32);
-int conv_i2c_pick_stages(int n, bool tf32);
+size_t conv_i2c_smem_bytes(int stages, bool tf32);
+int conv_i2c_pick_stages(bool tf32);
 void conv_i2c_prepare();
 size_t conv_tc_smem_bytes(int n, int stages);
 int conv_tc_pick_stages(int n);
