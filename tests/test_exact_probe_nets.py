@@ -18,6 +18,10 @@ A net that violates them fails there; it never quietly weakens the comparison.
 Then evaluate_planes must return the reference's scalars and logits exactly, in bf16 and fp32 and under every kernel switch.
 evaluate_packed returns moves_left exactly; value, WDL and probabilities go through expf / tanhf and are held to a bound built
 from CUDA's documented errors (2 ulp for expf and tanhf, IEEE division, n 2^-24 relative for an n-term sum of positive terms).
+
+The batches reach the sizes where the persistent kernels loop: tower8k up to 16 units per CTA (9,472 boards), heads8 up to 32
+tiles per CTA, conv_i2c over many waves of pair tiles; test_rows_past_the_batch_do_not_leak leaves NaN rows behind the batch.
+The values these nets store are exact in bf16 and TF32, so the rounding on store is checked by test_rounding_probes.py.
 """
 import functools
 from dataclasses import dataclass
@@ -32,9 +36,10 @@ import oracle
 from helpers import bf16_round
 from oracle.graph_exec import OnnxOracle
 from kzero_b200 import mapping, netgen
-from kzero_b200.network import B200Network, Mapper, PRECISION_BF16, PRECISION_FP32, RawWeights
+from kzero_b200.network import B200Network, KzbError, Mapper, PRECISION_BF16, PRECISION_FP32, PRECISION_TF32, RawWeights
 
-BF16, FP32 = PRECISION_BF16, PRECISION_FP32
+BF16, FP32, TF32 = PRECISION_BF16, PRECISION_FP32, PRECISION_TF32
+PRECISION_NAMES = {BF16: "bf16", TF32: "tf32", FP32: "fp32"}
 U = 2.0 ** -24  # unit roundoff of f32
 BN_EPS = np.float32(1e-5)
 IDENTITY_VAR = np.float32(1 - 1e-5)  # with eps: an f32 BatchNormalization that is exactly the identity
@@ -64,6 +69,27 @@ class Case:
 V = lambda **env: tuple(sorted(env.items()))  # noqa: E731
 NO_HEADS8, NO_TOWER8 = V(KZB_NO_HEADS8="1"), V(KZB_NO_TOWER8="1")
 TAIL_8X8 = 6  # encode, tower8k, policy conv1, scalar conv, policy conv2, tail kernel
+GO = lambda depth: 2 * depth + 6  # noqa: E731  encode, 2 depth + 1 tower convs, policy conv1, scalar conv, policy conv2, tail
+PDL0, B_SLOTS2 = V(KZB_PDL="0"), V(KZB_B_SLOTS="2")
+
+# The large batches below are chosen for a B200's 148 SMs (74 SM pairs), as are the unit and tile counts of the older cases.
+# tower8k, uniform scheme (outside the balanced band of 6..8 boards per CTA): 4-board units, their count rounded up to even.
+#   1186: 298 units, 2 to 3 per CTA;  4001: 1002 units, 6 to 7 per CTA, the last real unit holds 1 board, then a padding unit;
+#   9469: 2368 units, 16 per CTA (kMaxLocalUnits), the last unit holds 1 board;  9472: the same, every unit full.
+#   Depth 2: five layers, so every ready[] barrier changes phase at least 4 times.  heads8 at 9472: 4736 tiles, 32 per CTA.
+# conv_i2c, 128-row tiles in pairs: go-19 b400 1129 tiles (565 pair tiles over 74 clusters); raw-19x9 b120 161 tiles, so the last
+# pair's second CTA lies wholly past the batch; go-9 b116 74 tiles (37 pair tiles: the split doubles), b117 75 tiles (38: it does not).
+LARGE = [
+    Case("chess-c32-d2-b1186", channels=32, depth=2, batch=1186, max_batch=9472, launches=3),
+    Case("chess-c32-d2-b4001", channels=32, depth=2, batch=4001, max_batch=9472, launches=3, variants=(PDL0, B_SLOTS2)),
+    Case("chess-c32-d2-b9469", channels=32, depth=2, batch=9469, max_batch=9472, launches=3),
+    Case("chess-c32-d2-b9472", channels=32, depth=2, batch=9472, launches=3, variants=(NO_HEADS8, PDL0, B_SLOTS2)),
+    Case("chess-c96-d2-b3000", channels=96, depth=2, batch=3000, max_batch=9472, launches=3, variants=(NO_HEADS8,)),
+    Case("ataxx-5-b4001", game="ataxx-5", channels=32, depth=2, batch=4001, launches=3, variants=(PDL0,)),
+    Case("go-19-c64-b400", game="go-19", channels=64, depth=1, batch=400, launches=GO(1), variants=(PDL0,)),
+    Case("raw-19x9-b120", game=None, board=(19, 9), channels=64, depth=1, batch=120, launches=GO(1)),
+    *[Case(f"go-9-c192-b{n}", game="go-9", channels=192, depth=1, batch=n, launches=GO(1)) for n in (116, 117)],
+]
 
 CASES = [
     # ---- tower8k + heads8 (encode, tower8k, heads8: 3 launches)
@@ -75,7 +101,7 @@ CASES = [
     Case("chess-c128-d0-b5", channels=128, depth=0, batch=5, launches=3),
     Case("chess-c40-d3-b1", channels=40, depth=3, batch=1, launches=3),
     Case("chess-c72-d0-b3", channels=72, depth=0, batch=3, launches=3, variants=(NO_TOWER8,)),
-    Case("chess-16x128-b1024", channels=128, depth=16, batch=1024, launches=3),
+    Case("chess-16x128-b1024", channels=128, depth=16, batch=1024, launches=3, variants=(V(KZB_NO_BALANCE="1"),)),
     *[Case(f"chess-c64-b{n}", channels=64, depth=1, batch=n, launches=3) for n in (887, 888, 1184, 1185)],
     Case("chess-c64-max9472", channels=64, depth=1, batch=16, max_batch=9472, launches=3),
     Case("chess-c64-max9473", channels=64, depth=1, batch=16, max_batch=9473, launches=2 * 1 + 3),  # conv_i2c per layer, heads8
@@ -104,6 +130,7 @@ CASES = [
     *[Case(f"go-19-hc{hc}", game="go-19", channels=64, hc=hc, batch=5) for hc in (1, 9, 15)],
     *[Case(f"att-q{q}", game="chess-att", channels=128 if q == 128 else 32, q=q, batch=5) for q in (16, 64, 128)],
     Case("go-256-fp32", game="go-256", channels=8, depth=1, batch=1, precisions=(FP32,)),
+    *LARGE,
 ]
 CASE_IDS = [c.id for c in CASES]
 assert len(set(CASE_IDS)) == len(CASE_IDS)
@@ -389,14 +416,7 @@ def reference(net: Net, planes, check=False, fault=None):
         bulk_w, under_w, q = net.att
         bulk = head_conv(bulk_w, x, "attention bulk conv", False, stored_bf16=False)
         under = head_conv(under_w, x[:, :, 7:8, :], "attention under conv", False, stored_bf16=False)
-        qf = bulk[:, :q].reshape(n, q, 64)
-        qto = np.concatenate([bulk[:, q:].reshape(n, q, 64), under.reshape(n, q, 24)], axis=2)
-        mm = np.einsum("nqf,nqt->nft", qf, qto)
-        if check:
-            assert_exact_sum("attention dot", qf, qto, 0.0, np.einsum("nqf,nqt->nft", np.abs(qf), np.abs(qto)))
-        # one IEEE f32 division by the f32 constant the graph holds, as the oracle's Div and the tail kernel do
-        att = mm.astype(np.float32) / np.array(float(q) ** 0.5, dtype=np.float32)
-        logits = att.reshape(n, -1)[:, mapping.chess_flat_to_att()].astype(np.float64)
+        logits = attention_logits(bulk, under, q, check)
     else:
         h1 = head_conv(net.policy_conv1, x, "policy conv1", True)
         pm = head_conv(net.policy_conv2, h1, "policy conv2", False, stored_bf16=False).reshape(n, -1)
@@ -409,6 +429,19 @@ def reference(net: Net, planes, check=False, fault=None):
     if check:
         assert np.array_equal(scalars.astype(np.float32), scalars) and np.array_equal(logits.astype(np.float32), logits)
     return scalars, logits
+
+
+def attention_logits(bulk, under, q, check):
+    """The chess attention head's logits from the f32 outputs of its two convs."""
+    n = bulk.shape[0]
+    qf = bulk[:, :q].reshape(n, q, 64)
+    qto = np.concatenate([bulk[:, q:].reshape(n, q, 64), under.reshape(n, q, 24)], axis=2)
+    mm = np.einsum("nqf,nqt->nft", qf, qto)
+    if check:
+        assert_exact_sum("attention dot", qf, qto, 0.0, np.einsum("nqf,nqt->nft", np.abs(qf), np.abs(qto)))
+    # one IEEE f32 division by the f32 constant the graph holds, as the oracle's Div and the tail kernel do
+    att = mm.astype(np.float32) / np.array(float(q) ** 0.5, dtype=np.float32)
+    return att.reshape(n, -1)[:, mapping.chess_flat_to_att()].astype(np.float64)
 
 
 def decode64(scalars, logits, mv_idx, mv_off):
@@ -576,10 +609,37 @@ def test_faults_change_the_probe_outputs(capsys):
 
 
 # ----------------------------------------------------------------------------------------------------------- GPU matrix
-def run_gpu(case: Case, precision, env, monkeypatch, stats):
+def expected(ref_s, ref_p, mv_idx, mv_off):
+    """-> (scalars, logits, values, probabilities, bound on values, bound on probabilities) the GPU must meet."""
+    return (ref_s, ref_p) + decode64(ref_s, ref_p, mv_idx, mv_off)
+
+
+@functools.lru_cache(maxsize=8)
+def case_reference(case: Case):
+    """expected() of a case, computed once and shared by every precision and switch."""
     b = build(case)
-    ref_s, ref_p = reference(b.net, b.planes)
-    ref_v, ref_probs, bound_v, bound_p = decode64(ref_s, ref_p, b.mv_idx, b.mv_off)
+    return expected(*reference(b.net, b.planes), b.mv_idx, b.mv_off)
+
+
+def compare(tag, ref, s, p, values, probs, stats):
+    """Scalars, logits and moves_left bit for bit, the decoded values and probabilities within their bounds."""
+    ref_s, ref_p, ref_v, ref_probs, bound_v, bound_p = ref
+    assert np.array_equal(s, ref_s.astype(np.float32)), f"{tag}: scalars differ in {np.count_nonzero(s != ref_s)} places"
+    bad = np.argwhere(p != ref_p)
+    assert bad.size == 0, f"{tag}: {len(bad)} logits differ, first (board, index) {bad[:4].tolist()}"
+    assert np.array_equal(values[:, 4], ref_s[:, 4].astype(np.float32)), tag
+    err_v = np.abs(values - ref_v)
+    err_p = np.abs(probs - ref_probs)
+    assert (err_v <= bound_v).all(), f"{tag}: values off by {err_v.max()}"
+    assert (err_p <= bound_p).all(), f"{tag}: probabilities off by {err_p.max()}"
+    stats.append(max((err_v[:, :4] / bound_v[:, :4]).max(), (err_p / bound_p).max() if err_p.size else 0.0))
+
+
+def run_gpu(case: Case, precision, env, monkeypatch, stats, b=None, ref=None):
+    """One network of the case in one precision under the switches env, against the reference (by default the case's net and
+    inputs and their float64 reference; b and ref replace both)."""
+    if b is None:
+        b, ref = build(case), case_reference(case)
     for key, val in env:
         monkeypatch.setenv(key, val)
     try:
@@ -591,16 +651,7 @@ def run_gpu(case: Case, precision, env, monkeypatch, stats):
     finally:
         for key, _ in env:
             monkeypatch.delenv(key)
-    tag = f"{case.id} {'bf16' if precision == BF16 else 'fp32'} {dict(env) or 'default'}"
-    assert np.array_equal(s, ref_s.astype(np.float32)), f"{tag}: scalars differ in {np.count_nonzero(s != ref_s)} places"
-    bad = np.argwhere(p != ref_p)
-    assert bad.size == 0, f"{tag}: {len(bad)} logits differ, first (board, index) {bad[:4].tolist()}"
-    assert np.array_equal(values[:, 4], ref_s[:, 4].astype(np.float32)), tag
-    err_v = np.abs(values - ref_v)
-    err_p = np.abs(probs - ref_probs)
-    assert (err_v <= bound_v).all(), f"{tag}: values off by {err_v.max()}"
-    assert (err_p <= bound_p).all(), f"{tag}: probabilities off by {err_p.max()}"
-    stats.append(max((err_v[:, :4] / bound_v[:, :4]).max(), (err_p / bound_p).max() if err_p.size else 0.0))
+    compare(f"{case.id} {PRECISION_NAMES[precision]} {dict(env) or 'default'}", ref, s, p, values, probs, stats)
     return p
 
 
@@ -632,3 +683,27 @@ def test_raw_weights_equal_the_onnx_net(case_id):
                 outs.append(net.evaluate_planes(b.planes) + net.evaluate_packed(b.bits, b.scalars, b.mv_idx, b.mv_off))
         for x, y in zip(*outs):
             assert np.array_equal(x, y)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("case_id", ["chess-c32-d2-b9469", "go-19-c64-b400"])
+@pytest.mark.parametrize("precision", [BF16, TF32], ids=["bf16", "tf32"])
+def test_rows_past_the_batch_do_not_leak(case_id, precision):
+    """Row i is independent of the other rows and of batch (DESIGN §1), also of rows an earlier call left behind.  A call on
+    three more boards, whose scalars are NaN, fails and leaves NaN in every activation buffer behind the batch; the next call's
+    last tower8k unit, heads8 tile or conv pair tile holds those rows, and its results must still equal the reference."""
+    case = BY_ID[case_id]
+    b = build(case)
+    n = case.batch
+    assert case.max_batch in (0, n + 3)
+    counts = np.diff(b.mv_off.astype(np.int64))
+    last = slice(int(b.mv_off[n - 3]), int(b.mv_off[n]))
+    mv_off = np.concatenate([b.mv_off, b.mv_off[n] + np.cumsum(counts[-3:])]).astype(np.uint32)
+    nan_scalars = np.full((3, b.scalars.shape[1]), np.nan, np.float32)
+    with B200Network(b.mapper, creation(case, b), n + 3, precision=precision) as net:
+        with pytest.raises(KzbError, match="strictly positive"):
+            net.evaluate_packed(np.concatenate([b.bits, b.bits[-3:]]), np.concatenate([b.scalars, nan_scalars]),
+                                np.concatenate([b.mv_idx, b.mv_idx[last]]), mv_off)
+        s, p = net.evaluate_planes(b.planes)
+        values, probs = net.evaluate_packed(b.bits, b.scalars, b.mv_idx, b.mv_off)
+    compare(f"{case_id} {PRECISION_NAMES[precision]} after NaN rows", case_reference(case), s, p, values, probs, [])

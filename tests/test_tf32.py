@@ -6,9 +6,9 @@ tf32_round in kzero_b200/csrc/kernels.cuh), so the results do not depend on what
 CPU: the host rounding on known bit patterns; a CPU emulation of the TF32 arithmetic (every Conv operand and every residual Add
 rounded to TF32, f32 accumulation) stays below half of the GPU bar on deep towers; the exact-arithmetic probe nets are TF32-exact;
 precision values are checked.
-GPU: the probe matrix bit for bit against the float64 reference; random-init nets against the f32 oracle within
-4e-3 * max(1, max |logit|) on logits and raw scalars and 1e-3 on probabilities; batch independence, graph replay, the packed decode,
-NaN reporting, the launch count of an 8x8 net (it takes the row path), and self-play.
+GPU: the probe matrix bit for bit against the float64 reference (the rounding on store: test_rounding_probes.py); random-init
+nets against the f32 oracle within 4e-3 * max(1, max |logit|) on logits and raw scalars and 1e-3 on probabilities; batch
+independence, graph replay, the packed decode, NaN reporting, the launch count of an 8x8 net (it takes the row path), and self-play.
 """
 import subprocess
 from pathlib import Path
@@ -238,106 +238,6 @@ def test_tf32_raw_weights_equal_the_onnx_net(case_id):
             outs.append(net.evaluate_planes(b.planes) + net.evaluate_packed(b.bits, b.scalars, b.mv_idx, b.mv_off))
     for x, y in zip(*outs):
         assert np.array_equal(x, y)
-
-
-# ----------------------------------------------------------------------------------------------------------- rounding on store
-# The probe nets above are TF32-exact, so the epilogues' rounding never changes a value there.  These nets are the probe nets with
-# the first conv's weights and every tower and head bias scaled by ROUND_SCALE: every value stays an integer (or on the 2^-5 / 2^-6
-# grid of the heads), every f32 sum stays exact, but the tower outputs reach 2^16, where most integers are not TF32 values.  The
-# reference applies the path's rounding (round to nearest, ties away) to exactly what the GPU stores TF32-rounded: every tower
-# layer's output, the residual stream, policy conv1's output.  A path that skipped the rounding, rounded differently or rounded
-# the f32 head outputs would differ from it.
-ROUND_SCALE = 257.0
-ROUND_CASES = ["chess-c40-d1-b3", "go-9-c192-b7", "raw-19x9", "ataxx-5"]
-
-
-def _rounding_net(case_id):
-    from dataclasses import replace
-
-    b = probes.build(probes.BY_ID[case_id])
-    net = b.net
-    k = ROUND_SCALE
-    scaled = replace(net, first=(net.first[0] * k, net.first[1] * k), blocks=[(w, bias * k) for w, bias in net.blocks],
-                     scalar_conv=(net.scalar_conv[0], net.scalar_conv[1] * k), fc1=(net.fc1[0], net.fc1[1] * k),
-                     fc2=(net.fc2[0], net.fc2[1] * k), policy_conv1=(net.policy_conv1[0], net.policy_conv1[1] * k),
-                     policy_conv2=(net.policy_conv2[0], net.policy_conv2[1] * k))
-    if net.extra_conv is not None:
-        scaled = replace(scaled, extra_conv=(net.extra_conv[0], net.extra_conv[1] * k), extra_fc=(net.extra_fc[0], net.extra_fc[1] * k))
-    return b, scaled
-
-
-def _reference_tf32_stores(net, planes):
-    """float64 forward pass with the TF32 path's stores -> (scalars, logits, number of stored values the rounding changed).  Asserts
-    that every value is f32-exact before it is rounded and that every sum is exact in f32."""
-    n = planes.shape[0]
-    changed = [0]
-
-    def store(name, a):
-        f = a.astype(np.float32)
-        assert np.array_equal(f.astype(np.float64), a), f"{name}: not f32-exact before rounding"
-        r = tf32_round(f).astype(np.float64)
-        changed[0] += int((r != a).sum())
-        return r
-
-    def conv(name, xin, wb):
-        w, b = wb
-        probes.assert_exact_sum(name, xin, w, b, probes.conv64(np.abs(xin), np.abs(w), np.abs(b)))
-        return probes.conv64(xin, w, b)
-
-    def fc(name, xin, wb):
-        w, b = wb
-        probes.assert_exact_sum(name, xin, w, b, np.abs(xin) @ np.abs(w).T + np.abs(b))
-        return xin @ w.T + b
-
-    x = store("first conv", conv("first conv", planes.astype(np.float64), net.first))
-    for d in range(len(net.blocks) // 2):
-        t = store(f"block{d} conv1", probes.relu(conv(f"block{d} conv1", x, net.blocks[2 * d])))
-        x = store(f"block{d} output", x + probes.relu(conv(f"block{d} conv2", t, net.blocks[2 * d + 1])))
-    s1 = probes.relu(conv("scalar conv", x, net.scalar_conv))  # f32 outputs of the head convs: not rounded
-    scalars = fc("fc2", probes.relu(fc("fc1", s1.reshape(n, -1), net.fc1)), net.fc2)
-    h1 = store("policy conv1", probes.relu(conv("policy conv1", x, net.policy_conv1)))
-    pm = conv("policy conv2", h1, net.policy_conv2).reshape(n, -1)
-    src = net.policy_src
-    logits = np.where(src >= 0, pm[:, np.maximum(src, 0)], 0.0)
-    if net.extra_conv is not None:
-        e = conv("extra conv", x, net.extra_conv)
-        logits = np.where(src == -2, fc("extra fc", e.reshape(n, -1), net.extra_fc), logits)
-    assert np.array_equal(scalars.astype(np.float32), scalars) and np.array_equal(logits.astype(np.float32), logits)
-    return scalars, logits, changed[0]
-
-
-@pytest.mark.parametrize("case_id", ROUND_CASES)
-def test_rounding_probe_nets_are_exact_and_exercise_the_rounding(case_id):
-    b, net = _rounding_net(case_id)
-    _, _, changed = _reference_tf32_stores(net, b.planes)
-    assert changed > 0.05 * b.planes.shape[0] * b.planes.shape[2] * b.planes.shape[3]  # the rounding matters on these nets
-    # the host rounding keeps the conv weights (the biases are added in f32 by the epilogue and are not rounded)
-    w = [net.first[0], net.scalar_conv[0], net.policy_conv1[0], net.policy_conv2[0]] + [wb[0] for wb in net.blocks]
-    assert all(np.array_equal(tf32_round(np.float32(a)), np.float32(a)) for a in w)
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("case_id", ROUND_CASES)
-def test_tf32_stores_are_rounded_like_the_reference(case_id, monkeypatch):
-    """Scalars, logits and moves_left bit-identical to the reference that rounds every stored MMA operand to TF32."""
-    b, net = _rounding_net(case_id)
-    ref_s, ref_p, _ = _reference_tf32_stores(net, b.planes)
-    case = probes.BY_ID[case_id]
-    for env in SWITCHES:
-        for key, val in env:
-            monkeypatch.setenv(key, val)
-        try:
-            with B200Network(b.mapper, probes.raw_weights(net), case.max_batch or case.batch, precision=TF32) as gnet:
-                s, p = gnet.evaluate_planes(b.planes)
-                values, _ = gnet.evaluate_packed(b.bits, b.scalars, b.mv_idx, b.mv_off)
-        finally:
-            for key, _ in env:
-                monkeypatch.delenv(key)
-        tag = f"{case_id} {dict(env) or 'default'}"
-        assert np.array_equal(s, ref_s.astype(np.float32)), f"{tag}: scalars differ in {np.count_nonzero(s != ref_s)} places"
-        bad = np.argwhere(p != ref_p)
-        assert bad.size == 0, f"{tag}: {len(bad)} logits differ, first (board, index) {bad[:4].tolist()}"
-        assert np.array_equal(values[:, 4], ref_s[:, 4].astype(np.float32)), tag
 
 
 # ----------------------------------------------------------------------------------------------------------- GPU: random-init parity

@@ -18,8 +18,6 @@ CPU: the probe preconditions (bf16- and TF32-exact, exact f32 sums) and the f32 
 GPU: the probe nets bit for bit in every precision and under KZB_PDL=0 / KZB_CONV_SPLIT=0, the launch count of the 256-wide net,
 raw-weight and ONNX creation, rows independent of batch and split, random-init parity at size, and the limits' messages.
 """
-import functools
-
 import numpy as np
 import pytest
 
@@ -33,7 +31,7 @@ from kzero_b200.network import B200Network, KzbError, PRECISION_BF16, PRECISION_
 BF16, TF32, FP32 = PRECISION_BF16, PRECISION_TF32, PRECISION_FP32
 BF16_TOL = 2e-2  # logits: BF16_TOL * max(1, max |logit|)
 Case = probes.Case
-GO = lambda depth: 2 * depth + 6  # noqa: E731  encode, 2 depth + 1 tower convs, policy conv1, scalar conv, policy conv2, tail
+GO = probes.GO
 
 # `launches`: bf16 launches_per_eval, the count of the same net at 256 channels
 WIDE = [
@@ -51,15 +49,6 @@ WIDE_IDS = [c.id for c in WIDE]
 BY_ID = {c.id: c for c in WIDE}
 assert not set(WIDE_IDS) & set(probes.CASE_IDS)
 SWITCHES = ((), probes.V(KZB_PDL="0"), probes.V(KZB_CONV_SPLIT="0"))
-
-
-_probe_reference = probes.reference
-
-
-@functools.lru_cache(maxsize=None)
-def _reference(case_id):
-    b = probes.build(BY_ID[case_id])
-    return _probe_reference(b.net, b.planes)
 
 
 # ----------------------------------------------------------------------------------------------------------- CPU
@@ -100,8 +89,6 @@ def test_wide_equals_float64_reference(case_id, monkeypatch, capsys):
     and fp32; the packed decode within the bounds of test_exact_probe_nets; the bf16 launch count that of the 256-wide net."""
     case = BY_ID[case_id]
     stats = []
-    # run_gpu recomputes the reference on every call; it is the same for every precision and switch
-    monkeypatch.setattr(probes, "reference", lambda net, planes: _reference(case_id))
     for precision in (BF16, TF32):
         for env in SWITCHES:
             probes.run_gpu(case, precision, env, monkeypatch, stats)
