@@ -18,7 +18,7 @@ CSRC = PKG / "csrc"
 OBJ = PKG / "_obj"
 LIB = PKG / "libkzb200.so"
 
-SOURCES = ["onnx_reader.cpp", "net_spec.cpp", "api.cpp", "executor.cu", "encode.cu", "conv_fp32.cu", "conv_tc.cu", "conv_i2c.cu", "tower8k.cu", "heads.cu", "heads8.cu", "selfplay/selfplay.cpp"]
+SOURCES = ["onnx_reader.cpp", "net_spec.cpp", "api.cpp", "executor.cu", "encode.cu", "conv_fp32.cu", "conv_i2c.cu", "tower8k.cu", "heads.cu", "heads8.cu", "selfplay/selfplay.cpp"]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--expt-relaxed-constexpr",
               "-Xcompiler", "-fPIC,-fvisibility=hidden,-Wall,-Wno-unknown-pragmas", "-Xptxas", "-v"]

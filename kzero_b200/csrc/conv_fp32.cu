@@ -1,7 +1,7 @@
 // fp32-accurate conv (precision 0): CUDA-core implicit GEMM, plain FMA, no TF32, no tensor cores.
 // Exists so the whole path can be checked against the oracle at <= 1e-4 max-abs (BASELINE.json
 // north_star "fp32 path"), and so index arithmetic of the tensor-core path has an on-device twin.
-// It is a correctness mode, not the throughput mode: the bf16 tcgen05 kernel in conv_tc.cu is.
+// It is a correctness mode, not the throughput mode: the bf16 tcgen05 kernels in tower8k.cu and conv_i2c.cu are.
 //
 // GEMM view: M = positions (batch*H*W), N = cout, K = taps*cin.  Tile 64x64x16, 256 threads, 4x4 per thread.
 #include "kernels.cuh"

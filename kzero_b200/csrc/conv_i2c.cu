@@ -1,5 +1,5 @@
-// K1i: conv3x3 (and conv1x1: p.taps = 1) as an implicit GEMM on DENSE rows -- TMA im2col loads + the CTA-pair MMA.  The 3x3 layers of every board the
-// 8x8 whole-tower kernel does not cover (go 9x9 / 19x19, wide nets).
+// K1i: conv3x3 (and conv1x1: p.taps = 1) as an implicit GEMM on DENSE rows -- TMA im2col loads + the CTA-pair MMA.  The layers of every board the
+// 8x8 whole-tower kernel does not cover (go 9x9 / 19x19, wide nets), and the head 1x1 convs of every net the fused heads kernel does not cover.
 //
 // GEMM view: D[pixels, cout] += A_tap[pixels, 64 ch] * W_tap[cout, 64 ch] over 9 taps x cin/64 k-blocks.  Activations are plain
 // channels-last rows [board][y][x][C] with NO padding rows: the TMA engine's im2col mode (cuTensorMapEncodeIm2col, bounding box
@@ -20,8 +20,8 @@
 // Epilogue (warps 2..5, one TMEM lane quarter = 32 pixel rows each; thread = row): 32 output channels at a time,
 // tcgen05.ld -> +bias -> relu -> +residual -> bf16, through a per-warp ring of four 2 KB SWIZZLE_64B staging boxes: the residual box
 // arrives by TMA two chunks ahead, is updated IN PLACE and leaves by TMA store -- no per-thread global loads / stores, and a code
-// body of a few hundred instructions (the shared conv_epilogue_tile unrolls to 90 KB of code and kept the epilogue warps busy 80-90 %
-// of a tile's MMA time: profiles/r02_go_kernels.md).
+// body of a few hundred instructions (a per-thread epilogue with global loads / stores unrolled to 90 KB of code and kept the
+// epilogue warps busy 80-90 % of a tile's MMA time: profiles/r02_go_kernels.md).
 // Output channels in slices (p.n_split): a work item is one 256-pixel tile x one slice of n / n_split output channels, so every MMA
 // has N = n / n_split <= 256 (the cta_group::2 limit; also the largest TMA box and half of a CTA's 512 TMEM columns, since an
 // accumulator pair takes 2 N columns).  Layers wider than 256 always run in slices; small batches split further to fill the SMs
@@ -32,9 +32,18 @@
 // Two instances, one per operand type T; a k-block is one 128-byte row in either:
 //   bf16  (p.tf32 = 0): 64 channels per k-block, kind::f16 MMAs of K = 16, bf16 rows, 2 KB SWIZZLE_64B staging boxes
 //   float (p.tf32 = 1): 32 channels per k-block, kind::tf32 MMAs of K = 8 on f32 values that are TF32-exact; f32 rows, 4 KB
-//                       SWIZZLE_128B staging boxes, and every stored value rounded to TF32 (tf32_round), since it is the next
-//                       layer's MMA operand.  Twice the k-blocks of bf16 for the same channels, so twice the stages per layer.
+//                       SWIZZLE_128B staging boxes, and every value the tower form stores rounded to TF32 (tf32_round), since it is
+//                       the next layer's MMA operand.  Twice the k-blocks of bf16 for the same channels, so twice the stages per layer.
 // Stages, the pair logic, PDL, n_split and the barrier protocol are the same in both.
+//
+// Each comes in two forms (kHead, p.head) that differ only in the epilogue:
+//   tower form: relu on the whole layer or none, optional residual, output in the operand type (the next layer's MMA operand)
+//   head form (the head 1x1 convs: scalar conv merged with the extra policy conv, policy conv2, the attention convs): relu on output
+//               channels < p.relu_n, no residual, f32 output that is NOT rounded (the tail kernel's CUDA-core FCs read it), through
+//               4 KB SWIZZLE_128B staging boxes in both operand types.  The MMA width p.n is the stored width rounded up to 32; the
+//               output map's inner dimension is the stored width, so the TMA store clips the padding columns.
+#include <type_traits>
+
 #include "kernels.cuh"
 #include "tc_common.cuh"
 
@@ -132,15 +141,16 @@ __device__ __forceinline__ void umma2_commit(uint64_t* bar) {  // arrives on `ba
                  : "memory");
 }
 
-template <typename T>
+template <typename T, bool kHead>
 __global__ void __launch_bounds__(kThreads, 1)
     conv_i2c_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_bh, const __grid_constant__ CUtensorMap tmap_out,
                     const __grid_constant__ CUtensorMap tmap_res, const ConvTcParams p) {
+    using Out = std::conditional_t<kHead, float, T>;  // element type of the stored output
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    const SmemLayout sm = carve<T>(smem, p.stages);
+    const SmemLayout sm = carve<Out>(smem, p.stages);
     constexpr int kBlockK = kBlockKOf<T>;
-    constexpr uint32_t kStgBytes = kStgBytesOf<T>;
+    constexpr uint32_t kStgBytes = kStgBytesOf<Out>;
     const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
     const uint32_t rank = cluster_ctarank();
     const bool leader = rank == 0;
@@ -265,8 +275,8 @@ __global__ void __launch_bounds__(kThreads, 1)
         const int quarter = warp % 4;  // TMEM lanes [32*quarter, 32*quarter+32) are the ones this warp may read
         uint8_t* stg = sm.staging + size_t(quarter) * kStgBufs * kStgBytes;
         uint64_t* res_bar = sm.res_full + quarter * kStgBufs;
-        const bool has_res = p.res != nullptr;
-        const bool relu = p.relu_n > 0;  // whole layers only (the executor checks relu_n is 0 or n)
+        const bool has_res = !kHead && p.has_res;
+        const bool relu = p.relu_n > 0;  // tower form: whole layers only (relu_n is 0 or n)
         const uint32_t cpi = uint32_t(n_eff / kChunk);  // chunks per work item
         const uint32_t local_items = cluster_id < num_items ? uint32_t((num_items - cluster_id + num_clusters - 1) / num_clusters) : 0u;
         const uint32_t total = local_items * cpi;
@@ -290,8 +300,8 @@ __global__ void __launch_bounds__(kThreads, 1)
         }
         // 16-byte chunk index ^ the address bits above the row: SWIZZLE_64B (64-byte bf16 rows) bits 7..8, SWIZZLE_128B (128-byte f32
         // rows) bits 7..9
-        const int sw = sizeof(T) == 4 ? (lane & 7) : ((lane >> 1) & 3);
-        constexpr int kVec = 16 / int(sizeof(T));  // channels per 16-byte unit
+        const int sw = sizeof(Out) == 4 ? (lane & 7) : ((lane >> 1) & 3);
+        constexpr int kVec = 16 / int(sizeof(Out));  // channels per 16-byte unit
 #pragma unroll 1
         for (uint32_t f = 0; f < total; f++) {
             const uint32_t li = f / cpi, c = f - li * cpi, buf = li & 1, sb = f % kStgBufs;
@@ -324,17 +334,22 @@ __global__ void __launch_bounds__(kThreads, 1)
                 if (lane == 0) tma_store_wait_read<kStgBufs - 1>();  // the store that last read this buffer (chunk f - 4) is done with it
                 __syncwarp();
             }
-            uint8_t* row_ptr = stg + sb * kStgBytes + lane * (kChunk * int(sizeof(T)));
+            uint8_t* row_ptr = stg + sb * kStgBytes + lane * (kChunk * int(sizeof(Out)));
 #pragma unroll
             for (int j = 0; j < kChunk / kVec; j++) {  // kVec channels = one 16-byte unit of the row
                 float v[kVec];
 #pragma unroll
                 for (int k = 0; k < kVec; k++) {
                     float x = __uint_as_float(r[j * kVec + k]) + bias[j * kVec + k];
-                    v[k] = relu ? (x < 0.0f ? 0.0f : x) : x;  // NaN stays NaN, like torch / ONNX Relu
+                    if constexpr (kHead)
+                        v[k] = (col0 + j * kVec + k < p.relu_n && x < 0.0f) ? 0.0f : x;
+                    else
+                        v[k] = relu ? (x < 0.0f ? 0.0f : x) : x;  // NaN stays NaN, like torch / ONNX Relu
                 }
                 uint4* cell = reinterpret_cast<uint4*>(row_ptr + ((j ^ sw) << 4));
-                if constexpr (sizeof(T) == 4) {
+                if constexpr (kHead) {
+                    *cell = make_uint4(__float_as_uint(v[0]), __float_as_uint(v[1]), __float_as_uint(v[2]), __float_as_uint(v[3]));
+                } else if constexpr (sizeof(T) == 4) {
                     if (has_res) {  // the reference block is x + relu(bn(conv(...))): relu BEFORE the add (post_act.py:218-228)
                         const uint4 q = *cell;
                         v[0] += __uint_as_float(q.x);
@@ -384,28 +399,30 @@ __global__ void __launch_bounds__(kThreads, 1)
 
 }  // namespace
 
-// the same for every layer width: the ring holds up to 128 weight rows per CTA (a slice of <= 256 channels), biases are not staged
-size_t conv_i2c_smem_bytes(int stages, bool tf32) {
-    const size_t stg = tf32 ? kStgBytesOf<float> : kStgBytesOf<__nv_bfloat16>;
-    return 1024 /*alignment slack*/ + size_t(stages) * kStageBytes + 4 * kStgBufs * stg + (2 * stages + 4 + 4 * kStgBufs) * 8 + 16;
+// the same for every layer width: the ring holds up to 128 weight rows per CTA (a slice of <= 256 channels), biases are not staged;
+// out_esz: bytes per output element (2: bf16 tower layers, 4: TF32 tower layers and every head conv)
+size_t conv_i2c_smem_bytes(int stages, int out_esz) {
+    return 1024 /*alignment slack*/ + size_t(stages) * kStageBytes + 4 * kStgBufs * (32 * kChunk * size_t(out_esz)) + (2 * stages + 4 + 4 * kStgBufs) * 8 + 16;
 }
 
-// bf16: 6 stages; TF32: 5 (its staging boxes take 32 KB more)
-int conv_i2c_pick_stages(bool tf32) {
+// bf16 output: 6 stages; f32 output: 5 (its staging boxes take 32 KB more)
+int conv_i2c_pick_stages(int out_esz) {
     const size_t budget = 227 * 1024;
     int stages = 6;
-    while (stages > 2 && conv_i2c_smem_bytes(stages, tf32) > budget) stages--;
+    while (stages > 2 && conv_i2c_smem_bytes(stages, out_esz) > budget) stages--;
     return stages;
 }
 
 void conv_i2c_prepare() {
-    cudaFuncSetAttribute(conv_i2c_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    cudaFuncSetAttribute(conv_i2c_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaFuncSetAttribute(conv_i2c_kernel<__nv_bfloat16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaFuncSetAttribute(conv_i2c_kernel<float, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaFuncSetAttribute(conv_i2c_kernel<__nv_bfloat16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaFuncSetAttribute(conv_i2c_kernel<float, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
 }
 
 // tmap_a: im2col map over the dense channels-last activations (C, W, H, boards), one k-block x 128 pixels per load, SWIZZLE_128B;
 // tmap_bh: weight map whose box holds p.n / p.n_split / 2 rows (this CTA's half of a slice); tmap_out / tmap_res: output / residual rows, box (32 channels, 32 rows),
-// SWIZZLE_64B for bf16, SWIZZLE_128B for TF32 (tmap_res is only read when p.res is set)
+// SWIZZLE_64B for bf16, SWIZZLE_128B for f32 (tmap_res is only read when p.has_res is set)
 void launch_conv_i2c(const CUtensorMap& tmap_a, const CUtensorMap& tmap_bh, const CUtensorMap& tmap_out, const CUtensorMap& tmap_res,
                      const ConvTcParams& p, int grid, cudaStream_t s) {
     if (p.num_tiles <= 0) return;
@@ -413,7 +430,7 @@ void launch_conv_i2c(const CUtensorMap& tmap_a, const CUtensorMap& tmap_bh, cons
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(unsigned(2 * std::min(grid / 2, items)));
     cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = conv_i2c_smem_bytes(p.stages, p.tf32 != 0);
+    cfg.dynamicSmemBytes = conv_i2c_smem_bytes(p.stages, p.tf32 || p.head ? 4 : 2);
     cfg.stream = s;
     cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -424,10 +441,9 @@ void launch_conv_i2c(const CUtensorMap& tmap_a, const CUtensorMap& tmap_bh, cons
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = p.pdl ? 2 : 1;
-    if (p.tf32)
-        cudaLaunchKernelEx(&cfg, conv_i2c_kernel<float>, tmap_a, tmap_bh, tmap_out, tmap_res, p);
-    else
-        cudaLaunchKernelEx(&cfg, conv_i2c_kernel<__nv_bfloat16>, tmap_a, tmap_bh, tmap_out, tmap_res, p);
+    auto kernel = p.head ? (p.tf32 ? conv_i2c_kernel<float, true> : conv_i2c_kernel<__nv_bfloat16, true>)
+                         : (p.tf32 ? conv_i2c_kernel<float, false> : conv_i2c_kernel<__nv_bfloat16, false>);
+    cudaLaunchKernelEx(&cfg, kernel, tmap_a, tmap_bh, tmap_out, tmap_res, p);
 }
 
 }  // namespace kzb

@@ -313,7 +313,6 @@ void Net::build_tc() {
     mode_ = (!tf32 && W == 8 && H == 8 && !(force && force[0] == '1')) ? 1 : 0;
     // DENSE rows, one per square: conv_i2c.cu gets a 3x3 layer's zero padding from the TMA engine's im2col mode
     lay_ = RowLayout{W, H};
-    conv_tc_prepare();
     conv_i2c_prepare();
     if (mode_ == 1) {
         // 8x8: whole 4-board units; the cluster-pair tower kernel pads the batch to an even number of units
@@ -339,11 +338,15 @@ void Net::build_tc() {
     att_stride_ = spec_.has_attention ? spec_.att_chan_base.back() : 0;
     act_att_.alloc(size_t(rows_alloc_) * att_stride_ * 4);
 
+    // `width` output channels stored per row of `out` (stride `out_stride`, from channel out_off on).  Tower form: the output is the
+    // next layer's operand (bf16 / TF32), width a multiple of 32, relu_n 0 or width.  Head form (`head`, the 1x1 head convs): f32
+    // output, not rounded; the MMA runs width rounded up to 32 channels and the output map clips the rest.
     auto add = [&](const std::string& name, const ConvParams& c, DeviceBuffer& in, int in_stride, const DeviceBuffer* res,
-                   DeviceBuffer& out, int out_stride, bool out_f32, int n, int relu_n, int out_off = 0) {
+                   DeviceBuffer& out, int out_stride, bool head, int width, int relu_n, int out_off = 0) {
         auto st = std::make_unique<ConvStep>();
         st->name = name;
         st->taps = c.ksize * c.ksize;
+        const int n = round_up(width, 32);
         const int cin_pad = in_stride;
         const int ktot = st->taps * cin_pad;
         std::vector<float> wf(size_t(n) * ktot, 0.0f);
@@ -368,51 +371,37 @@ void Net::build_tc() {
             uint32_t box[2] = {uint32_t(kb), uint32_t(rows)};
             return make_tmap(st->w_tc.ptr, 2, dims, strides, box, true, false, dtype);
         };
-        if (n <= 256) st->tmap_b = wmap(n);  // conv_tc.cu and heads8.cu: every output channel in one box
-        int slice = n;                       // output channels per MMA
-        if (out_f32) {  // the head convs: 1x1 (net_spec.cpp), conv_tc.cu
-            if (st->taps != 1) throw std::logic_error("internal: conv_tc.cu runs 1x1 convs only");
-            uint64_t dims[2] = {uint64_t(in_stride), uint64_t(rows_alloc_)};
-            uint64_t strides[1] = {uint64_t(in_stride) * esz};
-            uint32_t box[2] = {uint32_t(kb), 128};
-            st->tmap_a = make_tmap(in.ptr, 2, dims, strides, box, true, false, dtype);
-        } else {  // conv_i2c.cu: cin_pad and n are multiples of kb, relu_n is 0 or n, out_off is 0
-            st->tmap_i2c = make_tmap_im2col(in.ptr, in_stride, W, H, boards_i2c_, kb, 128, st->taps == 9 ? 1 : 0, dtype);
-            auto rows_map = [&](void* ptr, int stride) {  // staging boxes of 32 rows x 32 channels: 64-byte (bf16) or 128-byte (f32) rows
-                uint64_t dims[2] = {uint64_t(stride), uint64_t(rows_alloc_)};
-                uint64_t strides[1] = {uint64_t(stride) * esz};
-                uint32_t box[2] = {32, 32};
-                return make_tmap(ptr, 2, dims, strides, box, tf32, !tf32, dtype);
-            };
-            st->tmap_out = rows_map(out.ptr, out_stride);
-            st->tmap_res = res ? rows_map(res->ptr, c_pad_) : st->tmap_out;
-            // output channels in split0 slices (twice as many for small batches, run_network); each CTA of a pair stages half of
-            // every weight tile of its slice
-            st->split0 = base_split(n);
-            if (st->split0 == 0) throw std::logic_error("internal: conv_i2c layer of " + std::to_string(n) + " channels has no slicing");
-            slice = n / st->split0;
-            st->split_double = slice % 64 == 0;  // the halved slice is still whole 32-channel chunks
-            st->tmap_w[0] = wmap(slice / 2);
-            st->tmap_w[1] = st->split_double ? wmap(slice / 4) : st->tmap_w[0];
-            st->use_i2c = true;
-            st->i2c_stages = conv_i2c_pick_stages(tf32);
-        }
+        st->tmap_i2c = make_tmap_im2col(in.ptr, in_stride, W, H, boards_i2c_, kb, 128, st->taps == 9 ? 1 : 0, dtype);
+        // staging boxes of 32 rows x 32 channels: 64-byte (bf16) or 128-byte (f32) rows; `cols` channels of rows `stride` apart
+        auto rows_map = [&](void* ptr, int cols, int stride, bool f32) {
+            uint64_t dims[2] = {uint64_t(cols), uint64_t(rows_alloc_)};
+            uint64_t strides[1] = {uint64_t(stride) * (f32 ? 4 : 2)};
+            uint32_t box[2] = {32, 32};
+            return make_tmap(ptr, 2, dims, strides, box, f32, !f32, f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
+        };
+        const bool f32_out = tf32 || head;
+        st->tmap_out = rows_map(static_cast<uint8_t*>(out.ptr) + size_t(out_off) * (f32_out ? 4 : 2), width, out_stride, f32_out);
+        st->tmap_res = res ? rows_map(res->ptr, c_pad_, c_pad_, tf32) : st->tmap_out;
+        // output channels in split0 slices (twice as many for small batches, run_network); each CTA of a pair stages half of
+        // every weight tile of its slice
+        st->split0 = base_split(n);
+        if (st->split0 == 0) throw std::logic_error("internal: conv_i2c layer of " + std::to_string(n) + " channels has no slicing");
+        const int slice = n / st->split0;
+        st->split_double = slice % 64 == 0;  // the halved slice is still whole 32-channel chunks
+        st->tmap_w[0] = wmap(slice / 2);
+        st->tmap_w[1] = st->split_double ? wmap(slice / 4) : st->tmap_w[0];
         ConvTcParams& p = st->tc;
         p.taps = st->taps;
         p.cin_pad = cin_pad;
         p.kblocks = cin_pad / kb;
         p.tf32 = tf32 ? 1 : 0;
+        p.head = head ? 1 : 0;
         p.n = n;
         p.lay = lay_;
         p.bias = st->bias.as<float>();
         p.relu_n = relu_n;
-        p.res = res ? res->ptr : nullptr;
-        p.res_stride = c_pad_;
-        p.out = static_cast<uint8_t*>(out.ptr) + size_t(out_off) * (out_f32 ? 4 : esz);
-        p.out_stride = out_stride;
-        p.out_f32 = out_f32 ? 1 : 0;
-        p.n_store = n;
-        p.stages = conv_tc_pick_stages(n);
+        p.has_res = res ? 1 : 0;
+        p.stages = conv_i2c_pick_stages(f32_out ? 4 : 2);
         int cols = 32;  // two accumulators of the widest slice
         while (cols < 2 * slice) cols *= 2;
         p.tmem_cols = cols;
@@ -429,12 +418,12 @@ void Net::build_tc() {
     }
     head_first_ = convs_.size();
     if (spec_.has_attention) {
-        add("scalar_conv", merged_small_conv(spec_), act_x_, c_pad_, nullptr, act_s1_, s1_stride_, true, 16, spec_.scalar_conv.cout);
+        add("scalar_conv", merged_small_conv(spec_), act_x_, c_pad_, nullptr, act_s1_, s1_stride_, true, s1_stride_, spec_.scalar_conv.cout);
         for (const AttChunk& ch : att_chunks(spec_))
             add(ch.name, ch.conv, act_x_, c_pad_, nullptr, act_att_, att_stride_, true, round_up(ch.conv.cout, 16), 0, ch.out_off);
     } else {
         add("policy_conv1", spec_.policy_conv1, act_x_, c_pad_, nullptr, act_h1_, cp_pad_, false, cp_pad_, cp_pad_);
-        add("scalar_conv", merged_small_conv(spec_), act_x_, c_pad_, nullptr, act_s1_, s1_stride_, true, 16, spec_.scalar_conv.cout);
+        add("scalar_conv", merged_small_conv(spec_), act_x_, c_pad_, nullptr, act_s1_, s1_stride_, true, s1_stride_, spec_.scalar_conv.cout);
         add("policy_conv2", spec_.policy_conv2, act_h1_, cp_pad_, nullptr, act_pm_, pm_stride_, true, pm_stride_, 0);
     }
 
@@ -458,9 +447,16 @@ void Net::build_tc() {
             hp.b1 = c1.bias.as<float>();
             hp.bs = cs.bias.as<float>();
             hp.b2 = c2.bias.as<float>();
-            heads_maps_.w1 = c1.tmap_b;
-            heads_maps_.ws = cs.tmap_b;
-            heads_maps_.w2 = c2.tmap_b;
+            // the first `rows` output channels of a 1x1 step's bf16 weights [n][cin_pad], all of them in one box
+            auto wmap = [&](const ConvStep& st, int rows) {
+                uint64_t dims[2] = {uint64_t(st.tc.cin_pad), uint64_t(rows)};
+                uint64_t strides[1] = {uint64_t(st.tc.cin_pad) * 2};
+                uint32_t box[2] = {64, uint32_t(rows)};
+                return make_tmap(st.w_tc.ptr, 2, dims, strides, box);
+            };
+            heads_maps_.w1 = wmap(c1, hp.n1);
+            heads_maps_.ws = wmap(cs, 16);
+            heads_maps_.w2 = wmap(c2, hp.n2);
             uint64_t dims[2] = {uint64_t(c_pad_), uint64_t(rows_alloc_)};
             uint64_t strides[1] = {uint64_t(c_pad_) * 2};
             uint32_t box[2] = {64, 128};
@@ -765,20 +761,13 @@ void Net::run_network(int batch, const StepHook& hook) {
         auto& st = convs_[si];
         if (precision_ != 0) {
             ConvTcParams p = st->tc;
-            p.valid_rows = batch * lay_.W * lay_.H;
-            p.num_tiles = (p.valid_rows + 127) / 128;
-            if (st->use_i2c) {
-                p.stages = st->i2c_stages;
-                // the output channels in split0 slices of <= 256; small batches: twice the slices, so that twice as many SM pairs
-                // share the layer, when the work items fill at most half of them (KZB_CONV_SPLIT=0: never)
-                const char* split = std::getenv("KZB_CONV_SPLIT");
-                const bool dbl = !(split && split[0] == '0') && st->split_double && p.n_store == p.n &&
-                                 2 * ((p.num_tiles + 1) / 2) * st->split0 <= num_sms_ / 2;
-                p.n_split = st->split0 * (dbl ? 2 : 1);
-                launch_conv_i2c(st->tmap_i2c, st->tmap_w[dbl ? 1 : 0], st->tmap_out, st->tmap_res, p, num_sms_, stream_);
-            } else {
-                launch_conv_tc(st->tmap_a, st->tmap_b, p, num_sms_, stream_);
-            }
+            p.num_tiles = (batch * lay_.W * lay_.H + 127) / 128;
+            // the output channels in split0 slices of <= 256; small batches: twice the slices, so that twice as many SM pairs share
+            // the layer, when the work items fill at most half of them (KZB_CONV_SPLIT=0: never)
+            const char* split = std::getenv("KZB_CONV_SPLIT");
+            const bool dbl = !(split && split[0] == '0') && st->split_double && 2 * ((p.num_tiles + 1) / 2) * st->split0 <= num_sms_ / 2;
+            p.n_split = st->split0 * (dbl ? 2 : 1);
+            launch_conv_i2c(st->tmap_i2c, st->tmap_w[dbl ? 1 : 0], st->tmap_out, st->tmap_res, p, num_sms_, stream_);
         } else {
             ConvF32Params p = st->f32;
             p.batch = batch;

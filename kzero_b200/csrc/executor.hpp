@@ -45,13 +45,10 @@ struct PinnedBuffer {
 struct ConvStep {
     std::string name;
     int taps = 9;
-    // tensor-core form (bf16, or f32 rounded to TF32)
-    CUtensorMap tmap_a{}, tmap_b{};  // tmap_b: weight box of all n rows (n <= 256 only)
-    bool use_i2c = false;  // conv_i2c.cu (TMA im2col, CTA-pair MMA); otherwise conv_tc.cu (1x1, f32 output)
-    int i2c_stages = 0;
-    CUtensorMap tmap_out{}, tmap_res{};  // conv_i2c: output / residual rows, box (32 channels, 32 rows), SWIZZLE_64B
+    // tensor-core form (bf16, or f32 rounded to TF32): conv_i2c.cu
+    CUtensorMap tmap_out{}, tmap_res{};  // output / residual rows, box (32 channels, 32 rows): SWIZZLE_64B bf16, SWIZZLE_128B f32
     CUtensorMap tmap_i2c{};  // im2col map of the input rows
-    // conv_i2c output channel slices: split0 slices of n / split0 <= 256 channels, or (split_double, small batches) 2 * split0;
+    // output channel slices: split0 slices of n / split0 <= 256 channels, or (split_double, small batches) 2 * split0;
     // tmap_w[i]: weight box of half a slice (n / split0 / 2, n / split0 / 4 rows)
     int split0 = 1;
     bool split_double = false;

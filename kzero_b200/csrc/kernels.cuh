@@ -1,6 +1,6 @@
 // Device-side parameter blocks and host launchers for the hot path's kernels (sm_100a only).
 //   K2  encode      packed bitboards + scalars -> input planes          (encode.cu)      HBM-bound
-//   K1  conv tower  implicit-GEMM conv3x3/1x1 on tcgen05 + TMA + TMEM   (tower8k.cu, conv_i2c.cu, conv_tc.cu)  tensor-bound
+//   K1  conv tower  implicit-GEMM conv3x3/1x1 on tcgen05 + TMA + TMEM   (tower8k.cu, conv_i2c.cu)  tensor-bound
 //       conv fp32   CUDA-core fp32 implicit GEMM, the <=1e-4 parity mode (conv_fp32.cu)
 //   K3  heads tail  scalar-head FCs, policy gather, masked softmax      (heads.cu, decode: head_decode.cuh)  HBM/latency-bound
 #pragma once
@@ -94,34 +94,24 @@ struct ConvTcParams {
     int taps;       // 1 or 9
     int kblocks;    // cin_pad / (channels per 128-byte k-block: 64 bf16 or 32 TF32)
     int cin_pad;
-    int n;  // padded cout: conv_tc UMMA N, multiple of 16, <= 256; conv_i2c multiple of 32, <= 1024 (UMMA N = n / n_split <= 256)
+    int n;  // padded cout, the MMA width: multiple of 32, <= 1024 (UMMA N = n / n_split <= 256)
     RowLayout lay;
-    int valid_rows;  // rows >= valid_rows are not stored
     const float* bias;  // [n]
-    int relu_n;
-    const void* res;  // optional [rows][res_stride], the activation type
-    int res_stride;
-    void* out;  // [rows][out_stride] bf16 or f32 (conv_i2c TF32: f32 rounded to TF32)
-    int out_stride;
-    int out_f32;
-    int n_store;  // channels written per row (multiple of 16, <= n)
+    int relu_n;         // relu on output channels < relu_n (tower form: 0 or n)
+    int has_res;        // tower form: add the residual rows (tmap_res) after the relu
     int stages;
     int tmem_cols;
-    int n_split;  // conv_i2c: slices of the output channels; a work item is one 256-pixel tile x n / n_split channels (n / n_split <= 256, multiple of 32)
-    int pdl;      // conv_i2c: launched with programmatic stream serialization (set-up and the first weight tiles overlap the previous layer's tail)
+    int n_split;  // slices of the output channels; a work item is one 256-pixel tile x n / n_split channels (n / n_split <= 256, multiple of 32)
+    int pdl;      // launched with programmatic stream serialization (set-up and the first weight tiles overlap the previous layer's tail)
     int tf32;     // operands and activations are f32 rounded to TF32 (tcgen05 kind::tf32, 32 channels per k-block); 0: bf16
+    int head;     // head form: f32 output, not rounded, no residual (the head 1x1 convs); 0: tower form, output in the operand type
 };
-// conv_tc.cu: conv1x1 on dense rows (tmap_a: box (one 128-byte k-block of channels, 128 rows), tmap_b: weight box (k-block, p.n))
-void launch_conv_tc(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const ConvTcParams& p, int grid, cudaStream_t s);
 // conv_i2c.cu: conv3x3 / conv1x1 (p.taps) on DENSE rows, activation tiles by TMA im2col, CTA-pair MMA (tmap_bh: weight box of p.n / p.n_split / 2 rows)
 void launch_conv_i2c(const CUtensorMap& tmap_a_im2col, const CUtensorMap& tmap_bh, const CUtensorMap& tmap_out, const CUtensorMap& tmap_res,
                      const ConvTcParams& p, int grid, cudaStream_t s);
-size_t conv_i2c_smem_bytes(int stages, bool tf32);
-int conv_i2c_pick_stages(bool tf32);
-void conv_i2c_prepare();
-size_t conv_tc_smem_bytes(int n, int stages);
-int conv_tc_pick_stages(int n);
-void conv_tc_prepare();  // per-device (both operand types): opt in to 227 KB dynamic shared memory
+size_t conv_i2c_smem_bytes(int stages, int out_esz);
+int conv_i2c_pick_stages(int out_esz);  // out_esz: bytes per output element
+void conv_i2c_prepare();  // per-device (every instance): opt in to 227 KB dynamic shared memory
 
 // whole-tower persistent kernel for 8x8 boards (tower8k.cu)
 struct TowerLayerDev {

@@ -116,7 +116,7 @@ CASES = [
     Case("heads8-n2-128", channels=64, n2=128, batch=5, launches=3),
     Case("tail8-hs33", channels=32, hs=33, batch=5, launches=TAIL_8X8),
     Case("tail8-n1-192", channels=64, n1=192, batch=5, launches=TAIL_8X8),
-    # ---- conv_i2c + conv_tc + tail kernel (go: encode, 2 depth + 1 convs, 3 head convs, tail)
+    # ---- conv_i2c (tower and head form) + tail kernel (go: encode, 2 depth + 1 convs, 3 head convs, tail)
     Case("go-3-c64-b1", game="go-3", channels=64, depth=1, batch=1),
     Case("go-5-c96-b2", game="go-5", channels=96, depth=1, batch=2, variants=(V(KZB_PDL="0"),)),
     Case("go-9-c192-b7", game="go-9", channels=192, depth=1, batch=7, variants=(V(KZB_CONV_SPLIT="0"),)),

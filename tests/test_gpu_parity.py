@@ -136,7 +136,7 @@ def test_bf16_packed_vs_oracle(game, depth, ch, n, variant, monkeypatch):
     (KZB_NO_TOWER8=1; by default for layers wider than 128 channels, and for chess batch 9600, which has more 4-board units per SM than
     the whole-tower kernel keeps), no 8x8 conv kernel at all (KZB_NO_TOWER8=1 and KZB_NO_HEADS8=1: conv_i2c.cu on 8x8 boards, per-op
     head convs + tail kernel), and the row kernels of every other board (go; KZB_FORCE_LINEAR=1 / KZB_NO_EMBED8=1 push chess / ataxx
-    there): dense rows with TMA im2col loads and the CTA-pair MMA (conv_i2c.cu), the head 1x1 convs (conv_tc.cu) and the tail kernel,
+    there): dense rows with TMA im2col loads and the CTA-pair MMA (conv_i2c.cu, also the head 1x1 convs) and the tail kernel,
     without programmatic dependent launch (KZB_PDL=0), and without sharing a tile's output channels between two SM pairs at small
     batches (KZB_CONV_SPLIT=0).  Boards smaller than 8x8 (ataxx 7x7) are embedded in the 8x8 grid and masked after every layer."""
     row_variants = ("linear", "no_pdl", "no_conv_split")  # everything off the 8x8 kernels

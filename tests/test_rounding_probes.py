@@ -57,7 +57,7 @@ FORMATS = {
 }
 
 # case id -> the switches run besides the default.  Together the bf16 cases cover every bf16 path: tower8k with heads8 (chess,
-# ataxx-5 embedded, 9472 boards), the tail kernel with conv_tc and conv_i2c for the 1x1 convs (KZB_NO_HEADS8), conv_i2c for the 8x8
+# ataxx-5 embedded, 9472 boards), the tail kernel with conv_i2c for the 1x1 convs (KZB_NO_HEADS8), conv_i2c for the 8x8
 # tower (KZB_NO_TOWER8) and for a small board (KZB_NO_EMBED8), go with and without the doubled channel split, a non-square board,
 # a layer in slices, and the attention head created through ONNX.
 CASES = {
